@@ -225,6 +225,29 @@ def rel_err(a, b) -> dict:
             "max_rel_to_absmax": float(d.max() / (b.abs().max() + 1e-12))}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """``--dump-outputs``: write each result as ``out_dir/<name>.npy`` in float32, so that two builds run with the same
+    arguments can be compared output for output.  An array over its share of ``DUMP_BYTES`` is replaced by a fixed
+    seeded sample of its flattened elements (the same positions for the same shape)."""
+    if not out_dir:
+        return
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // (4 * len(arrays))
+    for name, t in arrays.items():
+        flat = t.detach().float().flatten().cpu()
+        if flat.numel() > cap:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            flat = flat[idx]
+        else:
+            flat = flat.view(t.shape)
+        np.save(os.path.join(out_dir, name + ".npy"), flat.numpy())
+
+
 DTYPE_NAMES = {"bf16": "bf16", "fp8": "fp8 (MXFP8 block-scaled tcgen05 GEMMs for the block linears = 99.9% of the FLOPs; "
                                       "attention, norms, embedders bf16/fp32)"}
 
@@ -365,6 +388,10 @@ def run_ours(args) -> int:
         import torch.distributed as dist
         dist.destroy_process_group()
     if rank == 0:
+        dumps = {"x_next": main["result"]}
+        if "bf16" in extra:
+            dumps["bf16_x_next"] = alt["result"]
+        dump_outputs(args.dump_outputs, dumps)
         emit(make_line(args, "ours", main["ms"], main["ms_e2e"], main["clocks"], h2d, d2h, main["launches"],
                        main["finite"], DTYPE_NAMES[args.dtype], main["notes"], extra))
     return 0
@@ -458,6 +485,7 @@ def run_nodes(args) -> int:
         sync_all()
         extra["output_matches_n1"] = rel_err(got, want)
     launches = sum(getattr(s.replica, "launches_per_step", 0) for s in eng.slots) * args.steps
+    dump_outputs(args.dump_outputs, {"x_next": result_host})
     pa.cleanup_parallel_model(model)
     host_only_release(world)
     notes = {"parallelism": "ONE process, ComfyUI node API: native sm_100a replicas, in-kernel NVLink scatter/gather, "
@@ -550,6 +578,7 @@ def run_reference(args) -> int:
     ms_e2e = timed(step_e2e, args.steps, max(3, args.warmup // 2), 1)
     clocks = sampler.stop(args.gpus)
     finite = bool(torch.isfinite(result_host.float()).all().item())
+    dump_outputs(args.dump_outputs, {"x_next": result_host})
     host_only_release(world)
     notes = {"parallelism": f"reference threads x{args.gpus} (single process, stock torch kernels); idle torchrun ranks "
                             "hold no CUDA context",
@@ -577,7 +606,12 @@ def main() -> int:
                     help="fp8 (default; BASELINE config 3 names fp8) = MXFP8 block-scaled GEMMs for the block linears; "
                          "the bf16 number of the same workload is measured in the same run and reported under 'bf16'")
     ap.add_argument("--no-bf16", action="store_true", help="with --dtype fp8: skip the additional bf16 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step (the next latent) as DIR/x_next.npy in float32; "
+                         "when --dtype fp8 also measures bf16, that run's result as DIR/bf16_x_next.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     quiet_stdout()
     if args.impl == "reference":

@@ -1,3 +1,4 @@
+import importlib.util
 import os
 import sys
 
@@ -6,6 +7,27 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+
+
+def _import_repository_package():
+    """The repository root is a package as well (ComfyUI loads it through its ``__init__.py``), so pytest collects it as
+    one and imports it by its directory name through the parent directory.  That import fails, and with it every test,
+    when the parent directory may be entered but not listed.  Importing the package here from its own path leaves pytest
+    a module to find in ``sys.modules``; its relative import of the inner package gets the copy the tests use."""
+    import comfyui_parallelanything_b200
+    name = os.path.basename(ROOT)
+    if (not name.isidentifier() or name in sys.modules
+            or os.path.isfile(os.path.join(os.path.dirname(ROOT), "__init__.py"))):
+        return                      # pytest names or finds the root package without a listing of the parent
+    sys.modules[name + ".comfyui_parallelanything_b200"] = comfyui_parallelanything_b200
+    spec = importlib.util.spec_from_file_location(name, os.path.join(ROOT, "__init__.py"),
+                                                  submodule_search_locations=[ROOT])
+    module = importlib.util.module_from_spec(spec)
+    sys.modules[name] = module
+    spec.loader.exec_module(module)
+
+
+_import_repository_package()
 
 
 def pytest_configure(config):
@@ -27,12 +49,3 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip_gpu)
         if "multigpu" in item.keywords and ngpu < 2:
             item.add_marker(skip_multi)
-
-
-@pytest.fixture(scope="session")
-def reference():
-    from baseline import ref_loader
-    try:
-        return ref_loader.load()
-    except ref_loader.ReferenceUnavailable as e:
-        pytest.skip(f"reference unavailable: {e}")
