@@ -8,10 +8,22 @@ from __future__ import annotations
 
 from typing import Callable, Optional
 
+import torch
 import torch.nn as nn
 
 
 WORKSPACE_LIMIT = 6     # distinct (batch, resolution, text length) activation workspaces kept per executor
+
+
+def bf16(t: torch.Tensor, device) -> torch.Tensor:
+    """A weight as a contiguous bf16 tensor on ``device``, detached from the source module."""
+    return t.detach().to(device=device, dtype=torch.bfloat16).contiguous()
+
+
+def conditioning_sig(ctx: torch.Tensor) -> tuple:
+    """Identity of a conditioning tensor: results computed from it stay valid while this is unchanged (same buffer,
+    same shape, not written in place since)."""
+    return (ctx.data_ptr(), tuple(ctx.shape), ctx._version)
 
 
 def cache_workspace(cache: dict, key, ws: dict, device=None, on_evict: Optional[Callable] = None) -> dict:
@@ -25,7 +37,6 @@ def cache_workspace(cache: dict, key, ws: dict, device=None, on_evict: Optional[
         if old == key:
             break
         if device is not None:
-            import torch
             if torch.cuda.is_available():
                 torch.cuda.synchronize(device)
         if on_evict is not None:

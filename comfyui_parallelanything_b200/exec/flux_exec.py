@@ -19,41 +19,30 @@ Per step: 19*13 + 38*4 + ~12 = ~410 kernel launches, optionally replayed as one 
 from __future__ import annotations
 
 import os
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional
 
 import torch
 import torch.nn as nn
 
 from .. import ops
-from . import cache_workspace, recognize, touch_workspace
-from .graphs import GraphCache
+from . import bf16, block_linear, quantize_block_weights
+from .dit import DiTExecutor, head_gather, rope_layout
 from ..models import flux as flux_model
-from ..utils import log
 from ..utils.log import nvtx_range
 
 
-def _bf16(t: torch.Tensor, device) -> torch.Tensor:
-    return t.detach().to(device=device, dtype=torch.bfloat16).contiguous()
-
-
-class FluxExecutor(nn.Module):
+class FluxExecutor(DiTExecutor):
     pa_family = "flux"
-    pa_native = True
 
     def __init__(self, model: "flux_model.Flux", device, cuda_graphs: bool = False, fp8: bool = False):
-        super().__init__()
-        ops.require()
-        self.device = torch.device(device)
-        # hyper-parameters come from the module's STRUCTURE (weight shapes, ComfyUI attribute names), so a
-        # comfy.ldm.flux.model.Flux is packed exactly like the repository's own oracle class
-        p = self.params = recognize.params_of(model, "flux")
+        super().__init__(model, device, cuda_graphs)
+        p = self.params
         self.hid, self.heads = p.hidden_size, p.num_heads
         if self.hid // self.heads != 128:
             raise ValueError("FluxExecutor is specialised for head_dim 128")
         if p.patch_size != 2:
             raise ValueError("FluxExecutor is specialised for 2x2 patches")
         self.mlp = int(p.hidden_size * p.mlp_ratio)
-        self.cuda_graphs = cuda_graphs
         # fp8=True: the block GEMMs (qkv / proj / mlp / linear1 / linear2 = 99.9 % of the FLOPs) run as MXFP8
         # block-scaled tcgen05 GEMMs (weights quantised once here, activations per GEMM); embedders,
         # modulation and the final layer stay bf16.
@@ -64,8 +53,8 @@ class FluxExecutor(nn.Module):
         W: Dict[str, torch.Tensor] = {}
 
         def lin(name, m):
-            W[name + ".w"] = _bf16(m.weight, d)
-            W[name + ".b"] = _bf16(m.bias, d) if m.bias is not None else None
+            W[name + ".w"] = bf16(m.weight, d)
+            W[name + ".b"] = bf16(m.bias, d) if m.bias is not None else None
 
         lin("img_in", model.img_in)
         lin("txt_in", model.txt_in)
@@ -77,7 +66,7 @@ class FluxExecutor(nn.Module):
             outs.append(model.guidance_in.out_layer)
         outs.append(model.vector_in.out_layer)
         # vec = sum_i out_i(h_i)  ==  [h_t | h_g | h_y] @ [W_t | W_g | W_y]^T + (b_t + b_g + b_y)
-        W["vec_out.w"] = torch.cat([_bf16(o.weight, d) for o in outs], dim=1).contiguous()
+        W["vec_out.w"] = torch.cat([bf16(o.weight, d) for o in outs], dim=1).contiguous()
         W["vec_out.b"] = sum(o.bias.detach().float().to(d) for o in outs).to(torch.bfloat16)
         mods, self.mod_off = [], {}
         off = 0
@@ -91,73 +80,51 @@ class FluxExecutor(nn.Module):
                 lin(f"d{i}.{s}.proj", getattr(blk, s + "_attn").proj)
                 lin(f"d{i}.{s}.mlp0", getattr(blk, s + "_mlp")[0])
                 lin(f"d{i}.{s}.mlp2", getattr(blk, s + "_mlp")[2])
-                W[f"d{i}.{s}.qs"] = _bf16(getattr(blk, s + "_attn").norm.query_norm.scale, d)
-                W[f"d{i}.{s}.ks"] = _bf16(getattr(blk, s + "_attn").norm.key_norm.scale, d)
+                W[f"d{i}.{s}.qs"] = bf16(getattr(blk, s + "_attn").norm.query_norm.scale, d)
+                W[f"d{i}.{s}.ks"] = bf16(getattr(blk, s + "_attn").norm.key_norm.scale, d)
         for i, blk in enumerate(model.single_blocks):
             mods.append(blk.modulation.lin)
             self.mod_off[("s", i)] = off
             off += blk.modulation.lin.weight.shape[0]
             lin(f"s{i}.l1", blk.linear1)
             lin(f"s{i}.l2", blk.linear2)
-            W[f"s{i}.qs"] = _bf16(blk.norm.query_norm.scale, d)
-            W[f"s{i}.ks"] = _bf16(blk.norm.key_norm.scale, d)
+            W[f"s{i}.qs"] = bf16(blk.norm.query_norm.scale, d)
+            W[f"s{i}.ks"] = bf16(blk.norm.key_norm.scale, d)
         fin = model.final_layer.adaLN_modulation[1]
         mods.append(fin)
         self.mod_off[("final",)] = off
         off += fin.weight.shape[0]
         self.mod_total = off
-        W["mod.w"] = torch.cat([_bf16(m.weight, d) for m in mods], dim=0).contiguous()
-        W["mod.b"] = torch.cat([_bf16(m.bias, d) for m in mods], dim=0).contiguous()
+        W["mod.w"] = torch.cat([bf16(m.weight, d) for m in mods], dim=0).contiguous()
+        W["mod.b"] = torch.cat([bf16(m.bias, d) for m in mods], dim=0).contiguous()
         lin("final", model.final_layer.linear)
         self.W = W
         if self.fp8:
-            big = [k[:-2] for k in list(W) if k.endswith(".w") and (k.startswith("d") or k.startswith("s"))
-                   and k.split(".")[-2] in ("qkv", "proj", "mlp0", "mlp2", "l1", "l2")]
+            names = [k[:-2] for k in W if k.endswith(".w") and (k.startswith("d") or k.startswith("s"))
+                     and k.split(".")[-2] in ("qkv", "proj", "mlp0", "mlp2", "l1", "l2")]
             # the modulation table (all blocks' adaLN linears, 1 056 768 x 3072 for FLUX.1-dev) is a pure weight stream
             # (6.5 GB in bf16 for <= 8 rows of activations): as MXFP8 it is half the bytes
             if os.environ.get("PA_FP8_MOD", "1") != "0":
-                big.append("mod")
-            for name in big:
-                w = W.pop(name + ".w")
-                if w.shape[0] % 128 or w.shape[1] % 128:
-                    W[name + ".w"] = w
-                    continue
-                # B-tile width the GEMM will use: 256 (single accumulator) for the fused QKV epilogues,
-                # 224 (double-buffered accumulators) for everything else
-                tile = 256 if name.split(".")[-1] in ("qkv", "l1") else 224
-                W[name + ".q"], W[name + ".sf"] = ops.quantize_mxfp8(w, tile)
-                W[name + ".tile"] = tile
-                del w
+                names.append("mod")
+            # B-tile width the GEMM will use: 256 (single accumulator) for the fused QKV epilogues,
+            # 224 (double-buffered accumulators) for everything else
+            quantize_block_weights(W, names, lambda n: 256 if n.split(".")[-1] in ("qkv", "l1") else 224)
             torch.cuda.empty_cache()
         self.n_double, self.n_single = len(model.double_blocks), len(model.single_blocks)
-        self._ws: Dict[Tuple, dict] = {}
-        self._graphs = GraphCache(self.device, enabled=cuda_graphs)
         # fork the txt / img chains of the double blocks onto two streams with disjoint SM budgets (PA_DUAL_STREAM=0: off)
         self.dual_stream = os.environ.get("PA_DUAL_STREAM", "1") != "0"
         # fp8: attention / GELU epilogues emit the next GEMM's MXFP8 A operand themselves (PA_FP8_FUSED_QUANT=0: separate
         # quantise kernels in front of every GEMM)
         self.fused_quant = os.environ.get("PA_FP8_FUSED_QUANT", "1") != "0"
         self._side = self._ev_fork = self._ev_join = None
-        self.launches_per_step = 0
-
-    # nn.Module plumbing so engine utilities (module_device, .to("meta") on cleanup) work
-    def parameters(self, recurse: bool = True):  # type: ignore[override]
-        return iter(())
-
-    def release(self) -> None:
-        self.W.clear()
-        self._ws.clear()
-        self._graphs.clear()
-
-    def weight_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in self.W.values() if isinstance(t, torch.Tensor))
 
     # ------------------------------------------------------------------ workspaces
-    def workspace(self, B: int, H: int, Wd: int, Lt: int) -> dict:
-        key = (B, H, Wd, Lt)
-        ws = touch_workspace(self._ws, key)
-        if ws is not None:
-            return ws
+    def rope(self, H: int, Wd: int, Lt: int) -> torch.Tensor:
+        """fp32 [Lt + (H/2)*(W/2), 64, 2] RoPE table of the joint [txt | img] sequence."""
+        ids = flux_model.position_ids(1, H // 2, Wd // 2, Lt, self.device)
+        return rope_layout(flux_model.EmbedND(128, self.params.theta, self.params.axes_dim)(ids))
+
+    def _new_workspace(self, B: int, H: int, Wd: int, Lt: int) -> dict:
         d, hid, mlp = self.device, self.hid, self.mlp
         Li = (H // 2) * (Wd // 2)
         L = Lt + Li
@@ -184,33 +151,10 @@ class FluxExecutor(nn.Module):
             ws["XM8"], ws["XM8_SF"] = u8(B, L, hid), sfb(L, hid)            # LayerNorm+modulate outputs, per chain
             ws["XM8I"], ws["XM8I_SF"] = u8(B, Li, hid), sfb(Li, hid)
             ws["XM8T"], ws["XM8T_SF"] = u8(B, Lt, hid), sfb(Lt, hid)
-        m = flux_model.Flux.__new__(flux_model.Flux)
-        m.patch_size = 2
-        ids = flux_model.Flux.make_ids(m, 1, H, Wd, Lt, d)
-        pe = flux_model.EmbedND(128, self.params.theta, self.params.axes_dim)(ids)     # [1,1,L,64,2,2]
-        ws["ROPE"] = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float().contiguous()
-        cache_workspace(self._ws, key, ws, device=self.device, on_evict=lambda _k: self._graphs.clear())
+        ws["ROPE"] = self.rope(H, Wd, Lt)
         return ws
 
     # ------------------------------------------------------------------ schedule
-    def _lin(self, a, name: str, mode: str, a8=None, **kw) -> int:
-        """One block Linear: bf16 tcgen05 GEMM, or (fp8) quantise the activation + block-scaled fp8 GEMM.  ``a8`` =
-        (e4m3 bytes, scale chunks) when the producer already emitted the MXFP8 operand.  Returns the launch count."""
-        W = self.W
-        if name + ".q" in W:
-            n = 1
-            if a8 is None:
-                a8 = ops.quantize_mxfp8(a)
-                n = 3
-            ops.gemm_fp8(a8[0], a8[1], W[name + ".q"], W[name + ".sf"], mode, W[name + ".tile"], bias=W[name + ".b"], **kw)
-            return n
-        ops.gemm(a, W[name + ".w"], mode, bias=W[name + ".b"], **kw)
-        return 1
-
-    def _mod(self, ws, key, idx):
-        off = self.mod_off[key] + idx * self.hid
-        return ws["MOD"][:, off:off + self.hid]
-
     def _run(self, ws, x_ptr: int, t, ctx, y, guidance, out, x_in=None, sigmas=None, out_ptr: Optional[int] = None,
              out_sample_off: int = 0, t_ptr: Optional[int] = None, g_ptr: Optional[int] = None, x_copy=None):
         W, hid, mlp, Lt, B = self.W, self.hid, self.mlp, ws["Lt"], ws["B"]
@@ -249,7 +193,7 @@ class FluxExecutor(nn.Module):
             n += 1
         ops.gemm(y, W["vector_in.in.w"], "silu", out=HC[:, col:col + hid], bias=W["vector_in.in.b"])
         ops.gemm(HC, W["vec_out.w"], "silu", out=ws["SVEC"], bias=W["vec_out.b"])          # silu(vec)
-        n += 2 + self._lin(ws["SVEC"], "mod", "bias", out=ws["MOD"])                         # all modulations
+        n += 2 + block_linear(W, ws["SVEC"], "mod", "bias", out=ws["MOD"])                   # all modulations
         # ---- double-stream blocks
         # Between two joint attentions the txt and img chains are independent.  Run back to back, the 512-row txt
         # GEMMs fill 24-96 of the 74 CTA-pair slots and the img GEMMs end in a partial wave; forked onto two streams
@@ -277,11 +221,11 @@ class FluxExecutor(nn.Module):
             k = ("d", i, s)
             if fused8 and f"d{i}.{s}.qkv.q" in W:
                 a8 = ln8(xs, s, self._mod(ws, k, 1), self._mod(ws, k, 0))
-                return 1 + self._lin(None, f"d{i}.{s}.qkv", "qkv_rope", a8=a8, q=Q, k=K, v=V, q_scale=W[f"d{i}.{s}.qs"],
-                                     k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=seq_off)
+                return 1 + block_linear(W, None, f"d{i}.{s}.qkv", "qkv_rope", a8=a8, q=Q, k=K, v=V,
+                                        q_scale=W[f"d{i}.{s}.qs"], k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=seq_off)
             ops.layernorm_modulate(xs, xms, scale=self._mod(ws, k, 1), shift=self._mod(ws, k, 0))
-            return 1 + self._lin(xms, f"d{i}.{s}.qkv", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"d{i}.{s}.qs"],
-                                 k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=seq_off)
+            return 1 + block_linear(W, xms, f"d{i}.{s}.qkv", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"d{i}.{s}.qs"],
+                                    k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=seq_off)
 
         # joint attention of the double blocks straight to MXFP8: the txt / img proj GEMMs read row ranges of ONE
         # [B, L, hid] e4m3 buffer (scale chunks: L/128 per sample, the img range starts at chunk Lt/128)
@@ -293,19 +237,20 @@ class FluxExecutor(nn.Module):
         def post(i, s, xs, xms, a, mh):
             k = ("d", i, s)
             if att8 and f"d{i}.{s}.proj.q" in W:
-                m = self._lin(None, f"d{i}.{s}.proj", "gate_res", a8=A8[s], sfa_mtiles=ws["L"] // 128, out=xs, residual=xs,
-                              gate=self._mod(ws, k, 2))
+                m = block_linear(W, None, f"d{i}.{s}.proj", "gate_res", a8=A8[s], sfa_mtiles=ws["L"] // 128, out=xs,
+                                 residual=xs, gate=self._mod(ws, k, 2))
             else:
-                m = self._lin(a, f"d{i}.{s}.proj", "gate_res", out=xs, residual=xs, gate=self._mod(ws, k, 2))
+                m = block_linear(W, a, f"d{i}.{s}.proj", "gate_res", out=xs, residual=xs, gate=self._mod(ws, k, 2))
             if fused8 and f"d{i}.{s}.mlp0.q" in W and f"d{i}.{s}.mlp2.q" in W:
                 a8 = ln8(xs, s, self._mod(ws, k, 4), self._mod(ws, k, 3))
                 m8 = (ws["MH8I"], ws["MH8I_SF"]) if s == "img" else (ws["MH8T"], ws["MH8T_SF"])
-                m += self._lin(None, f"d{i}.{s}.mlp0", "gelu", a8=a8, out8=m8[0], sf8=m8[1])   # GELU + MX quantisation
-                m += self._lin(None, f"d{i}.{s}.mlp2", "gate_res", a8=m8, out=xs, residual=xs, gate=self._mod(ws, k, 5))
+                m += block_linear(W, None, f"d{i}.{s}.mlp0", "gelu", a8=a8, out8=m8[0], sf8=m8[1])  # GELU + MX quant.
+                m += block_linear(W, None, f"d{i}.{s}.mlp2", "gate_res", a8=m8, out=xs, residual=xs,
+                                  gate=self._mod(ws, k, 5))
                 return m + 1
             ops.layernorm_modulate(xs, xms, scale=self._mod(ws, k, 4), shift=self._mod(ws, k, 3))
-            m += self._lin(xms, f"d{i}.{s}.mlp0", "gelu", out=mh)
-            m += self._lin(mh, f"d{i}.{s}.mlp2", "gate_res", out=xs, residual=xs, gate=self._mod(ws, k, 5))
+            m += block_linear(W, xms, f"d{i}.{s}.mlp0", "gelu", out=mh)
+            m += block_linear(W, mh, f"d{i}.{s}.mlp2", "gate_res", out=xs, residual=xs, gate=self._mod(ws, k, 5))
             return m + 1
 
         def both(f_img, f_txt):
@@ -343,116 +288,68 @@ class FluxExecutor(nn.Module):
                 # linear2's A operand [attention | GELU(mlp)] is written as MXFP8 by its two producers
                 c8 = (ws["CAT8"], ws["CAT8_SF"])
                 a8 = ln8(X, "all", self._mod(ws, k, 1), self._mod(ws, k, 0))
-                n += self._lin(None, f"s{i}.l1", "qkv_rope", a8=a8, q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"],
-                               k_scale=W[f"s{i}.ks"], rope=ROPE, seq_off=0, out8=c8[0], sf8=c8[1], out8_col_off=hid)
+                n += block_linear(W, None, f"s{i}.l1", "qkv_rope", a8=a8, q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"],
+                                  k_scale=W[f"s{i}.ks"], rope=ROPE, seq_off=0, out8=c8[0], sf8=c8[1], out8_col_off=hid)
                 C.attention_fp8out(Q, K, V, c8[0], c8[1], 128 ** -0.5)
-                n += self._lin(None, f"s{i}.l2", "gate_res", a8=c8, out=X, residual=X, gate=self._mod(ws, k, 2))
+                n += block_linear(W, None, f"s{i}.l2", "gate_res", a8=c8, out=X, residual=X, gate=self._mod(ws, k, 2))
                 n += 2
                 continue
             ops.layernorm_modulate(X, XM, scale=self._mod(ws, k, 1), shift=self._mod(ws, k, 0))
-            n += self._lin(XM, f"s{i}.l1", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"], k_scale=W[f"s{i}.ks"],
-                           rope=ROPE, seq_off=0, out=CAT, mlp_col_off=hid)
+            n += block_linear(W, XM, f"s{i}.l1", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"], k_scale=W[f"s{i}.ks"],
+                              rope=ROPE, seq_off=0, out=CAT, mlp_col_off=hid)
             ops.attention(Q, K, V, out=ATT)
-            n += self._lin(CAT, f"s{i}.l2", "gate_res", out=X, residual=X, gate=self._mod(ws, k, 2))
+            n += block_linear(W, CAT, f"s{i}.l2", "gate_res", out=X, residual=X, gate=self._mod(ws, k, 2))
             n += 2
         # ---- final layer: AdaLN + Linear + unpatchify (+ Euler update, + peer store)
         k = ("final",)
         ops.layernorm_modulate(Xi, XMi, scale=self._mod(ws, k, 1), shift=self._mod(ws, k, 0))
-        kw = dict(bias=W["final.b"], C=self.params.out_channels // 4, Hl=ws["H"], Wl=ws["Wd"],
-                  xout_sample_off=out_sample_off)
-        if out_ptr is not None:
-            kw["x_out_ptr"] = out_ptr
-        else:
-            kw["x_out"] = out
-        if sigmas is not None:
-            kw["sigmas"], kw["x_in"] = sigmas, x_in
-        ops.gemm(XMi, W["final.w"], "euler_unpatch", **kw)
+        head_gather(XMi, W["final.w"], W["final.b"], self.params.out_channels // 4, ws["H"], ws["Wd"], out=out,
+                    out_ptr=out_ptr, out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas)
         n += 2
         self.launches_per_step = n
         return out
 
     # ------------------------------------------------------------------ public entry points
-    def _prep(self, x, timesteps, context, y, guidance):
-        d = self.device
-        B = x.shape[0]
-        bf = lambda t: t.to(device=d, dtype=torch.bfloat16).contiguous()  # noqa: E731
-        x, context = bf(x), bf(context)
-        timesteps = bf(timesteps)
+    def _inputs(self, B: int, timesteps, context, y, guidance) -> tuple:
+        timesteps, context = super()._inputs(B, timesteps, context)
+        p, d = self.params, self.device
         if y is None:
-            y = torch.zeros(B, self.params.vec_in_dim, device=d, dtype=torch.bfloat16)
-        y = bf(y[:, :self.params.vec_in_dim])
-        if self.params.guidance_embed:
+            y = torch.zeros(B, p.vec_in_dim, device=d, dtype=torch.bfloat16)
+        y = y[:, :p.vec_in_dim].to(device=d, dtype=torch.bfloat16).contiguous()
+        if p.guidance_embed:
             if guidance is None:
                 raise ValueError("guidance-distilled model needs a guidance strength")
-            guidance = bf(guidance)
-        return x, timesteps, context, y, guidance
+            guidance = guidance.to(device=d, dtype=torch.bfloat16).contiguous()
+        return timesteps, context, y, guidance
+
+    def _prep(self, x, timesteps, context, y, guidance):
+        x = x.to(device=self.device, dtype=torch.bfloat16).contiguous()
+        return (x,) + self._inputs(x.shape[0], timesteps, context, y, guidance)
 
     @torch.no_grad()
     def forward(self, x, timesteps, context=None, y=None, guidance=None, control=None, transformer_options=None,
                 **kwargs):
         """Same contract as ``models.flux.Flux.forward``: returns the velocity [B, 16, H, W]."""
-        with torch.cuda.device(self.device):
-            x, timesteps, context, y, guidance = self._prep(x, timesteps, context, y, guidance)
-            ws = self.workspace(x.shape[0], x.shape[2], x.shape[3], context.shape[1])
-            out = torch.empty_like(x)
-            self._run(ws, x.data_ptr(), timesteps, context, y, guidance, out)
-            return out
-
-    def _shard_args(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, y, guidance):
-        B = shape[0]
-        dummy = torch.empty(0, device=self.device)
-        _, timesteps, context, y, guidance = self._prep(dummy.new_empty((B, 1, 1, 1), dtype=torch.bfloat16),
-                                                         timesteps, context, y, guidance)
-        key = ("shard", tuple(shape), x_src_ptr, timesteps.data_ptr(), context.data_ptr(), tuple(context.shape),
-               y.data_ptr(), guidance.data_ptr() if guidance is not None else 0, out_ptr, out_sample_off)
-        return key, timesteps, context, y, guidance
+        return self._forward(x, timesteps, context, y, guidance)
 
     @torch.no_grad()
     def forward_shard(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, y=None,
                       guidance=None, **_ignored):
-        """In-process multi-GPU path: pull this replica's latent shard from the lead GPU's tensor (peer
-        pointer) inside the first kernel and store the velocity rows straight into the lead's output.
-        The engine stages every tensor argument into fixed device buffers, so the key (= all baked pointers) repeats
-        from step to step and the step replays as one CUDA graph."""
-        with torch.cuda.device(self.device):
-            key, timesteps, context, y, guidance = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr,
-                                                                     out_sample_off, y, guidance)
-            ws = self.workspace(shape[0], shape[2], shape[3], context.shape[1])
-            self._graphs.run(key, lambda: self._run(ws, x_src_ptr, timesteps, context, y, guidance, None,
-                                                    out_ptr=out_ptr, out_sample_off=out_sample_off))
+        """``DiTExecutor.forward_shard`` with the pooled text vector ``y`` and the guidance strength."""
+        self._forward_shard(x_src_ptr, shape, out_ptr, out_sample_off, timesteps, context, y, guidance)
 
     def shard_graph_handle(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, y=None,
                            guidance=None, **_ignored) -> int:
-        """``cudaGraphExec_t`` of the captured step for exactly these buffers (0 = not captured yet): lets the engine
-        hand the replay to a native host thread instead of calling ``forward_shard`` from Python."""
-        with torch.cuda.device(self.device):
-            key = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off, y, guidance)[0]
-        return self._graphs.exec_handle(key)
+        return self._graph_handle(x_src_ptr, shape, out_ptr, out_sample_off, timesteps, context, y, guidance)
 
     @torch.no_grad()
     def denoise_step(self, x, timesteps, context, y, guidance, sigmas, out=None, out_ptr=None, out_sample_off=0,
                      x_src_ptr: Optional[int] = None, t_src_ptr: Optional[int] = None,
                      g_src_ptr: Optional[int] = None):
-        """Model forward + Euler update ``x + (sigma_next - sigma) * v`` fused into the last GEMM's
-        epilogue; the result may be stored straight into a peer GPU's buffer (``out_ptr``).
-        ``x_src_ptr`` / ``t_src_ptr`` / ``g_src_ptr`` let the first kernel pull the latent shard and the
-        per-sample scalars from a peer mapping (then ``x`` is filled with a local copy as a side effect)."""
-        with torch.cuda.device(self.device):
-            ws = self.workspace(x.shape[0], x.shape[2], x.shape[3], context.shape[1])
-            if out is None and out_ptr is None:
-                out = ws["OUT"]
-
-            def body():
-                self._run(ws, x_src_ptr if x_src_ptr is not None else x.data_ptr(), timesteps, context, y, guidance,
-                          out, x_in=x, sigmas=sigmas, out_ptr=out_ptr, out_sample_off=out_sample_off, t_ptr=t_src_ptr,
-                          g_ptr=g_src_ptr, x_copy=x if (x_src_ptr is not None and self.fused_embed) else None)
-
-            key = (tuple(x.shape), x.data_ptr(), timesteps.data_ptr(), context.data_ptr(), tuple(context.shape),
-                   y.data_ptr(), guidance.data_ptr() if guidance is not None else 0, sigmas.data_ptr(),
-                   out.data_ptr() if out is not None else 0, out_ptr or 0, out_sample_off, x_src_ptr or 0,
-                   t_src_ptr or 0, g_src_ptr or 0)
-            self._graphs.run(key, body)
-            return out
+        """``DiTExecutor.denoise_step``; ``g_src_ptr`` lets the first kernel pull the guidance strength from a peer
+        mapping as well."""
+        return self._denoise(x, (timesteps, context, y, guidance), sigmas, out, out_ptr, out_sample_off, x_src_ptr,
+                             t_src_ptr, g_ptr=g_src_ptr)
 
 
 def build_flux_executor(model: nn.Module, device, **kw) -> FluxExecutor:

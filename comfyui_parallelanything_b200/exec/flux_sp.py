@@ -23,8 +23,9 @@ from typing import List, Optional
 import torch
 
 from .. import ops
-from ..models import flux as flux_model
-from .sp_common import UlyssesBase
+from . import block_linear
+from .dit import head_gather
+from .sp_common import UlyssesBase, attention_variant
 
 
 def supported(executors) -> Optional[str]:
@@ -140,11 +141,7 @@ class FluxUlysses(UlyssesBase):
             ws["T1"], ws["T2"] = e(1, 256), e(1, 256)
             ws["HC"] = e(1, ex.W["vec_out.w"].shape[1])
             ws["SVEC"], ws["MOD"] = e(1, hid), e(1, ex.mod_total)
-            m = flux_model.Flux.__new__(flux_model.Flux)
-            m.patch_size = 2
-            ids = flux_model.Flux.make_ids(m, 1, H, Wd, Lt, d)
-            pe = flux_model.EmbedND(128, ex.params.theta, ex.params.axes_dim)(ids)
-            ws["ROPE"] = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float().contiguous()
+            ws["ROPE"] = ex.rope(H, Wd, Lt)
             wss.append(ws)
         # descriptor tables (static addresses -> built once, baked into the graphs)
         ptrs = [{k: ws[k].data_ptr() for k in ("Q", "K", "V", "QF", "KF", "VF", "ATTF", "CAT")} for ws in wss]
@@ -187,25 +184,16 @@ class FluxUlysses(UlyssesBase):
             nl += 2
         ops.gemm(y, W["vector_in.in.w"], "silu", out=HC[:, col:col + hid], bias=W["vector_in.in.b"])
         ops.gemm(HC, W["vec_out.w"], "silu", out=ws["SVEC"], bias=W["vec_out.b"])
-        nl += 2 + ex._lin(ws["SVEC"], "mod", "bias", out=ws["MOD"])
+        nl += 2 + block_linear(W, ws["SVEC"], "mod", "bias", out=ws["MOD"])
 
-        def mod(key, idx):
-            off = ex.mod_off[key] + idx * hid
-            return ws["MOD"][:, off:off + hid]
-
-        def lin(a, name, mode, **kw):
-            return ex._lin(a, name, mode, **kw)
-
-        # few heads per GPU: the ping-pong kernel (two 128-row query tiles per CTA) would leave most SMs idle - with fewer
-        # than ~3/4 of a wave, the one-tile-per-CTA kernel doubles the CTA count and halves the attention latency
-        att_variant = 1 if hpg * ((ws["L"] + 255) // 256) < 110 else None
+        att_variant = attention_variant(hpg, ws["L"])
         slot = 0
         for i in range(ex.n_double):
             for s, xs, xms, off, ro in (("img", Xi, XMi, Ltl, ro_i), ("txt", Xt, XMt, 0, ro_t)):
                 k = ("d", i, s)
-                ops.layernorm_modulate(xs, xms, scale=mod(k, 1), shift=mod(k, 0))
-                nl += 1 + lin(xms, f"d{i}.{s}.qkv", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"d{i}.{s}.qs"],
-                              k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=off, rope_off=ro)
+                ops.layernorm_modulate(xs, xms, scale=ex._mod(ws, k, 1), shift=ex._mod(ws, k, 0))
+                nl += 1 + block_linear(W, xms, f"d{i}.{s}.qkv", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"d{i}.{s}.qs"],
+                                       k_scale=W[f"d{i}.{s}.ks"], rope=ROPE, seq_off=off, rope_off=ro)
             self._exchange(g, ws, slot, "QKV")                      # all heads / my tokens -> my heads / all tokens
             ops.attention(ws["QF"], ws["KF"], ws["VF"], out=ws["ATTF"], variant=att_variant)
             self._exchange(g, ws, slot + 1, "ATT")                  # my heads / all tokens -> all heads / my tokens
@@ -213,26 +201,27 @@ class FluxUlysses(UlyssesBase):
             nl += 5
             for s, xs, xms, a, mh in (("img", Xi, XMi, ATT[:, Ltl:], MH[:, Ltl:]), ("txt", Xt, XMt, ATT[:, :Ltl], MH[:, :Ltl])):
                 k = ("d", i, s)
-                nl += lin(a, f"d{i}.{s}.proj", "gate_res", out=xs, residual=xs, gate=mod(k, 2))
-                ops.layernorm_modulate(xs, xms, scale=mod(k, 4), shift=mod(k, 3))
-                nl += lin(xms, f"d{i}.{s}.mlp0", "gelu", out=mh)
-                nl += lin(mh, f"d{i}.{s}.mlp2", "gate_res", out=xs, residual=xs, gate=mod(k, 5))
+                nl += block_linear(W, a, f"d{i}.{s}.proj", "gate_res", out=xs, residual=xs, gate=ex._mod(ws, k, 2))
+                ops.layernorm_modulate(xs, xms, scale=ex._mod(ws, k, 4), shift=ex._mod(ws, k, 3))
+                nl += block_linear(W, xms, f"d{i}.{s}.mlp0", "gelu", out=mh)
+                nl += block_linear(W, mh, f"d{i}.{s}.mlp2", "gate_res", out=xs, residual=xs, gate=ex._mod(ws, k, 5))
                 nl += 1
         for i in range(ex.n_single):
             k = ("s", i)
-            ops.layernorm_modulate(X, XM, scale=mod(k, 1), shift=mod(k, 0))
-            nl += 1 + lin(XM, f"s{i}.l1", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"], k_scale=W[f"s{i}.ks"],
-                          rope=ROPE, seq_off=0, rope_off=ro_t, rope_off2=ro_i, seg_rows=Ltl, out=CAT, mlp_col_off=hid)
+            ops.layernorm_modulate(X, XM, scale=ex._mod(ws, k, 1), shift=ex._mod(ws, k, 0))
+            nl += 1 + block_linear(W, XM, f"s{i}.l1", "qkv_rope", q=Q, k=K, v=V, q_scale=W[f"s{i}.qs"],
+                                   k_scale=W[f"s{i}.ks"], rope=ROPE, seq_off=0, rope_off=ro_t, rope_off2=ro_i,
+                                   seg_rows=Ltl, out=CAT, mlp_col_off=hid)
             self._exchange(g, ws, slot, "QKV")
             ops.attention(ws["QF"], ws["KF"], ws["VF"], out=ws["ATTF"], variant=att_variant)
             self._exchange(g, ws, slot + 1, "ATT")
             slot += 2
-            nl += 5 + lin(CAT, f"s{i}.l2", "gate_res", out=X, residual=X, gate=mod(k, 2))
+            nl += 5 + block_linear(W, CAT, f"s{i}.l2", "gate_res", out=X, residual=X, gate=ex._mod(ws, k, 2))
         # ---- final layer on my image tokens: AdaLN + Linear + unpatchify, rows stored into the LEAD GPU's output
         k = ("final",)
-        ops.layernorm_modulate(Xi, XMi, scale=mod(k, 1), shift=mod(k, 0))
-        ops.gemm(XMi, W["final.w"], "euler_unpatch", bias=W["final.b"], C=p.out_channels // 4, Hl=ws["H"], Wl=ws["Wd"],
-                 xout_sample_off=0, x_out_ptr=out_ptr, tok_off=g * Lil)
+        ops.layernorm_modulate(Xi, XMi, scale=ex._mod(ws, k, 1), shift=ex._mod(ws, k, 0))
+        head_gather(XMi, W["final.w"], W["final.b"], p.out_channels // 4, ws["H"], ws["Wd"], out_ptr=out_ptr,
+                    tok_off=g * Lil)
         # (no closing handshake: the engine orders the lead's staging-buffer rewrite after every GPU's stream, and a GPU
         # cannot run ahead into the next step's first exchange before all peers signalled it)
         self._end_step(g)

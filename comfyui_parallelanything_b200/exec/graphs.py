@@ -71,22 +71,7 @@ class GraphCache:
         engine therefore captures all GPUs' graphs first, from one thread, and only then launches them."""
         if not self.enabled or self._graphs.get(key) != _SEEN:
             return self.captured(key) is not None
-        with _CAPTURE_LOCK:
-            torch.cuda.synchronize(self.device)
-            graph = torch.cuda.CUDAGraph()
-            if self._stream is None:
-                self._stream = torch.cuda.Stream(device=self.device)
-            try:
-                with torch.cuda.graph(graph, stream=self._stream, capture_error_mode="thread_local"):
-                    body()
-            except Exception as e:
-                log.warn("CUDA graph capture failed on %s (%s); staying eager for this shape", self.device, e)
-                torch.cuda.synchronize(self.device)
-                self._graphs[key] = _EAGER
-                return False
-        self._graphs[key] = graph
-        self.captures += 1
-        return True
+        return self._capture(key, body, eager_on_failure=False)
 
     def replay(self, key) -> None:
         g = self.captured(key)
@@ -106,14 +91,17 @@ class GraphCache:
                 self._graphs = {k: v for k, v in self._graphs.items() if v != _SEEN}
             self._graphs[key] = _SEEN
         elif g == _SEEN:
-            self._capture(key, body)
+            if self._capture(key, body, eager_on_failure=True):
+                self.replay(key)
         elif g == _EAGER:
             body()
         else:
             g.replay()
             self.replays += 1
 
-    def _capture(self, key, body) -> None:
+    def _capture(self, key, body: Callable[[], None], eager_on_failure: bool) -> bool:
+        """Record ``body`` as the graph of ``key``.  A failed capture pins the key to eager and returns False, after
+        running ``body`` eagerly once if ``eager_on_failure`` (never lose a step to a failed capture)."""
         # "thread_local" keeps other threads' CUDA calls legal while we record (the in-process engine drives one
         # executor per GPU from its own thread); the lock serialises captures, whose prologue synchronises.
         with _CAPTURE_LOCK:
@@ -124,13 +112,13 @@ class GraphCache:
             try:
                 with torch.cuda.graph(graph, stream=self._stream, capture_error_mode="thread_local"):
                     body()
-            except Exception as e:                      # never lose a step to a failed capture
+            except Exception as e:
                 log.warn("CUDA graph capture failed on %s (%s); staying eager for this shape", self.device, e)
                 torch.cuda.synchronize(self.device)
                 self._graphs[key] = _EAGER
-                body()
-                return
+                if eager_on_failure:
+                    body()
+                return False
         self._graphs[key] = graph
         self.captures += 1
-        graph.replay()
-        self.replays += 1
+        return True

@@ -18,6 +18,13 @@ import torch
 from .. import ops
 
 
+def attention_variant(hpg: int, L: int) -> Optional[int]:
+    """Attention kernel for ``hpg`` heads per GPU over ``L`` tokens.  With few heads the ping-pong kernel (two 128-row
+    query tiles per CTA) would leave most SMs idle: below ~3/4 of a wave, the one-tile-per-CTA kernel (variant 1)
+    doubles the CTA count and halves the attention latency.  None: the default kernel."""
+    return 1 if hpg * ((L + 255) // 256) < 110 else None
+
+
 class UlyssesBase:
     family = "?"
 

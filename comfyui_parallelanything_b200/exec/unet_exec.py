@@ -23,12 +23,8 @@ import torch
 import torch.nn as nn
 
 from .. import ops
-from . import recognize
+from . import bf16 as _bf, conditioning_sig, recognize
 from .graphs import GraphCache
-
-
-def _bf(t: torch.Tensor, d) -> torch.Tensor:
-    return t.detach().to(device=d, dtype=torch.bfloat16).contiguous()
 
 
 def _pad32(t: torch.Tensor) -> torch.Tensor:
@@ -122,7 +118,7 @@ class _TBlock:
         """K/V projections of the conditioning depend only on ``ctx``: computed once per sampling run, EAGERLY (never
         inside the per-step CUDA graph, which reads the persistent ``_kv`` buffer; SURVEY K3 - the reference
         re-sends and re-projects the constant conditioning every step).  Returns the number of launches."""
-        sig = (ctx.data_ptr(), tuple(ctx.shape), ctx._version)
+        sig = conditioning_sig(ctx)
         if self._kv_sig == sig:
             return 0
         inner = self.wkv2.shape[0] // 2
@@ -259,7 +255,7 @@ class UNetExecutor(nn.Module):
         return sum(tb.prepare_ctx(ctx) for tb in self._tblocks)
 
     def _ctx_ready(self, ctx) -> bool:
-        sig = (ctx.data_ptr(), tuple(ctx.shape), ctx._version)
+        sig = conditioning_sig(ctx)
         return all(tb._kv_sig == sig for tb in self._tblocks)
 
     def release(self) -> None:

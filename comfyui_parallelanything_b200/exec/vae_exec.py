@@ -16,7 +16,8 @@ import torch.nn as nn
 
 from .. import ops
 from ..models import vae as vae_model
-from .unet_exec import _Conv, _GN, _bf
+from . import bf16 as _bf
+from .unet_exec import _Conv, _GN
 
 
 class _VRes:

@@ -15,31 +15,24 @@ LayerNorm kernel) plus what WAN needs on top:
 """
 from __future__ import annotations
 
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional
 
 import torch
 import torch.nn as nn
 
 from .. import ops
-from . import block_linear, cache_workspace, quantize_block_weights, recognize, touch_workspace
-from .graphs import GraphCache
+from . import bf16 as _bf, block_linear, conditioning_sig, quantize_block_weights, recognize
+from .dit import DiTExecutor, head_gather, rope_layout
 from ..models import flux as flux_model
 from ..models import wan as wan_model
 
 
-def _bf(t: torch.Tensor, d) -> torch.Tensor:
-    return t.detach().to(device=d, dtype=torch.bfloat16).contiguous()
-
-
-class WanExecutor(nn.Module):
+class WanExecutor(DiTExecutor):
     pa_family = "wan"
-    pa_native = True
 
     def __init__(self, model: "wan_model.WanModel", device, cuda_graphs: bool = False, fp8: bool = False):
-        super().__init__()
-        ops.require()
-        d = self.device = torch.device(device)
-        p = self.params = recognize.params_of(model, "wan")      # from weight shapes / ComfyUI attribute names
+        super().__init__(model, device, cuda_graphs)
+        d, p = self.device, self.params
         self.dim, self.heads = p.dim, p.num_heads
         if p.dim // p.num_heads != 128 or tuple(p.patch_size) != (1, 2, 2) or p.in_dim != 16:
             raise ValueError("WanExecutor is specialised for head_dim 128, patch (1,2,2), 16 latent channels")
@@ -91,28 +84,14 @@ class WanExecutor(nn.Module):
             quantize_block_weights(W, names, lambda _n: 224)
             torch.cuda.empty_cache()
         self.eps = p.eps
-        self._ws: Dict[Tuple, dict] = {}
-        self._graphs = GraphCache(self.device, enabled=cuda_graphs)
-        self.launches_per_step = 0
 
-    def parameters(self, recurse: bool = True):  # type: ignore[override]
-        return iter(())
+    def rope(self, T: int, H: int, Wd: int) -> torch.Tensor:
+        """fp32 [T*(H/2)*(W/2), 64, 2] RoPE table of the clip's tokens (frame, row, column)."""
+        ids = wan_model.WanModel.make_ids(1, T, H // 2, Wd // 2, self.device)
+        dd = 128
+        return rope_layout(flux_model.EmbedND(dd, 10000, [dd - 4 * (dd // 6), 2 * (dd // 6), 2 * (dd // 6)])(ids))
 
-    def invalidate_conditioning(self) -> None:
-        """Forget the cached text embedding / cross-attention K/V (call when the prompt changes in place)."""
-        for ws in self._ws.values():
-            ws["ctx_sig"] = None
-
-    def release(self) -> None:
-        self.W.clear()
-        self._ws.clear()
-        self._graphs.clear()
-
-    def workspace(self, B: int, T: int, H: int, Wd: int, Lc: int) -> dict:
-        key = (B, T, H, Wd, Lc)
-        ws = touch_workspace(self._ws, key)
-        if ws is not None:
-            return ws
+    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int) -> dict:
         d, dim = self.device, self.dim
         L = T * (H // 2) * (Wd // 2)
         e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=d)  # noqa: E731
@@ -129,13 +108,8 @@ class WanExecutor(nn.Module):
         ws["CQ"] = e(B, L, dim)
         ws["CKV"] = [e(B, Lc, 2 * dim) for _ in range(self.n_blocks)]
         ws["OUT"] = e(B, self.params.out_dim, T, H, Wd)
-        m = wan_model.WanModel.__new__(wan_model.WanModel)
-        ids = wan_model.WanModel.make_ids(m, 1, T, H // 2, Wd // 2, d)
-        dd = 128
-        pe = flux_model.EmbedND(dd, 10000, [dd - 4 * (dd // 6), 2 * (dd // 6), 2 * (dd // 6)])(ids)
-        ws["ROPE"] = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float().contiguous()
+        ws["ROPE"] = self.rope(T, H, Wd)
         ws["ctx_sig"] = None
-        cache_workspace(self._ws, key, ws, device=self.device, on_evict=lambda _k: self._graphs.clear())
         return ws
 
     def _heads(self, t: torch.Tensor, which: int, n: int) -> torch.Tensor:
@@ -148,7 +122,7 @@ class WanExecutor(nn.Module):
         they run EAGERLY and only when the conditioning changed (tensor identity / version, or after
         ``invalidate_conditioning``) - never inside the per-step CUDA graph, which reads the results from the
         workspace's fixed ``CKV`` buffers (SURVEY K3: the reference re-sends constant conditioning every step)."""
-        sig = (ctx.data_ptr(), tuple(ctx.shape), ctx._version)
+        sig = conditioning_sig(ctx)
         if ws["ctx_sig"] == sig:
             return 0
         W, dim = self.W, self.dim
@@ -186,99 +160,34 @@ class WanExecutor(nn.Module):
         for i in range(self.n_blocks):
             # ---- self attention
             ops.layernorm_modulate(X, XM, scale=mod(i, 1), shift=mod(i, 0), eps=self.eps)
-            block_linear(W, XM, f"b{i}.qkv", "bias", out=QKV)
+            n += block_linear(W, XM, f"b{i}.qkv", "bias", out=QKV)
             C.rms_rope(QKV[:, :, :dim], W[f"b{i}.nq"], ROPE, self.eps)
             C.rms_rope(QKV[:, :, dim:2 * dim], W[f"b{i}.nk"], ROPE, self.eps)
             ops.attention(self._heads(QKV, 0, 3), self._heads(QKV, 1, 3), self._heads(QKV, 2, 3), out=ATT)
-            block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2))
+            n += block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2))
             # ---- text cross attention
             ops.layernorm_modulate(X, XM, gamma=W[f"b{i}.n3.g"], beta=W[f"b{i}.n3.b"], eps=self.eps)
-            block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
+            n += block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
             C.rms_rope(ws["CQ"], W[f"b{i}.cnq"], None, self.eps)
             ops.attention(self._heads(ws["CQ"], 0, 1), self._heads(ws["CKV"][i], 0, 2), self._heads(ws["CKV"][i], 1, 2),
                           out=ATT)
-            block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
+            n += block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
             # ---- FFN
             ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=self.eps)
-            block_linear(W, XM, f"b{i}.f0", "gelu", out=FF)
-            block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5))
-            n += 14
+            n += block_linear(W, XM, f"b{i}.f0", "gelu", out=FF)
+            n += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5))
+            n += 8
         # ---- head: AdaLN + Linear + unpatchify (+ Euler, + peer store)
         ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=self.eps)
-        kw = dict(bias=W["head.b"], C=self.params.out_dim, Hl=TH, Wl=ws["Wd"], xout_sample_off=out_sample_off)
-        if out_ptr is not None:
-            kw["x_out_ptr"] = out_ptr
-        else:
-            kw["x_out"] = out
-        if sigmas is not None:
-            kw["sigmas"], kw["x_in"] = sigmas, x_in
-        ops.gemm(XM, W["head.w"], "euler_unpatch", **kw)
+        head_gather(XM, W["head.w"], W["head.b"], self.params.out_dim, TH, ws["Wd"], out=out, out_ptr=out_ptr,
+                    out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas)
         n += 2
         self.launches_per_step = n
         return out
 
-    def _prep(self, x, timesteps, context):
-        d = self.device
-        bf = lambda t: t.to(device=d, dtype=torch.bfloat16).contiguous()  # noqa: E731
-        return bf(x), bf(timesteps), bf(context)
-
     @torch.no_grad()
     def forward(self, x, timesteps, context=None, clip_fea=None, transformer_options=None, **kwargs):
-        with torch.cuda.device(self.device):
-            x, timesteps, context = self._prep(x, timesteps, context)
-            B, _, T, H, Wd = x.shape
-            ws = self.workspace(B, T, H, Wd, context.shape[1])
-            out = torch.empty_like(x)
-            self._prepare_ctx(ws, context)
-            self._run(ws, x.data_ptr(), timesteps, context, out)
-            return out
-
-    def _shard_args(self, x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off):
-        d = self.device
-        timesteps = timesteps.to(device=d, dtype=torch.bfloat16).contiguous()
-        context = context.to(device=d, dtype=torch.bfloat16).contiguous()
-        key = ("shard", tuple(shape), x_src_ptr, timesteps.data_ptr(), context.data_ptr(), tuple(context.shape), out_ptr,
-               out_sample_off)
-        return key, timesteps, context
-
-    @torch.no_grad()
-    def forward_shard(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, **_ignored):
-        with torch.cuda.device(self.device):
-            key, timesteps, context = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off)
-            ws = self.workspace(shape[0], shape[2], shape[3], shape[4], context.shape[1])
-            self._prepare_ctx(ws, context)
-            self._graphs.run(key, lambda: self._run(ws, x_src_ptr, timesteps, context, None, out_ptr=out_ptr,
-                                                    out_sample_off=out_sample_off))
-
-    def shard_graph_handle(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int,
-                           **_ignored) -> int:
-        with torch.cuda.device(self.device):
-            key, _t, context = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off)
-            ws = self.workspace(shape[0], shape[2], shape[3], shape[4], context.shape[1])
-            if ws["ctx_sig"] != (context.data_ptr(), tuple(context.shape), context._version):
-                return 0                    # conditioning changed: take the Python path once (eager K/V precompute)
-        return self._graphs.exec_handle(key)
-
-    @torch.no_grad()
-    def denoise_step(self, x, timesteps, context, sigmas, out=None, out_ptr=None, out_sample_off=0,
-                     x_src_ptr: Optional[int] = None, t_src_ptr: Optional[int] = None):
-        with torch.cuda.device(self.device):
-            B, _, T, H, Wd = x.shape
-            ws = self.workspace(B, T, H, Wd, context.shape[1])
-            if out is None and out_ptr is None:
-                out = ws["OUT"]
-            self._prepare_ctx(ws, context)
-
-            def body():
-                self._run(ws, x_src_ptr if x_src_ptr is not None else x.data_ptr(), timesteps, context, out, x_in=x,
-                          sigmas=sigmas, out_ptr=out_ptr, out_sample_off=out_sample_off, t_ptr=t_src_ptr,
-                          x_copy=x if x_src_ptr is not None else None)
-
-            key = (tuple(x.shape), x.data_ptr(), timesteps.data_ptr(), context.data_ptr(), tuple(context.shape),
-                   sigmas.data_ptr(), out.data_ptr() if out is not None else 0, out_ptr or 0, out_sample_off,
-                   x_src_ptr or 0, t_src_ptr or 0)
-            self._graphs.run(key, body)
-            return out
+        return self._forward(x, timesteps, context)
 
 
 def build_wan_executor(model: nn.Module, device, **kw) -> WanExecutor:

@@ -21,10 +21,9 @@ from typing import List, Optional
 import torch
 
 from .. import ops
-from ..models import flux as flux_model
-from ..models import wan as wan_model
 from . import block_linear
-from .sp_common import UlyssesBase
+from .dit import head_gather
+from .sp_common import UlyssesBase, attention_variant
 
 
 def supported(executors) -> Optional[str]:
@@ -113,12 +112,7 @@ class WanUlysses(UlyssesBase):
             ws["CTX_H"], ws["CTX"] = e(1, Lc, dim), e(1, Lc, dim)
             ws["CQ"] = e(1, Ll, dim)
             ws["CKV"] = [e(1, Lc, 2 * dim) for _ in range(ex.n_blocks)]
-            m = wan_model.WanModel.__new__(wan_model.WanModel)
-            ids = wan_model.WanModel.make_ids(m, 1, T, H // 2, Wd // 2, d)
-            dd = 128
-            pe = flux_model.EmbedND(dd, 10000, [dd - 4 * (dd // 6), 2 * (dd // 6), 2 * (dd // 6)])(ids)
-            rope = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float()
-            ws["ROPE"] = rope[g * Ll:(g + 1) * Ll].contiguous()       # RoPE rows of MY tokens
+            ws["ROPE"] = ex.rope(T, H, Wd)[g * Ll:(g + 1) * Ll].contiguous()       # RoPE rows of MY tokens
             ws["ctx_sig"] = None
             wss.append(ws)
         ptrs = [{k: ws[k].data_ptr() for k in ("QKV", "QF", "KF", "VF", "ATTF", "ATT")} for ws in wss]
@@ -161,7 +155,7 @@ class WanUlysses(UlyssesBase):
         def heads_of(tk: torch.Tensor, nh: int) -> torch.Tensor:      # token-major [1, rows, nh*128] -> [1, nh, rows, 128] view
             return tk.view(1, tk.shape[1], nh, 128).permute(0, 2, 1, 3)
 
-        att_variant = 1 if hpg * ((L + 255) // 256) < 110 else None
+        att_variant = attention_variant(hpg, L)
         slot = 0
         for i in range(ex.n_blocks):
             # ---- self attention: token-sliced QKV + q/k norm + RoPE, head-sliced attention between two exchanges
@@ -187,8 +181,7 @@ class WanUlysses(UlyssesBase):
             nl += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5))
         # ---- head on my tokens: AdaLN + Linear + unpatchify, rows stored into the LEAD GPU's output
         ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=ex.eps)
-        ops.gemm(XM, W["head.w"], "euler_unpatch", bias=W["head.b"], C=ex.params.out_dim, Hl=TH, Wl=ws["Wd"],
-                 xout_sample_off=0, x_out_ptr=out_ptr, tok_off=g * Ll)
+        head_gather(XM, W["head.w"], W["head.b"], ex.params.out_dim, TH, ws["Wd"], out_ptr=out_ptr, tok_off=g * Ll)
         self._end_step(g)
         nl += 3
         return nl

@@ -16,31 +16,24 @@ family needs (SURVEY §2.6 "DiT attention + RoPE ... Z-Image"; the reference lis
 """
 from __future__ import annotations
 
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional
 
 import torch
 import torch.nn as nn
 
 from .. import ops
-from . import block_linear, cache_workspace, quantize_block_weights, recognize, touch_workspace
-from .graphs import GraphCache
+from . import bf16 as _bf, block_linear, conditioning_sig, quantize_block_weights, recognize
+from .dit import DiTExecutor, head_gather, rope_layout
 from ..models import flux as flux_model
 from ..models import zimage as zimage_model
 
 
-def _bf(t: torch.Tensor, d) -> torch.Tensor:
-    return t.detach().to(device=d, dtype=torch.bfloat16).contiguous()
-
-
-class ZImageExecutor(nn.Module):
+class ZImageExecutor(DiTExecutor):
     pa_family = "zimage"
-    pa_native = True
 
     def __init__(self, model: "zimage_model.ZImageModel", device, cuda_graphs: bool = False, fp8: bool = False):
-        super().__init__()
-        ops.require()
-        d = self.device = torch.device(device)
-        p = self.params = recognize.params_of(model, "zimage")   # from weight shapes / ComfyUI attribute names
+        super().__init__(model, device, cuda_graphs)
+        d, p = self.device, self.params
         self.dim, self.heads = p.dim, p.n_heads
         if p.dim // p.n_heads != 128 or p.patch_size != 2 or p.in_channels != 16:
             raise ValueError("ZImageExecutor is specialised for head_dim 128, 2x2 patches, 16 latent channels")
@@ -99,31 +92,15 @@ class ZImageExecutor(nn.Module):
         self.W = W
         self.n_cr, self.n_nr, self.n_layers = len(model.context_refiner), len(model.noise_refiner), len(model.layers)
         self.eps = p.norm_eps
-        self._ws: Dict[Tuple, dict] = {}
-        self._graphs = GraphCache(self.device, enabled=cuda_graphs)
-        self.launches_per_step = 0
 
-    def parameters(self, recurse: bool = True):  # type: ignore[override]
-        return iter(())
+    def rope(self, H: int, Wd: int, Lc: int) -> torch.Tensor:
+        """fp32 [Lc + (H/2)*(W/2), 64, 2] RoPE table of the joint [caption | image] sequence."""
+        ids = zimage_model.ZImageModel.make_ids(1, Lc, H // 2, Wd // 2, self.device)
+        return rope_layout(flux_model.EmbedND(128, self.params.rope_theta, self.params.axes_dims)(ids))
 
-    def invalidate_conditioning(self) -> None:
-        """Forget the cached caption path (call when the conditioning buffer is rewritten in place)."""
-        for ws in self._ws.values():
-            ws["ctx_sig"] = None
-
-    def release(self) -> None:
-        self.W.clear()
-        self._ws.clear()
-        self._graphs.clear()
-
-    def workspace(self, B: int, H: int, Wd: int, Lc: int) -> dict:
-        key = (B, H, Wd, Lc)
-        ws = touch_workspace(self._ws, key)
-        if ws is not None:
-            return ws
+    def _new_workspace(self, B: int, H: int, Wd: int, Lc: int) -> dict:
         d, dim, p = self.device, self.dim, self.params
-        hh, ww = H // 2, Wd // 2
-        Li = hh * ww
+        Li = (H // 2) * (Wd // 2)
         L = Lc + Li
         e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=d)  # noqa: E731
         ws = dict(B=B, H=H, Wd=Wd, Lc=Lc, Li=Li, L=L)
@@ -132,45 +109,40 @@ class ZImageExecutor(nn.Module):
         for nm, n in (("", L), ("i", Li), ("t", Lc)):
             ws["Q" + nm], ws["K" + nm], ws["V" + nm] = (e(B, self.heads, n, 128) for _ in range(3))
         ws["CAPN"], ws["XT0"] = e(B, Lc, p.cap_feat_dim), e(B, Lc, dim)
-        ws["T1"], ws["TH"], ws["TE"], ws["STE"] = e(B, 256), e(B, W_mid(self)), e(B, p.adaln_dim), e(B, p.adaln_dim)
+        ws["T1"], ws["TH"] = e(B, 256), e(B, self.W["t0.w"].shape[0])
+        ws["TE"], ws["STE"] = e(B, p.adaln_dim), e(B, p.adaln_dim)
         ws["MOD"] = e(B, self.W["mod.w"].shape[0])
         ws["OUT"] = e(B, p.in_channels, H, Wd)
-        ids = zimage_model.ZImageModel.make_ids(1, Lc, hh, ww, d)
-        pe = flux_model.EmbedND(128, p.rope_theta, p.axes_dims)(ids)                      # [1,1,L,64,2,2]
-        ws["ROPE"] = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float().contiguous()
+        ws["ROPE"] = self.rope(H, Wd, Lc)
         ws["ROPE_I"] = ws["ROPE"][Lc:].contiguous()
         ws["ctx_sig"] = None
-        cache_workspace(self._ws, key, ws, device=self.device, on_evict=lambda _k: self._graphs.clear())
         return ws
 
     # ------------------------------------------------------------------ schedule
-    def _mod(self, ws, name: str, idx: int):
-        off = self.mod_off[name] + idx * self.dim
-        return ws["MOD"][:, off:off + self.dim]
-
     def _block(self, ws, name: str, xs, xms, ys, att, ff, q, k, v, rope, modulated: bool) -> int:
         W, eps = self.W, self.eps
         sc_a = self._mod(ws, name, 0) if modulated else None
         g_a = self._mod(ws, name, 1) if modulated else None
         sc_m = self._mod(ws, name, 2) if modulated else None
         g_m = self._mod(ws, name, 3) if modulated else None
+        n = 5
         ops.rmsnorm_modulate(xs, xms, weight=W[name + ".n1"], scale=sc_a, eps=eps)
-        block_linear(W, xms, name + ".qkv", "qkv_rope", q=q, k=k, v=v, q_scale=W[name + ".qs"], k_scale=W[name + ".ks"],
-                     rope=rope, seq_off=0, qk_eps=eps)
+        n += block_linear(W, xms, name + ".qkv", "qkv_rope", q=q, k=k, v=v, q_scale=W[name + ".qs"],
+                          k_scale=W[name + ".ks"], rope=rope, seq_off=0, qk_eps=eps)
         ops.attention(q, k, v, out=att)
-        block_linear(W, att, name + ".out", "bias", out=ys)
+        n += block_linear(W, att, name + ".out", "bias", out=ys)
         ops.rmsnorm_modulate(ys, xs, weight=W[name + ".n2"], gate=g_a, residual=xs, eps=eps)
         ops.rmsnorm_modulate(xs, xms, weight=W[name + ".f1"], scale=sc_m, eps=eps)
-        block_linear(W, xms, name + ".w13", "swiglu", out=ff)
-        block_linear(W, ff, name + ".w2", "bias", out=ys)
+        n += block_linear(W, xms, name + ".w13", "swiglu", out=ff)
+        n += block_linear(W, ff, name + ".w2", "bias", out=ys)
         ops.rmsnorm_modulate(ys, xs, weight=W[name + ".f2"], gate=g_m, residual=xs, eps=eps)
-        return 9
+        return n
 
     def _prepare_ctx(self, ws, ctx) -> int:
         """Caption path (RMSNorm + Linear + ``context_refiner`` blocks): a function of the conditioning only, so it
         runs EAGERLY and only when the conditioning changed - never inside the per-step CUDA graph, which reads the
         refined caption tokens from the workspace's fixed ``XT0`` buffer."""
-        sig = (ctx.data_ptr(), tuple(ctx.shape), ctx._version)
+        sig = conditioning_sig(ctx)
         if ws["ctx_sig"] == sig:
             return 0
         W, Lc, n = self.W, ws["Lc"], 2
@@ -208,85 +180,16 @@ class ZImageExecutor(nn.Module):
             n += self._block(ws, f"l{i}", X, XM, Y, ATT, FF, ws["Q"], ws["K"], ws["V"], ws["ROPE"], True)
         # head: LayerNorm * (1 + scale) + Linear + unpatchify (+ Euler, + peer store)
         ops.layernorm_modulate(Xi, XM[:, Lc:], scale=self._mod(ws, "final", 0), eps=1e-6)
-        kw = dict(bias=W["final.b"], C=p.in_channels, Hl=ws["H"], Wl=ws["Wd"], xout_sample_off=out_sample_off)
-        if out_ptr is not None:
-            kw["x_out_ptr"] = out_ptr
-        else:
-            kw["x_out"] = out
-        if sigmas is not None:
-            kw["sigmas"], kw["x_in"] = sigmas, x_in
-        ops.gemm(XM[:, Lc:], W["final.w"], "euler_unpatch", **kw)
+        head_gather(XM[:, Lc:], W["final.w"], W["final.b"], p.in_channels, ws["H"], ws["Wd"], out=out, out_ptr=out_ptr,
+                    out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas)
         n += 2
         self.launches_per_step = n
         return out
 
-    def _prep(self, x, timesteps, context):
-        d = self.device
-        bf = lambda t: t.to(device=d, dtype=torch.bfloat16).contiguous()  # noqa: E731
-        return bf(x), bf(timesteps), bf(context)
-
     @torch.no_grad()
     def forward(self, x, timesteps, context=None, num_tokens=None, attention_mask=None, transformer_options=None,
                 **kwargs):
-        with torch.cuda.device(self.device):
-            x, timesteps, context = self._prep(x, timesteps, context)
-            B, _, H, Wd = x.shape
-            ws = self.workspace(B, H, Wd, context.shape[1])
-            out = torch.empty_like(x)
-            self._prepare_ctx(ws, context)
-            self._run(ws, x.data_ptr(), timesteps, context, out)
-            return out
-
-    def _shard_args(self, x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off):
-        d = self.device
-        timesteps = timesteps.to(device=d, dtype=torch.bfloat16).contiguous()
-        context = context.to(device=d, dtype=torch.bfloat16).contiguous()
-        key = ("shard", tuple(shape), x_src_ptr, timesteps.data_ptr(), context.data_ptr(), tuple(context.shape), out_ptr,
-               out_sample_off)
-        return key, timesteps, context
-
-    @torch.no_grad()
-    def forward_shard(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, **_ignored):
-        with torch.cuda.device(self.device):
-            key, timesteps, context = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off)
-            ws = self.workspace(shape[0], shape[2], shape[3], context.shape[1])
-            self._prepare_ctx(ws, context)
-            self._graphs.run(key, lambda: self._run(ws, x_src_ptr, timesteps, context, None, out_ptr=out_ptr,
-                                                    out_sample_off=out_sample_off))
-
-    def shard_graph_handle(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int,
-                           **_ignored) -> int:
-        with torch.cuda.device(self.device):
-            key, _t, context = self._shard_args(x_src_ptr, shape, timesteps, context, out_ptr, out_sample_off)
-            ws = self.workspace(shape[0], shape[2], shape[3], context.shape[1])
-            if ws["ctx_sig"] != (context.data_ptr(), tuple(context.shape), context._version):
-                return 0                    # conditioning changed: take the Python path once (eager caption path)
-        return self._graphs.exec_handle(key)
-
-    @torch.no_grad()
-    def denoise_step(self, x, timesteps, context, sigmas, out=None, out_ptr=None, out_sample_off=0,
-                     x_src_ptr: Optional[int] = None, t_src_ptr: Optional[int] = None):
-        with torch.cuda.device(self.device):
-            B, _, H, Wd = x.shape
-            ws = self.workspace(B, H, Wd, context.shape[1])
-            if out is None and out_ptr is None:
-                out = ws["OUT"]
-            self._prepare_ctx(ws, context)
-
-            def body():
-                self._run(ws, x_src_ptr if x_src_ptr is not None else x.data_ptr(), timesteps, context, out, x_in=x,
-                          sigmas=sigmas, out_ptr=out_ptr, out_sample_off=out_sample_off, t_ptr=t_src_ptr,
-                          x_copy=x if x_src_ptr is not None else None)
-
-            key = (tuple(x.shape), x.data_ptr(), timesteps.data_ptr(), context.data_ptr(), tuple(context.shape),
-                   sigmas.data_ptr(), out.data_ptr() if out is not None else 0, out_ptr or 0, out_sample_off,
-                   x_src_ptr or 0, t_src_ptr or 0)
-            self._graphs.run(key, body)
-            return out
-
-
-def W_mid(ex: "ZImageExecutor") -> int:
-    return ex.W["t0.w"].shape[0]
+        return self._forward(x, timesteps, context)
 
 
 def build_zimage_executor(model: nn.Module, device, **kw) -> ZImageExecutor:

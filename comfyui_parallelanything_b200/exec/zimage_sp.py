@@ -17,11 +17,10 @@ from typing import List, Optional
 import torch
 
 from .. import ops
-from ..models import flux as flux_model
-from ..models import zimage as zimage_model
 from . import block_linear
+from .dit import head_gather
 from .flux_sp import exchange_tables
-from .sp_common import UlyssesBase
+from .sp_common import UlyssesBase, attention_variant
 
 
 def supported(executors) -> Optional[str]:
@@ -68,8 +67,7 @@ class ZImageUlysses(UlyssesBase):
             return got
         n, ex0 = self.n, self.ex[0]
         p, dim, heads = ex0.params, ex0.dim, ex0.heads
-        hh, ww = H // 2, Wd // 2
-        Li = hh * ww
+        Li = (H // 2) * (Wd // 2)
         L = Lc + Li
         Lcl, Lil = Lc // n, Li // n
         Ll, hpg = Lcl + Lil, heads // n
@@ -92,9 +90,7 @@ class ZImageUlysses(UlyssesBase):
             ws["TOK"] = e(1, Li, 4 * p.in_channels)
             ws["T1"], ws["TH"], ws["TE"], ws["STE"] = e(1, 256), e(1, ex.W["t0.w"].shape[0]), e(1, p.adaln_dim), e(1, p.adaln_dim)
             ws["MOD"] = e(1, ex.W["mod.w"].shape[0])
-            ids = zimage_model.ZImageModel.make_ids(1, Lc, hh, ww, d)
-            pe = flux_model.EmbedND(128, p.rope_theta, p.axes_dims)(ids)
-            ws["ROPE"] = torch.stack([pe[0, 0, :, :, 0, 0], pe[0, 0, :, :, 1, 0]], -1).float().contiguous()
+            ws["ROPE"] = ex.rope(H, Wd, Lc)
             ws["ROPE_I"] = ws["ROPE"][Lc:].contiguous()
             # scratch of the (replicated, eager) caption path: what ZImageExecutor._prepare_ctx expects of a workspace
             ws["CTXWS"] = dict(Lc=Lc, XM=e(1, Lc, dim), Y=e(1, Lc, dim), ATT=e(1, Lc, dim), FF=e(1, Lc, p.ffn_hidden),
@@ -156,22 +152,21 @@ class ZImageUlysses(UlyssesBase):
         ops.gemm(ws["STE"], W["mod.w"], "bias", out=ws["MOD"], bias=W["mod.b"])
         C.copy_rows(ws["CTXWS"]["XT0"][:, g * Lcl:(g + 1) * Lcl], Xt)
         nl += 8
-        variant = lambda rows: 1 if hpg * ((rows + 255) // 256) < 110 else None  # noqa: E731
         slot = 0
         for i in range(ex.n_nr):            # image tokens only; RoPE row of local image row r = g*Lil + r of the image table
             nl += self._block(g, ws, slot, f"nr{i}", Xi, XM[:, Lcl:], Y[:, Lcl:], ws["CATi"], FF[:, Lcl:], ws["Qi"], ws["Ki"],
-                              ws["Vi"], ws["QFi"], ws["KFi"], ws["VFi"], ws["ATTFi"], "_I", True, variant(ws["Li"]),
-                              rope=ws["ROPE_I"], rope_off=g * Lil)
+                              ws["Vi"], ws["QFi"], ws["KFi"], ws["VFi"], ws["ATTFi"], "_I", True,
+                              attention_variant(hpg, ws["Li"]), rope=ws["ROPE_I"], rope_off=g * Lil)
             slot += 2
         for i in range(ex.n_layers):        # joint sequence, local layout [caption slice | image slice]
             nl += self._block(g, ws, slot, f"l{i}", X, XM, Y, ws["CAT"], FF, ws["Q"], ws["K"], ws["V"], ws["QF"], ws["KF"],
-                              ws["VF"], ws["ATTF"], "", True, variant(ws["L"]), rope=ws["ROPE"], rope_off=g * Lcl,
-                              rope_off2=Lc + g * Lil - Lcl, seg_rows=Lcl)
+                              ws["VF"], ws["ATTF"], "", True, attention_variant(hpg, ws["L"]), rope=ws["ROPE"],
+                              rope_off=g * Lcl, rope_off2=Lc + g * Lil - Lcl, seg_rows=Lcl)
             slot += 2
         # ---- head on my image tokens: LayerNorm * (1 + scale) + Linear + unpatchify, rows stored into the LEAD GPU's output
         ops.layernorm_modulate(Xi, XM[:, Lcl:], scale=ex._mod(ws, "final", 0), eps=1e-6)
-        ops.gemm(XM[:, Lcl:], W["final.w"], "euler_unpatch", bias=W["final.b"], C=p.in_channels, Hl=ws["H"], Wl=ws["Wd"],
-                 xout_sample_off=0, x_out_ptr=out_ptr, tok_off=g * Lil)
+        head_gather(XM[:, Lcl:], W["final.w"], W["final.b"], p.in_channels, ws["H"], ws["Wd"], out_ptr=out_ptr,
+                    tok_off=g * Lil)
         self._end_step(g)
         nl += 3
         return nl

@@ -100,6 +100,16 @@ class EmbedND(nn.Module):
         return emb.unsqueeze(1)
 
 
+def position_ids(b: int, hh: int, ww: int, txt_len: int, device) -> torch.Tensor:
+    """[b, txt_len + hh*ww, 3] RoPE positions: text tokens at (0, 0, 0), image token (r, c) at (0, r, c)."""
+    img_ids = torch.zeros(hh, ww, 3, device=device, dtype=torch.float32)
+    img_ids[..., 1] = torch.arange(hh, device=device, dtype=torch.float32)[:, None]
+    img_ids[..., 2] = torch.arange(ww, device=device, dtype=torch.float32)[None, :]
+    img_ids = img_ids.reshape(1, hh * ww, 3).expand(b, -1, -1)
+    txt_ids = torch.zeros(b, txt_len, 3, device=device, dtype=torch.float32)
+    return torch.cat((txt_ids, img_ids), dim=1)
+
+
 class MLPEmbedder(nn.Module):
     def __init__(self, in_dim: int, hidden_dim: int):
         super().__init__()
@@ -283,14 +293,7 @@ class Flux(nn.Module):
         return t.reshape(b, c, h, w)
 
     def make_ids(self, b: int, h: int, w: int, txt_len: int, device) -> torch.Tensor:
-        ps = self.patch_size
-        hh, ww = h // ps, w // ps
-        img_ids = torch.zeros(hh, ww, 3, device=device, dtype=torch.float32)
-        img_ids[..., 1] = torch.arange(hh, device=device, dtype=torch.float32)[:, None]
-        img_ids[..., 2] = torch.arange(ww, device=device, dtype=torch.float32)[None, :]
-        img_ids = img_ids.reshape(1, hh * ww, 3).expand(b, -1, -1)
-        txt_ids = torch.zeros(b, txt_len, 3, device=device, dtype=torch.float32)
-        return torch.cat((txt_ids, img_ids), dim=1)
+        return position_ids(b, h // self.patch_size, w // self.patch_size, txt_len, device)
 
     def forward_orig(self, img, ids, txt, timesteps, y, guidance=None):
         img = self.img_in(img)

@@ -143,7 +143,8 @@ class WanModel(nn.Module):
         if dtype is not None or device is not None:
             self.to(device=device, dtype=dtype)
 
-    def make_ids(self, b: int, t: int, h: int, w: int, device) -> torch.Tensor:
+    @staticmethod
+    def make_ids(b: int, t: int, h: int, w: int, device) -> torch.Tensor:
         ids = torch.zeros(t, h, w, 3, device=device, dtype=torch.float32)
         ids[..., 0] = torch.arange(t, device=device, dtype=torch.float32)[:, None, None]
         ids[..., 1] = torch.arange(h, device=device, dtype=torch.float32)[None, :, None]

@@ -155,10 +155,9 @@ class SpmdFluxEngine:
         """Run the replica on this rank's shard.  ``fused``: pull x/t/g inside the first kernel from rank 0 and
         store the result rows into rank 0's output buffer from the last kernel's epilogue."""
         if fused:
-            x_bytes = self.C * self.H * self.W * 2
             self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["y"], loc["g"], loc["sig"],
                                  out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
-                                 x_src_ptr=self._src("x", x_bytes), t_src_ptr=self._src("t", 2),
+                                 x_src_ptr=self._src("x", self._row_bytes("x")), t_src_ptr=self._src("t", 2),
                                  g_src_ptr=self._src("g", 2))
             return None
         return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["y"], loc["g"], loc["sig"])
@@ -172,13 +171,18 @@ class SpmdFluxEngine:
     def _src(self, name: str, row_bytes: int) -> int:
         return self.heap.peer_ptr(0, self.off[name]) + self.off_local * row_bytes
 
-    def _peer_view(self, name: str) -> torch.Tensor:
-        """This rank's shard of rank 0's staging tensor as a (peer-mapped) torch view."""
+    def _row_bytes(self, name: str) -> int:
+        """Bytes of one sample of the staged input ``name``."""
         shape, dt = self.spec[name]
         row = 1
         for s_ in shape[1:]:
             row *= s_
-        row_bytes = row * torch.empty((), dtype=dt).element_size()
+        return row * torch.empty((), dtype=dt).element_size()
+
+    def _peer_view(self, name: str) -> torch.Tensor:
+        """This rank's shard of rank 0's staging tensor as a (peer-mapped) torch view."""
+        shape, dt = self.spec[name]
+        row_bytes = self._row_bytes(name)
         t = self.heap.C.tensor_from_ptr(self._src(name, row_bytes), row_bytes * self.n_local, self.dev.index)
         return t.view(dt).view(self.n_local, *shape[1:])
 
@@ -380,13 +384,12 @@ class SpmdUNetEngine(SpmdFluxEngine):
     def _launch(self, loc: dict, fused: bool):
         y = loc.get("y")
         if fused:
-            x_bytes = self.C * self.H * self.W * 2
             if getattr(self.ex, "fused_in", False):
                 # fused scatter + conv_in: the first kernel reads the latent shard AND the timesteps from rank 0's heap
                 # and leaves the local NCHW copy (x_in of the Euler gather) in loc["x"] - no separate pull
                 self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], y, loc["sig"],
                                      out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
-                                     x_src_ptr=self._src("x", x_bytes), t_src_ptr=self._src("t", 2))
+                                     x_src_ptr=self._src("x", self._row_bytes("x")), t_src_ptr=self._src("t", 2))
                 return None
             if self.rank != 0:
                 self._pull("x")
@@ -397,12 +400,26 @@ class SpmdUNetEngine(SpmdFluxEngine):
         return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], y, loc["sig"])
 
 
-class SpmdWanEngine(SpmdFluxEngine):
-    """WAN2.x video DiT replicas (``exec/wan_exec.py``).  ``height``/``width`` are pixel sizes, ``frames`` the
-    number of LATENT frames; the video latent is staged as [B, 16, T, H/8, W/8]."""
+class _SpmdTextDiTEngine(SpmdFluxEngine):
+    """WAN / Z-Image replicas: the step inputs are latent, timestep and text features (no pooled vector, no guidance);
+    latent and timestep are pulled by the fused patch-embed kernel from rank 0's heap, the text features are read
+    through a TMA descriptor on the peer mapping."""
 
     tma_peer_inputs = ("ctx",)
     kernel_pulled_inputs = ("x", "t")
+
+    def _launch(self, loc: dict, fused: bool):
+        if fused:
+            self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"],
+                                 out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
+                                 x_src_ptr=self._src("x", self._row_bytes("x")), t_src_ptr=self._src("t", 2))
+            return None
+        return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"])
+
+
+class SpmdWanEngine(_SpmdTextDiTEngine):
+    """WAN2.x video DiT replicas (``exec/wan_exec.py``).  ``height``/``width`` are pixel sizes, ``frames`` the
+    number of LATENT frames; the video latent is staged as [B, 16, T, H/8, W/8]."""
 
     def __init__(self, executor, global_batch: int, frames: int, height: int, width: int, txt_len: int, **kw):
         self.T = frames
@@ -417,22 +434,9 @@ class SpmdWanEngine(SpmdFluxEngine):
         return {"x": (shape, bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
                 "sig": ((B, 2), torch.float32), "out": (shape, bf)}
 
-    def _launch(self, loc: dict, fused: bool):
-        if fused:
-            x_bytes = self.C * self.T * self.H * self.W * 2
-            self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"],
-                                 out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
-                                 x_src_ptr=self._src("x", x_bytes), t_src_ptr=self._src("t", 2))
-            return None
-        return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"])
 
-
-class SpmdZImageEngine(SpmdFluxEngine):
-    """Z-Image / NextDiT replicas (``exec/zimage_exec.py``): latent and timestep are pulled by the fused patch-embed
-    kernel from rank 0's heap, the caption features are read through a TMA descriptor on the peer mapping."""
-
-    tma_peer_inputs = ("ctx",)
-    kernel_pulled_inputs = ("x", "t")
+class SpmdZImageEngine(_SpmdTextDiTEngine):
+    """Z-Image / NextDiT replicas (``exec/zimage_exec.py``)."""
 
     def _latent_channels(self) -> int:
         return self.ex.params.in_channels
@@ -442,12 +446,3 @@ class SpmdZImageEngine(SpmdFluxEngine):
         shape = (B, self.C, self.H, self.W)
         return {"x": (shape, bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.cap_feat_dim), bf),
                 "sig": ((B, 2), torch.float32), "out": (shape, bf)}
-
-    def _launch(self, loc: dict, fused: bool):
-        if fused:
-            x_bytes = self.C * self.H * self.W * 2
-            self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"],
-                                 out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
-                                 x_src_ptr=self._src("x", x_bytes), t_src_ptr=self._src("t", 2))
-            return None
-        return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"])
