@@ -641,7 +641,7 @@ class ParallelEngine:
         io = self._io.get(key)
         if io is None:
             io = {"x": torch.empty(tuple(x.shape), dtype=bf, device=lead_dev),
-                  "out": torch.empty(tuple(x.shape), dtype=bf, device=lead_dev),
+                  "out": torch.empty(sp.out_shape(x), dtype=bf, device=lead_dev),
                   "slots": [sp.slot_buffers(slot.device, x, context, kwargs) for slot in self.slots]}
             if len(self._io) >= 8:
                 self._io.pop(next(iter(self._io)))

@@ -101,7 +101,10 @@ def builder_for(module: nn.Module) -> Optional[Callable]:
             from .flux_exec import build_flux_executor
             return build_flux_executor
     elif fam == "wan":
-        if p.dim // p.num_heads == 128 and tuple(p.patch_size) == (1, 2, 2) and p.in_dim == 16:
+        # in_dim 36: WAN2.2 image-to-video ([noise | mask | image latent]).  Models with a CLIP image embedding keep the
+        # torch replica: the executor has no image cross-attention and must not drop ``clip_fea``
+        if (p.dim // p.num_heads == 128 and tuple(p.patch_size) == (1, 2, 2) and p.in_dim in (16, 36)
+                and p.out_dim == 16 and not p.has_img_emb):
             from .wan_exec import build_wan_executor
             return build_wan_executor
     elif fam == "zimage":

@@ -24,10 +24,12 @@ def rope_layout(pe: torch.Tensor) -> torch.Tensor:
 
 
 def head_gather(a, w, b, C: int, Hl: int, Wl: int, out=None, out_ptr: Optional[int] = None, out_sample_off: int = 0,
-                x_in=None, sigmas=None, tok_off: int = 0) -> None:
+                x_in=None, sigmas=None, tok_off: int = 0, xin_bstride: int = 0) -> None:
     """Head GEMM with the unpatchify epilogue: token rows -> [B, C, Hl, Wl] latent, written to ``out`` or through
     ``out_ptr`` (e.g. the lead GPU's buffer) at sample ``out_sample_off``.  With ``sigmas`` the epilogue applies the
-    Euler update ``x_in + (sigma_next - sigma) * v``.  ``tok_off``: first token of ``a`` (a sequence-parallel slice)."""
+    Euler update ``x_in + (sigma_next - sigma) * v``.  ``tok_off``: first token of ``a`` (a sequence-parallel slice).
+    ``xin_bstride``: elements per sample of ``x_in`` when it is wider than the output (0: ``C*Hl*Wl``); the update then
+    reads its first ``C`` channels."""
     kw = dict(bias=b, C=C, Hl=Hl, Wl=Wl, xout_sample_off=out_sample_off, tok_off=tok_off)
     if out_ptr is not None:
         kw["x_out_ptr"] = out_ptr
@@ -35,6 +37,8 @@ def head_gather(a, w, b, C: int, Hl: int, Wl: int, out=None, out_ptr: Optional[i
         kw["x_out"] = out
     if sigmas is not None:
         kw["sigmas"], kw["x_in"] = sigmas, x_in
+        if xin_bstride:
+            kw["xin_bstride"] = xin_bstride
     ops.gemm(a, w, "euler_unpatch", **kw)
 
 
@@ -95,6 +99,10 @@ class DiTExecutor(nn.Module):
                                  on_evict=lambda _k: self._graphs.clear())
         return ws
 
+    def out_shape(self, shape) -> Tuple[int, ...]:
+        """Shape of the model output for an input latent of ``shape`` (the same, unless a family says otherwise)."""
+        return tuple(shape)
+
     @staticmethod
     def _geometry(shape, context) -> tuple:
         return (shape[0],) + tuple(shape[2:]) + (context.shape[1],)
@@ -123,7 +131,7 @@ class DiTExecutor(nn.Module):
         with torch.cuda.device(self.device):
             x, *inputs = self._prep(x, *step_inputs)
             ws = self.workspace(*self._geometry(x.shape, inputs[1]))
-            out = torch.empty_like(x)
+            out = torch.empty(self.out_shape(tuple(x.shape)), dtype=x.dtype, device=x.device)
             if self._prepare_ctx is not None:
                 self._prepare_ctx(ws, inputs[1])
             self._run(ws, x.data_ptr(), *inputs, out)

@@ -130,7 +130,9 @@ def _wan(m: nn.Module) -> Optional[SimpleNamespace]:
         in_dim=int(pe.shape[1]), out_dim=out_dim, dim=dim, ffn_dim=int(b0.ffn[0].weight.shape[0]), num_heads=int(heads),
         num_layers=len(m.blocks), text_dim=int(m.text_embedding[0].weight.shape[1]),
         text_len=int(_hint(m, "text_len", default=512)), freq_dim=int(m.time_embedding[0].weight.shape[1]),
-        patch_size=patch, eps=float(_hint(m, "eps", default=1e-6)))
+        patch_size=patch, eps=float(_hint(m, "eps", default=1e-6)),
+        # CLIP image projection of WAN2.1 I2V / FLF2V and the Fun models: their blocks add an image cross-attention
+        has_img_emb=getattr(m, "img_emb", None) is not None)
 
 
 # --------------------------------------------------------------------------------------------- Z-Image / NextDiT

@@ -55,6 +55,10 @@ class UlyssesBase:
     def geometry(self, x, context) -> tuple:
         raise NotImplementedError
 
+    def out_shape(self, x) -> tuple:
+        """Shape of the step's output for the latent ``x`` (WAN image-to-video: fewer channels than its input)."""
+        return tuple(x.shape)
+
     def workspace(self, *geometry) -> list:
         raise NotImplementedError
 

@@ -3,8 +3,10 @@
 Same building blocks as the FLUX executor (tcgen05 GEMM with fused epilogues, TMEM attention, AdaLN
 LayerNorm kernel) plus what WAN needs on top:
 
-  * the video latent ``[B, 16, T, H, W]`` is patchified by the fused scatter kernel as a ``T*H`` tall image
-    (Conv3d(1,2,2) == the same 2x2 patch GEMM applied per frame), timestep sinusoid included;
+  * the video latent ``[B, in_dim, T, H, W]`` is patchified by the fused scatter kernel as a ``T*H`` tall image
+    (Conv3d(1,2,2) == the same 2x2 patch GEMM applied per frame), timestep sinusoid included.  ``in_dim`` is 16 for
+    text-to-video and 36 for WAN2.2 image-to-video, whose input is ``[noise 16 | mask 4 | image latent 16]``; the output
+    and the Euler update always cover the ``out_dim`` = 16 noise channels;
   * q/k use a *full-width* RMSNorm (over all heads) followed by 3-D RoPE: a dedicated in-place kernel on
     the fused QKV GEMM output; attention then reads q/k/v through strided 4-D TMA views;
   * per-block modulation = learned table + time projection: one broadcast-add kernel builds all 40x6
@@ -34,15 +36,16 @@ class WanExecutor(DiTExecutor):
         super().__init__(model, device, cuda_graphs)
         d, p = self.device, self.params
         self.dim, self.heads = p.dim, p.num_heads
-        if p.dim // p.num_heads != 128 or tuple(p.patch_size) != (1, 2, 2) or p.in_dim != 16:
-            raise ValueError("WanExecutor is specialised for head_dim 128, patch (1,2,2), 16 latent channels")
+        if p.dim // p.num_heads != 128 or tuple(p.patch_size) != (1, 2, 2) or p.in_dim not in (16, 36) or p.out_dim != 16:
+            raise ValueError("WanExecutor is specialised for head_dim 128, patch (1,2,2), 16 (T2V) or 36 (I2V) input "
+                             "and 16 output latent channels")
         W: Dict[str, Optional[torch.Tensor]] = {}
 
         def lin(name, m):
             W[name + ".w"] = _bf(m.weight, d)
             W[name + ".b"] = _bf(m.bias, d) if m.bias is not None else None
 
-        W["patch.w"] = _bf(model.patch_embedding.weight.reshape(p.dim, -1), d)          # [dim, 16*1*2*2]
+        W["patch.w"] = _bf(model.patch_embedding.weight.reshape(p.dim, -1), d)          # [dim, in_dim*1*2*2]
         W["patch.b"] = _bf(model.patch_embedding.bias, d)
         lin("text0", model.text_embedding[0])
         lin("text2", model.text_embedding[2])
@@ -90,6 +93,10 @@ class WanExecutor(DiTExecutor):
         ids = wan_model.WanModel.make_ids(1, T, H // 2, Wd // 2, self.device)
         dd = 128
         return rope_layout(flux_model.EmbedND(dd, 10000, [dd - 4 * (dd // 6), 2 * (dd // 6), 2 * (dd // 6)])(ids))
+
+    def out_shape(self, shape) -> tuple:
+        """[B, in_dim, T, H, W] -> [B, out_dim, T, H, W] (image-to-video predicts only the noise channels)."""
+        return (shape[0], self.params.out_dim) + tuple(shape[2:])
 
     def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int) -> dict:
         d, dim = self.device, self.dim
@@ -144,7 +151,7 @@ class WanExecutor(DiTExecutor):
         TH = ws["T"] * ws["H"]
         # fused scatter: video latent (as a T*H tall image) -> patch GEMM ; timestep sinusoid
         C.scatter_patch_embed(W["patch.w"], W["patch.b"], x_ptr, t_ptr if t_ptr is not None else t.data_ptr(), 0,
-                              ws["T1"], None, x_copy, X, 16, TH, ws["Wd"], 1.0)
+                              ws["T1"], None, x_copy, X, self.params.in_dim, TH, ws["Wd"], 1.0)
         ops.gemm(ws["T1"], W["time0.w"], "silu", out=ws["E_H"], bias=W["time0.b"])
         ops.gemm(ws["E_H"], W["time2.w"], "bias", out=ws["E"], bias=W["time2.b"])
         C.silu(ws["E"], ws["SE"])
@@ -179,8 +186,10 @@ class WanExecutor(DiTExecutor):
             n += 8
         # ---- head: AdaLN + Linear + unpatchify (+ Euler, + peer store)
         ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=self.eps)
-        head_gather(XM, W["head.w"], W["head.b"], self.params.out_dim, TH, ws["Wd"], out=out, out_ptr=out_ptr,
-                    out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas)
+        p = self.params
+        head_gather(XM, W["head.w"], W["head.b"], p.out_dim, TH, ws["Wd"], out=out, out_ptr=out_ptr,
+                    out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas,
+                    xin_bstride=p.in_dim * TH * ws["Wd"] if p.in_dim != p.out_dim else 0)
         n += 2
         self.launches_per_step = n
         return out

@@ -72,7 +72,7 @@ class WanUlysses(UlyssesBase):
 
     # ------------------------------------------------------------------ engine-facing protocol
     def accepts(self, x, context) -> bool:
-        if x.dim() != 5 or context.dim() != 3 or x.shape[1] != 16:
+        if x.dim() != 5 or context.dim() != 3 or x.shape[1] != self.ex[0].params.in_dim:
             return False
         T, H, Wd = x.shape[2], x.shape[3], x.shape[4]
         if H % 2 or Wd % 2:
@@ -80,6 +80,9 @@ class WanUlysses(UlyssesBase):
         L = T * (H // 2) * (Wd // 2)
         # a GPU's token slice must be whole 8-row groups (TMA swizzle atoms of the head-sliced views)
         return L % (8 * self.n) == 0
+
+    def out_shape(self, x) -> tuple:
+        return self.ex[0].out_shape(tuple(x.shape))
 
     def geometry(self, x, context) -> tuple:
         return (x.shape[2], x.shape[3], x.shape[4], context.shape[1])
@@ -98,7 +101,7 @@ class WanUlysses(UlyssesBase):
             d = ex.device
             e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=d)  # noqa: E731
             ws = dict(g=g, B=1, T=T, H=H, Wd=Wd, L=L, Ll=Ll, Lc=Lc, hpg=hpg)
-            ws["TOK"] = e(1, L, 64)
+            ws["TOK"] = e(1, L, 4 * ex.params.in_dim)
             ws["X"], ws["XM"] = e(1, Ll, dim), e(1, Ll, dim)
             ws["QKV"] = e(1, Ll, 3 * dim)                            # my tokens, all heads
             ws["QF"], ws["KF"], ws["VF"] = e(1, L, hpg * 128), e(1, L, hpg * 128), e(1, L, hpg * 128)   # all tokens, my heads
@@ -137,7 +140,7 @@ class WanUlysses(UlyssesBase):
         t = st["t"]
         nl = 0
         # ---- embedders: patchify the whole clip (a T*H tall image), embed only my token slice; time path is replicated
-        C.patchify(x_ptr, ws["TOK"], 1, 16, TH, ws["Wd"], 2)
+        C.patchify(x_ptr, ws["TOK"], 1, ex.params.in_dim, TH, ws["Wd"], 2)
         ops.gemm(ws["TOK"][:, g * Ll:(g + 1) * Ll], W["patch.w"], "bias", out=X, bias=W["patch.b"])
         ops.timestep_embedding(t, 256, time_factor=1.0, out=ws["T1"])
         ops.gemm(ws["T1"], W["time0.w"], "silu", out=ws["E_H"], bias=W["time0.b"])

@@ -42,6 +42,12 @@ def wan22_a14b_params() -> WanParams:
     return WanParams()
 
 
+def wan22_i2v_a14b_params() -> WanParams:
+    """WAN2.2-I2V-A14B: the T2V layer stack with a 36-channel input ([noise 16 | mask 4 | image latent 16], concatenated
+    by the sampler before every call) and the 16 noise channels as output."""
+    return WanParams(in_dim=36)
+
+
 def wan_tiny_params() -> WanParams:
     return WanParams(in_dim=16, out_dim=16, dim=256, ffn_dim=512, num_heads=2, num_layers=2, text_dim=64,
                      text_len=16)
@@ -180,6 +186,25 @@ def example_inputs(params: WanParams, batch: int, frames: int = 16, height: int 
     g = torch.Generator(device="cpu").manual_seed(seed)
     lt = max(1, frames // 4)
     x = torch.randn(batch, params.in_dim, lt, height // 8, width // 8, generator=g).to(device=device, dtype=dtype)
+    t = (torch.rand(batch, generator=g) * 1000).to(device=device, dtype=dtype)
+    ctx = torch.randn(batch, params.text_len, params.text_dim, generator=g).to(device=device, dtype=dtype)
+    return dict(x=x, timesteps=t, context=ctx)
+
+
+def i2v_inputs(params: WanParams, batch: int, frames: int = 16, height: int = 720, width: int = 1280,
+               device="cpu", dtype=torch.bfloat16, seed: int = 0):
+    """Image-to-video step inputs: ``x = cat(noise, mask, image latent)`` along the channels, as ComfyUI builds it for
+    WAN2.2 I2V.  The mask is ones on the first latent frame (the conditioning image) and zeros elsewhere."""
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    lt = max(1, frames // 4)
+    hl, wl = height // 8, width // 8
+    nc = params.out_dim
+    mc = params.in_dim - 2 * nc
+    noise = torch.randn(batch, nc, lt, hl, wl, generator=g)
+    mask = torch.zeros(batch, mc, lt, hl, wl)
+    mask[:, :, 0] = 1.0
+    image = torch.randn(batch, nc, lt, hl, wl, generator=g)
+    x = torch.cat([noise, mask, image], 1).to(device=device, dtype=dtype)
     t = (torch.rand(batch, generator=g) * 1000).to(device=device, dtype=dtype)
     ctx = torch.randn(batch, params.text_len, params.text_dim, generator=g).to(device=device, dtype=dtype)
     return dict(x=x, timesteps=t, context=ctx)

@@ -419,7 +419,8 @@ class _SpmdTextDiTEngine(SpmdFluxEngine):
 
 class SpmdWanEngine(_SpmdTextDiTEngine):
     """WAN2.x video DiT replicas (``exec/wan_exec.py``).  ``height``/``width`` are pixel sizes, ``frames`` the
-    number of LATENT frames; the video latent is staged as [B, 16, T, H/8, W/8]."""
+    number of LATENT frames; the video latent is staged as [B, in_dim, T, H/8, W/8] (16 channels for text-to-video, 36
+    for image-to-video) and the result as [B, out_dim = 16, T, H/8, W/8]."""
 
     def __init__(self, executor, global_batch: int, frames: int, height: int, width: int, txt_len: int, **kw):
         self.T = frames
@@ -430,9 +431,8 @@ class SpmdWanEngine(_SpmdTextDiTEngine):
 
     def _make_spec(self, B: int) -> dict:
         p, bf = self.ex.params, torch.bfloat16
-        shape = (B, self.C, self.T, self.H, self.W)
-        return {"x": (shape, bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
-                "sig": ((B, 2), torch.float32), "out": (shape, bf)}
+        return {"x": ((B, self.C, self.T, self.H, self.W), bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
+                "sig": ((B, 2), torch.float32), "out": ((B, p.out_dim, self.T, self.H, self.W), bf)}
 
 
 class SpmdZImageEngine(_SpmdTextDiTEngine):

@@ -198,6 +198,21 @@ def gemm_euler_unpatch():
     return r
 
 
+@check
+def euler_unpatch_xin_stride():
+    """Euler update of the first 16 channels of a wider (36-channel, WAN I2V) input: ``xin_bstride`` = its sample size."""
+    B, C, Cin, Hl, Wl, hid = 2, 16, 36, 32, 48, 256
+    L = (Hl // 2) * (Wl // 2)
+    h, w, b = _rand(B, L, hid), _rand(C * 4, hid, scale=0.06), _rand(C * 4)
+    x = _rand(B, Cin, Hl, Wl)
+    sig = torch.tensor([[1.0, 0.9], [0.5, 0.25]], device=_dev())
+    xo = torch.zeros(B, C, Hl, Wl, dtype=torch.bfloat16, device=_dev())
+    ops.gemm(h, w, "euler_unpatch", bias=b, x_in=x, xin_bstride=Cin * Hl * Wl, x_out=xo, sigmas=sig, C=C, Hl=Hl, Wl=Wl)
+    v = _gemm_ref(h, w, b).view(B, Hl // 2, Wl // 2, C, 2, 2).permute(0, 3, 1, 4, 2, 5).reshape(B, C, Hl, Wl)
+    want = x[:, :C].float() + (sig[:, 1] - sig[:, 0])[:, None, None, None] * v
+    return _cmp("euler_unpatch_xin_stride", xo, want, 0.012)
+
+
 # ------------------------------------------------------------------------------ attention
 def _attn_case(name, B, H, Lq, Lk, tol=0.02):
     q, k, v = _rand(B, H, Lq, 128), _rand(B, H, Lk, 128, seed=1), _rand(B, H, Lk, 128, seed=2)
@@ -377,6 +392,31 @@ def scatter_patch_embed():
     r["temb_mean_rel"] = r2["mean_rel"]
     r["ok"] = r["ok"] and r2["ok"] and bool(torch.equal(xc, x)) and bool(X[:, :77].abs().max().item() == 0)
     return r
+
+
+@check
+def scatter_patch_embed_wide():
+    """Fused scatter kernel with latents wider than one 64-column K block (WAN2.2 I2V: 36 channels), 2..4 K blocks.
+    One sample, so the output columns are split over several CTAs; 260 tokens = a partial last token tile."""
+    from ..models import flux
+    C_ = ops.require()
+    m = flux.Flux.__new__(flux.Flux)
+    m.patch_size = 2
+    Hl, Wl, N = 26, 40, 768
+    Li = (Hl // 2) * (Wl // 2)
+    t = torch.tensor([0.7], device=_dev(), dtype=torch.bfloat16)
+    worst = None
+    for Cc in (20, 36, 64):
+        x, w, b = _rand(1, Cc, Hl, Wl), _rand(N, 4 * Cc, scale=0.1), _rand(N)
+        X = torch.zeros(1, 5 + Li, N, dtype=torch.bfloat16, device=_dev())
+        t_emb = torch.zeros(1, 256, dtype=torch.bfloat16, device=_dev())
+        xc = torch.zeros_like(x)
+        C_.scatter_patch_embed(w, b, x.data_ptr(), t.data_ptr(), 0, t_emb, None, xc, X[:, 5:], Cc, Hl, Wl, 1.0)
+        r = _cmp("scatter_patch_embed_wide", X[:, 5:], _gemm_ref(flux.Flux.patchify(m, x), w, b), 0.012, C=Cc)
+        r["ok"] = r["ok"] and bool(torch.equal(xc, x)) and bool(X[:, :5].abs().max().item() == 0)
+        if worst is None or not r["ok"] or (worst["ok"] and r["mean_rel"] > worst["mean_rel"]):
+            worst = r
+    return worst
 
 
 # ------------------------------------------------------------------------------ convolution
@@ -583,6 +623,54 @@ def wan_executor_tiny():
     r["euler_mean_rel"] = r2["mean_rel"]
     r["ok"] = r["ok"] and r2["ok"]
     return r
+
+
+def _wan_i2v_case(fp8: bool) -> dict:
+    """Tiny WAN2.2 I2V executor (36 input channels) against the fp32 oracle: ``forward``, then ``denoise_step`` eager,
+    captured and replayed twice with the latent changed in place between the calls."""
+    import dataclasses
+    from ..exec.wan_exec import WanExecutor
+    from ..models import wan
+    p = dataclasses.replace(wan.wan_tiny_params(), in_dim=36)
+    torch.manual_seed(3)
+    m = wan.WanModel(p).to(device=_dev(), dtype=torch.bfloat16).eval()
+    ex = WanExecutor(m, _dev(), cuda_graphs=True, fp8=fp8)
+    oracle = wan.WanModel(p).to(device=_dev(), dtype=torch.float32).eval()
+    oracle.load_state_dict({k: v.float() for k, v in m.state_dict().items()})
+    inp = wan.i2v_inputs(p, 2, frames=8, height=128, width=192, device=_dev(), dtype=torch.bfloat16, seed=4)
+    tol = 0.05 if fp8 else 0.03
+    name = "wan_i2v_executor_tiny" + ("_fp8" if fp8 else "")
+    with torch.no_grad():
+        got = ex(**inp)
+        want = oracle(**{k: v.float() for k, v in inp.items()})
+    r = _cmp(name, got, want, tol)
+    r["ok"] = r["ok"] and tuple(got.shape) == (2, 16) + tuple(inp["x"].shape[2:])
+    sig = torch.tensor([[1.0, 0.8], [0.6, 0.5]], device=_dev())
+    x, t, c = ex._prep(inp["x"], inp["timesteps"], inp["context"])
+    worst = 0.0
+    for it in range(4):                                 # eager, capture, replay, replay
+        x[:, :16].mul_(0.9)                             # only the noise channels change between steps
+        nxt = ex.denoise_step(x, t, c, sig).clone()
+        with torch.no_grad():
+            v = oracle(x.float(), t.float(), context=c.float())
+        want2 = x[:, :16].float() + (sig[:, 1] - sig[:, 0])[:, None, None, None, None] * v
+        r2 = _cmp(name + "_euler", nxt, want2, tol)
+        worst = max(worst, r2["mean_rel"])
+        r["ok"] = r["ok"] and r2["ok"]
+    r["euler_worst_mean_rel"] = worst
+    r["graphs"] = sorted(ex._graphs.state(k) for k in list(ex._graphs._graphs))
+    r["ok"] = r["ok"] and "graph" in r["graphs"]
+    return r
+
+
+@check
+def wan_i2v_executor_tiny():
+    return _wan_i2v_case(False)
+
+
+@check
+def wan_i2v_executor_tiny_fp8():
+    return _wan_i2v_case(True)
 
 
 @check

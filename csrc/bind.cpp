@@ -83,7 +83,7 @@ static void parse_epilogue(const py::kwargs& kw, pa::GemmParams& p, bool check_s
 }
 
 // gemm(A, W, mode, out=..., bias=..., residual=..., gate=..., q=,k=,v=,q_scale=,k_scale=,rope=,heads=,seq_off=,
-//      mlp_col_off=, qk_eps=, x_in=, x_out= | x_out_ptr=, xout_sample_off=, sigmas=, C=,Hl=,Wl=, force_bn=)
+//      mlp_col_off=, qk_eps=, x_in=, xin_bstride=, x_out= | x_out_ptr=, xout_sample_off=, sigmas=, C=,Hl=,Wl=, force_bn=)
 static void parse_modes(int mode, const py::kwargs& kw, pa::GemmParams& p);
 
 static void gemm(Tensor A, Tensor W, int mode, py::kwargs kw) {
@@ -188,6 +188,9 @@ static void parse_modes(int mode, const py::kwargs& kw, pa::GemmParams& p) {
     if (has(kw, "x_out_ptr")) p.x_out = reinterpret_cast<__nv_bfloat16*>(kw["x_out_ptr"].cast<uintptr_t>());
     else p.x_out = reinterpret_cast<__nv_bfloat16*>(ten(kw, "x_out").data_ptr());
     p.xout_sample_off = has(kw, "xout_sample_off") ? kw["xout_sample_off"].cast<long long>() : 0;
+    p.xin_bstride = has(kw, "xin_bstride") ? kw["xin_bstride"].cast<long long>() : 0;
+    TORCH_CHECK(p.xin_bstride == 0 || p.xin_bstride >= (long long)p.C * p.Hl * p.Wl,
+                "xin_bstride must cover the C*Hl*Wl elements the update reads");
     if (has(kw, "sigmas")) {
       Tensor s = ten(kw, "sigmas");
       TORCH_CHECK(s.scalar_type() == at::kFloat && s.is_contiguous(), "sigmas must be float32 [B, 2]");
@@ -301,7 +304,10 @@ static void scatter_patch_embed(Tensor W, Tensor bias, uintptr_t x_src, uintptr_
                                 c10::optional<Tensor> g_emb, c10::optional<Tensor> x_copy, Tensor out, int C, int Hl,
                                 int Wl, double time_factor) {
   c10::cuda::CUDAGuard guard(out.device());
-  TORCH_CHECK(W.dim() == 2 && W.size(1) == 64 && W.stride(1) == 1, "img_in weight must be [N, 64]");
+  // up to 16 channels the patch is one 64-column K block; wider latents use the plain [N, 4*C] patch reshape
+  const int64_t K = C <= 16 ? 64 : 4 * (int64_t)C;
+  TORCH_CHECK(W.dim() == 2 && W.size(1) == K && W.stride(1) == 1, "img_in weight must be [N, ", K, "]");
+  TORCH_CHECK(C <= 16 || (C <= 64 && C % 2 == 0), "scatter_patch_embed: wide latents need an even C <= 64, got ", C);
   pa::ScatterEmbedParams p{};
   int ob, orows;
   view3(out, ob, orows, p.ldo, p.out_bstride);

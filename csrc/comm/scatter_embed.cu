@@ -5,7 +5,12 @@
 // NVLink peer mapping; 4-byte loads, coalesced along W), applying the 2x2 patchify permutation on
 // the fly, and write them as the 128B-swizzled K-major A operand of a tcgen05 GEMM:
 //
-//     X[b, Lt + token, :] = patchify(x_peer[off + b])[token, :] @ W_img_in^T + bias      (K = 64)
+//     X[b, Lt + token, :] = patchify(x_peer[off + b])[token, :] @ W_img_in^T + bias      (K = 4*C)
+//
+// Up to 16 latent channels the patch is one 64-column K block (FLUX, Z-Image, WAN T2V).  Wider latents (WAN2.2 I2V:
+// 36 channels = noise | mask | image latent) take NKB = ceil(C / 16) K blocks: the producers write one swizzled slab
+// per block, the weight ring streams (n-tile, k-block) slabs (columns past 4*C come from the tensor map's zero fill,
+// so the weight stays the plain [N, 4*C] reshape) and the MMA warp accumulates over the blocks.
 //
 // W tiles stream through a TMA ring, accumulators are double buffered in TMEM, the epilogue adds the
 // bias and stores bf16 rows of the residual stream.  A spare warp of CTA 0 reads the shard's
@@ -21,19 +26,27 @@
 namespace pa {
 
 namespace se {
-constexpr int BM = 128, BN = 256, BK = 64, WSTAGES = 3;
-constexpr uint32_t A_BYTES = BM * BK * 2, W_BYTES = BN * BK * 2;
-constexpr uint32_t OFF_W = A_BYTES;
-constexpr uint32_t OFF_STAGE = OFF_W + WSTAGES * W_BYTES;      // 4 slabs of [128 rows x 64 cols] bf16, 128B-swizzled
-constexpr uint32_t STAGE_BYTES = BM * BN * 2;
-constexpr uint32_t OFF_BAR = OFF_STAGE + STAGE_BYTES;
-constexpr uint32_t SMEM_BYTES = OFF_BAR + 256 + 1024;
+constexpr int BM = 128, BN = 256, BK = 64, WSTAGES = 3, MAX_KB = 4;
+constexpr uint32_t A_BYTES = BM * BK * 2, W_BYTES = BN * BK * 2;   // A_BYTES: one K block (slab) of the token tile
+constexpr uint32_t STAGE_BYTES = BM * BN * 2;                      // 4 slabs of [128 rows x 64 cols] bf16, 128B-swizzled
+
+// shared-memory layout for NKB K blocks: [A slabs | W ring | store staging | barriers]
+template <int NKB>
+struct Smem {
+  static constexpr uint32_t OFF_W = NKB * A_BYTES;
+  static constexpr uint32_t OFF_STAGE = OFF_W + WSTAGES * W_BYTES;
+  static constexpr uint32_t OFF_BAR = OFF_STAGE + STAGE_BYTES;
+  static constexpr uint32_t BYTES = OFF_BAR + 256 + 1024;
+  static_assert(BYTES <= 227 * 1024, "scatter_patch_embed: shared memory over the 227 KB per-block limit");
+};
 }  // namespace se
 
+template <int NKB>
 __global__ void __launch_bounds__(256, 1)
 scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmO,
                            const ScatterEmbedParams p) {
   using namespace se;
+  constexpr uint32_t OFF_W = Smem<NKB>::OFF_W, OFF_STAGE = Smem<NKB>::OFF_STAGE, OFF_BAR = Smem<NKB>::OFF_BAR;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OFF_BAR);
@@ -87,12 +100,16 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
     const bool leader = ptx::elect_one();
     const uint32_t smem_u = __shfl_sync(0xffffffffu, ptx::smem_u32(smem), 0);
     for (int nt = 0; nt < num_n; ++nt) {
-      const int s = nt % WSTAGES;
-      const uint32_t ph = (nt / WSTAGES) & 1;
-      ptx::mbar_wait(&w_empty[s], ph ^ 1);
-      if (leader) {
-        ptx::mbar_arrive_expect_tx(&w_full[s], W_BYTES);
-        ptx::tma_load_2d_s(smem_u + OFF_W + s * W_BYTES, &tmW, &w_full[s], 0, (nt0 + nt) * BN);
+#pragma unroll
+      for (int kb = 0; kb < NKB; ++kb) {
+        const int it = nt * NKB + kb;
+        const int s = it % WSTAGES;
+        const uint32_t ph = (it / WSTAGES) & 1;
+        ptx::mbar_wait(&w_empty[s], ph ^ 1);
+        if (leader) {
+          ptx::mbar_arrive_expect_tx(&w_full[s], W_BYTES);
+          ptx::tma_load_2d_s(smem_u + OFF_W + s * W_BYTES, &tmW, &w_full[s], kb * BK, (nt0 + nt) * BN);
+        }
       }
     }
     __syncwarp();
@@ -105,16 +122,23 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
     ptx::tc_fence_after();
     const uint64_t adesc = ptx::make_desc_kmajor_sw128(smem_u);
     for (int nt = 0; nt < num_n; ++nt) {
-      const int s = nt % WSTAGES, acc = nt & 1;
-      ptx::mbar_wait(&w_full[s], (nt / WSTAGES) & 1);
-      ptx::mbar_wait(&tempty[acc], ((nt >> 1) & 1) ^ 1);
-      ptx::tc_fence_after();
-      if (leader) {
-        const uint64_t bdesc = ptx::make_desc_kmajor_sw128(smem_u + OFF_W + s * W_BYTES);
+      const int acc = nt & 1;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) ptx::mma_f16_ss(tmem_u + acc * BN, adesc + 2 * k, bdesc + 2 * k, IDESC, k != 0);
-        ptx::tc_commit(&w_empty[s]);
-        ptx::tc_commit(&tfull[acc]);
+      for (int kb = 0; kb < NKB; ++kb) {
+        const int it = nt * NKB + kb;
+        const int s = it % WSTAGES;
+        ptx::mbar_wait(&w_full[s], (it / WSTAGES) & 1);
+        if (kb == 0) ptx::mbar_wait(&tempty[acc], ((nt >> 1) & 1) ^ 1);
+        ptx::tc_fence_after();
+        if (leader) {
+          const uint64_t bdesc = ptx::make_desc_kmajor_sw128(smem_u + OFF_W + s * W_BYTES);
+          const uint64_t ad = adesc + kb * (A_BYTES >> 4);                 // descriptor address field is in 16 B units
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            ptx::mma_f16_ss(tmem_u + acc * BN, ad + 2 * k, bdesc + 2 * k, IDESC, (kb | k) != 0);
+          ptx::tc_commit(&w_empty[s]);
+          if (kb == NKB - 1) ptx::tc_commit(&tfull[acc]);
+        }
       }
     }
     __syncwarp();
@@ -149,10 +173,11 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
       const int hh = tok / Wp, ww = tok - hh * Wp;
       const long long sample = static_cast<long long>(b) * p.C * p.Hl * p.Wl;
       const __nv_bfloat16* xs = p.x_src + sample;
-      // all 32 peer loads are issued before the first use: one NVLink round trip (~2-3 us) instead of four
-      uint32_t v[32];
+      // every peer load of the row is issued before the first use: one NVLink round trip (~2-3 us) instead of one per
+      // channel pair (NKB * 32 four-byte loads; with four K blocks 128 registers, still without spills)
+      uint32_t v[NKB * 32];
 #pragma unroll
-      for (int c = 0; c < 16; ++c) {
+      for (int c = 0; c < NKB * 16; ++c) {
 #pragma unroll
         for (int ph = 0; ph < 2; ++ph) {
           const long long pix = (static_cast<long long>(c) * p.Hl + (hh * 2 + ph)) * p.Wl + ww * 2;
@@ -160,20 +185,20 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
         }
       }
 #pragma unroll
-      for (int c = 0; c < 16; ++c) {
+      for (int c = 0; c < NKB * 16; ++c) {
 #pragma unroll
         for (int ph = 0; ph < 2; ++ph) {
           if (p.x_copy && ns_i == 0 && c < p.C) {
             const long long pix = (static_cast<long long>(c) * p.Hl + (hh * 2 + ph)) * p.Wl + ww * 2;
             *reinterpret_cast<uint32_t*>(p.x_copy + sample + pix) = v[c * 2 + ph];
           }
-          const int chunk = (c >> 1) ^ sw;
-          *reinterpret_cast<uint32_t*>(arow + chunk * 16 + (c & 1) * 8 + ph * 4) = v[c * 2 + ph];
+          const int chunk = ((c & 15) >> 1) ^ sw;                          // K column 4*c + 2*ph + pw, slab c / 16
+          *reinterpret_cast<uint32_t*>(arow + (c >> 4) * A_BYTES + chunk * 16 + (c & 1) * 8 + ph * 4) = v[c * 2 + ph];
         }
       }
     } else {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) *reinterpret_cast<uint4*>(arow + i * 16) = make_uint4(0, 0, 0, 0);
+      for (int i = 0; i < NKB * 8; ++i) *reinterpret_cast<uint4*>(arow + (i >> 3) * A_BYTES + (i & 7) * 16) = make_uint4(0, 0, 0, 0);
     }
     ptx::fence_proxy_async_smem();
     ptx::mbar_arrive(a_full);
@@ -239,11 +264,30 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
   }
 }
 
+template <int NKB>
+static int launch_scatter_patch_embed(const CUtensorMap& tw, const CUtensorMap& to, const ScatterEmbedParams& q,
+                                      int blocks, cudaStream_t st) {
+  constexpr int bytes = static_cast<int>(se::Smem<NKB>::BYTES);
+  static bool attr_set[64] = {false};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (!attr_set[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(scatter_patch_embed_kernel<NKB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         bytes);
+    if (e != cudaSuccess) return (int)e;
+    attr_set[dev] = true;
+  }
+  scatter_patch_embed_kernel<NKB><<<blocks, 256, bytes, st>>>(tw, to, q);
+  return (int)cudaGetLastError();
+}
+
+// W: [N, 64] for C <= 16 (the one-block layout), else [N, 4*C] with C even (16-byte aligned rows)
 int scatter_patch_embed(const void* W, long long ldw, const ScatterEmbedParams& p, cudaStream_t st) {
   using namespace se;
-  if (p.C > 16 || p.N % 32 || (p.Wl & 1)) return -1;
+  if (p.C < 1 || p.C > MAX_KB * 16 || (p.C > 16 && (p.C & 1)) || p.N % 32 || (p.Wl & 1)) return -1;
+  const int nkb = p.C <= 16 ? 1 : (p.C + 15) / 16;
   CUtensorMap tw;
-  uint64_t dims[2] = {64, (uint64_t)p.N};
+  uint64_t dims[2] = {nkb == 1 ? 64u : (uint64_t)(4 * p.C), (uint64_t)p.N};
   uint64_t str[2] = {2, (uint64_t)ldw * 2};
   uint32_t box[2] = {64, (uint32_t)BN};
   if (make_tmap(&tw, W, 2, dims, str, box, 2)) return -20;
@@ -255,22 +299,17 @@ int scatter_patch_embed(const void* W, long long ldw, const ScatterEmbedParams& 
     if ((p.ldo % 8) || (p.out_bstride % 8) || (reinterpret_cast<uintptr_t>(p.out) & 15)) return -2;
     if (make_tmap(&to, p.out, 3, od, os, ob, 2)) return -21;
   }
-  static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(scatter_patch_embed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)SMEM_BYTES);
-    if (e != cudaSuccess) return (int)e;
-    attr_set[dev] = true;
-  }
   ScatterEmbedParams q = p;
   const int mtiles = p.n * ((p.Li + BM - 1) / BM);
   const int num_n = (p.N + BN - 1) / BN;
   q.nsplit = 1;
   while (mtiles * q.nsplit * 2 <= 160 && q.nsplit * 2 <= num_n) q.nsplit *= 2;      // fill ~148 SMs, whole tiles per CTA
-  scatter_patch_embed_kernel<<<mtiles * q.nsplit, 256, SMEM_BYTES, st>>>(tw, to, q);
-  return (int)cudaGetLastError();
+  switch (nkb) {
+    case 1: return launch_scatter_patch_embed<1>(tw, to, q, mtiles * q.nsplit, st);
+    case 2: return launch_scatter_patch_embed<2>(tw, to, q, mtiles * q.nsplit, st);
+    case 3: return launch_scatter_patch_embed<3>(tw, to, q, mtiles * q.nsplit, st);
+    default: return launch_scatter_patch_embed<4>(tw, to, q, mtiles * q.nsplit, st);
+  }
 }
 
 }  // namespace pa

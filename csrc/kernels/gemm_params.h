@@ -54,6 +54,8 @@ struct GemmParams {
   const __nv_bfloat16* x_in;        // local latent shard  [batch, C, Hl, Wl]
   __nv_bfloat16* x_out;             // destination (lead GPU buffer, possibly a peer mapping)
   long long xout_sample_off;        // first sample of this rank inside x_out
+  long long xin_bstride;            // elements per sample of x_in (0: C*Hl*Wl); a wider input (WAN I2V: noise | mask |
+                                    // image latent) is updated from its first C channels
   const float* sigmas;              // [batch, 2] (sigma, sigma_next) per sample, or nullptr => out = v
   int C, Hl, Wl, ps;
   int sfa_mtiles;                   // block-scaled fp8: 128-row scale chunks per batch entry of the A operand's buffer (0: ceil(rows/128));

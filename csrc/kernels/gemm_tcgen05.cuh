@@ -442,6 +442,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tadd
     float dt = 0.f;
     if (euler) dt = p.sigmas[2 * b + 1] - p.sigmas[2 * b];
     const long long sample_elems = static_cast<long long>(p.C) * p.Hl * p.Wl;
+    const long long xin_elems = p.xin_bstride ? p.xin_bstride : sample_elems;
 #pragma unroll 1
     for (int c = 0; c < BN / 32; ++c) {
       if (n0 + c * 32 >= p.N) break;
@@ -460,7 +461,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tadd
             const long long pix = (static_cast<long long>(ch) * p.Hl + (hh * 2 + ph)) * p.Wl + ww * 2;
             float v0 = x[j], v1 = x[j + 1];
             if (euler) {
-              const float2 xi = unpack_bf16(*reinterpret_cast<const uint32_t*>(p.x_in + b * sample_elems + pix));
+              const float2 xi = unpack_bf16(*reinterpret_cast<const uint32_t*>(p.x_in + b * xin_elems + pix));
               v0 = xi.x + dt * v0;
               v1 = xi.y + dt * v1;
             }

@@ -36,7 +36,10 @@ def run(a, hb, model_name: str, build_model, host: dict, config: dict) -> int:
     ones = (1,) * (host["x"].dim() - 1)
 
     def euler(x, e, sig):
-        return x + (sig[:, 1] - sig[:, 0]).view(-1, *ones).to(x.dtype) * e
+        # image-to-video models see [noise | mask | image latent] and predict the noise channels only: the update covers
+        # those, and the conditioning channels are concatenated back for the next call, as ComfyUI's sampler does
+        nxt = x[:, :e.shape[1]] + (sig[:, 1] - sig[:, 0]).view(-1, *ones).to(x.dtype) * e
+        return nxt if nxt.shape[1] == x.shape[1] else torch.cat([nxt, x[:, e.shape[1]:]], 1)
 
     state = {"x": d["x"]}
 

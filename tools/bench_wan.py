@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Secondary benchmark: WAN2.2-A14B-sized video DiT (14.3 B params, random init), 720p x 16 frames (latent
 [16, 4, 90, 160] -> 14 400 tokens per sample), batch 8, bf16 - BASELINE.json config 4.  Same protocol and JSON line as
-bench.py (one step = forward + Euler update; device-timed, max over ranks; e2e with per-step H2D/D2H).
+bench.py (one step = forward + Euler update; device-timed, max over ranks; e2e with per-step H2D/D2H).  ``--i2v`` runs
+WAN2.2-I2V-A14B instead: the same layer stack on a 36-channel input ([noise 16 | mask 4 | image latent 16]).
 
-    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8]
+    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8] [--i2v]
     python -m torch.distributed.run --nproc-per-node 8 ... tools/bench_wan.py --gpus 8
 """
 from __future__ import annotations
@@ -17,13 +18,15 @@ sys.path.insert(0, ROOT)
 import bench as hb  # noqa: E402  (helpers: ClockSampler, timed, emit, dist_env, ...)
 
 MODEL_NAME = "WAN2.2-A14B video DiT 720p x 16 frames"
+I2V_MODEL_NAME = "WAN2.2-I2V-A14B video DiT 720p x 16 frames"
 
 
-def host_inputs(B, cap_len):
+def host_inputs(B, cap_len, i2v=False):
     import torch
     from comfyui_parallelanything_b200.models import wan
-    cfg = wan.wan22_a14b_params()
-    inp = wan.example_inputs(cfg, B, frames=16, height=720, width=1280, device="cpu", dtype=torch.bfloat16)
+    cfg = wan.wan22_i2v_a14b_params() if i2v else wan.wan22_a14b_params()
+    make = wan.i2v_inputs if i2v else wan.example_inputs
+    inp = make(cfg, B, frames=16, height=720, width=1280, device="cpu", dtype=torch.bfloat16)
     inp["sig"] = torch.tensor([[1.0, 0.875]] * B, dtype=torch.float32)
     return cfg, {k: v.pin_memory() for k, v in inp.items()}
 
@@ -33,14 +36,15 @@ def run_nodes(a) -> int:
     import torch
     import _nodes_bench
     from comfyui_parallelanything_b200.models import wan
-    cfg, host = host_inputs(a.batch, a.cap_len)
+    cfg, host = host_inputs(a.batch, a.cap_len, a.i2v)
+    name = I2V_MODEL_NAME if a.i2v else MODEL_NAME
 
     def build(lead):
         with torch.device(lead):
             return wan.WanModel(cfg, dtype=torch.bfloat16).eval()
 
-    return _nodes_bench.run(a, hb, MODEL_NAME, build, host,
-                            {"model": MODEL_NAME, "global_batch": a.batch, "text_len": a.cap_len, "baseline_config": 4})
+    return _nodes_bench.run(a, hb, name, build, host,
+                            {"model": name, "global_batch": a.batch, "text_len": a.cap_len, "baseline_config": 4})
 
 
 def main() -> int:
@@ -55,6 +59,7 @@ def main() -> int:
     ap.add_argument("--api", default="spmd", choices=["spmd", "nodes"],
                     help="nodes = ONE process through the ComfyUI node API, new latent tensor every step (batch 1 -> "
                          "sequence-parallel over all GPUs)")
+    ap.add_argument("--i2v", action="store_true", help="WAN2.2-I2V-A14B (36-channel input) instead of T2V")
     a = ap.parse_args()
     if a.api == "nodes":
         return run_nodes(a)
@@ -76,7 +81,7 @@ def main() -> int:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
     from comfyui_parallelanything_b200.models import wan
-    cfg, host = host_inputs(B, a.cap_len)
+    cfg, host = host_inputs(B, a.cap_len, a.i2v)
     result_host = torch.empty(B, 16, 4, 90, 160, dtype=torch.bfloat16).pin_memory()
     h2d = sum(v.numel() * v.element_size() for v in host.values())
     d2h = result_host.numel() * result_host.element_size()
@@ -149,8 +154,8 @@ def main() -> int:
             d = {k: v.to(lead) for k, v in host.items()}
             stage = {k: torch.empty_like(v, device=lead) for k, v in host.items()}
 
-            def euler(x, e, sig):
-                return x + (sig[:, 1] - sig[:, 0]).view(-1, 1, 1, 1, 1).to(x.dtype) * e
+            def euler(x, e, sig):       # I2V: the update covers the predicted noise channels of x
+                return x[:, :e.shape[1]] + (sig[:, 1] - sig[:, 0]).view(-1, 1, 1, 1, 1).to(x.dtype) * e
 
             def step_device():
                 with torch.no_grad():
@@ -190,7 +195,7 @@ def main() -> int:
                  "e2e": {"value": round(1000.0 / ms_e2e, 4), "unit": "steps/s", "ms_per_step": round(ms_e2e, 3),
                          "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
                  "output_finite": bool(torch.isfinite(result_host.float()).all().item()),
-                 "config": {"model": MODEL_NAME, "global_batch": B, "text_len": a.cap_len, "baseline_config": 4, "parallelism": par}})
+                 "config": {"model": I2V_MODEL_NAME if a.i2v else MODEL_NAME, "global_batch": B, "text_len": a.cap_len, "baseline_config": 4, "parallelism": par}})
     return 0
 
 

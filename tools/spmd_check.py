@@ -96,7 +96,8 @@ def bcast_check(rank, world, dev) -> int:
 
 
 def other_family(family, rank, world, dev) -> int:
-    """Same comparison for the SDXL-class UNet (``unet``) and the WAN video DiT (``wan``) engines."""
+    """Same comparison for the SDXL-class UNet (``unet``), Z-Image (``zimage``) and the WAN video DiT engines: ``wan``
+    (text-to-video, 16 latent channels) and ``wan_i2v`` (image-to-video: 36 input channels, 16 output channels)."""
     import torch
     import torch.distributed as dist
     from comfyui_parallelanything_b200.parallel import spmd
@@ -127,9 +128,13 @@ def other_family(family, rank, world, dev) -> int:
         from comfyui_parallelanything_b200.exec.wan_exec import WanExecutor
         from comfyui_parallelanything_b200.models import wan
         p = wan.wan_tiny_params()
+        make_inputs = wan.example_inputs
+        if family == "wan_i2v":
+            import dataclasses
+            p, make_inputs = dataclasses.replace(p, in_dim=36), wan.i2v_inputs
         torch.manual_seed(2)
         ex = WanExecutor(wan.WanModel(p).to(device=dev, dtype=torch.bfloat16).eval(), dev, cuda_graphs=True)
-        inp = wan.example_inputs(p, B, frames=8, height=128, width=192, device=dev, dtype=torch.bfloat16)
+        inp = make_inputs(p, B, frames=8, height=128, width=192, device=dev, dtype=torch.bfloat16)
         x, t, c = ex._prep(inp["x"], inp["timesteps"], inp["context"])
         order = [x, t, c, sig]
         want = ex.denoise_step(*order).clone()
