@@ -528,6 +528,21 @@ class ParallelEngine:
         self._io[key] = io
         return io
 
+    def _stage_conditioning(self, st: dict, name: str, buf: torch.Tensor, src: torch.Tensor) -> torch.Tensor:
+        """Copy the step-invariant conditioning ``src`` into its staging buffer only when it changed (another tensor, or
+        written in place since), so the replica's conditioning cache and its captured graph stay valid across steps."""
+        # a split chunk is a fresh view object every step: identify it by the tensor it was split from (the sampler's
+        # conditioning, which stays the same object) plus where and how large the chunk is
+        base = src._base if src._base is not None else src
+        ident = (id(base), base.data_ptr(), base._version, src.data_ptr(), tuple(src.shape))
+        key = "ctx_src" if name == "ctx" else name + "_src"
+        if not self.config.cache_conditioning or st.get(key) is None or st[key][0] != ident:
+            buf.copy_(src, non_blocking=True)           # conditioning changed (or first step)
+            st[key] = (ident, base)                     # keep the source alive: id/ptr stay unique
+        else:
+            self.metrics.incr("cond_cache_hits")
+        return buf
+
     def _data_parallel_fused(self, step, batch, active, offs, x, t_chunks, c_chunks, k_chunks, lead_stream):
         """Every replica's FIRST kernel loads its latent shard from the lead GPU's staging buffer (NVLink peer loads)
         and its LAST kernel stores its output rows at their final offset in the lead GPU's output buffer; the host only
@@ -553,18 +568,14 @@ class ParallelEngine:
                     t_in = st["t"]
                 c_in = c_chunks[i]
                 if st["ctx"] is not None:
-                    src = c_in
-                    ident = (id(src), src.data_ptr(), src._version)
-                    if not self.config.cache_conditioning or st["ctx_src"] is None or st["ctx_src"][0] != ident:
-                        st["ctx"].copy_(src, non_blocking=True)           # conditioning changed (or first step)
-                        st["ctx_src"] = (ident, src)                      # keep src alive: id/ptr stay unique
-                    else:
-                        self.metrics.incr("cond_cache_hits")
-                    c_in = st["ctx"]
+                    c_in = self._stage_conditioning(st, "ctx", st["ctx"], c_in)
                 k_in = {}
+                cond_kw = getattr(slot.replica, "conditioning_kwargs", ())
                 for k, v in k_chunks[i].items():
                     buf = st["kw"].get(k)
-                    if buf is not None:
+                    if buf is not None and k in cond_kw:
+                        k_in[k] = self._stage_conditioning(st, "kw:" + k, buf, v)
+                    elif buf is not None:
                         buf.copy_(v, non_blocking=True)
                         k_in[k] = buf
                     else:
@@ -649,7 +660,7 @@ class ParallelEngine:
         t0 = time.perf_counter()
         xs, out = io["x"], io["out"]
         xs.copy_(x, non_blocking=True)
-        wss = sp.workspace(*sp.geometry(x, context))
+        wss = sp.workspace(*sp.geometry(x, context, kwargs))
         for g, (slot, st) in enumerate(zip(self.slots, io["slots"])):
             with torch.cuda.device(slot.device), torch.cuda.stream(slot.stream), torch.no_grad():
                 slot.stream.wait_stream(lead_stream)

@@ -101,12 +101,17 @@ def builder_for(module: nn.Module) -> Optional[Callable]:
             from .flux_exec import build_flux_executor
             return build_flux_executor
     elif fam == "wan":
-        # in_dim 36: WAN2.2 image-to-video ([noise | mask | image latent]).  Models with a CLIP image embedding keep the
-        # torch replica: the executor has no image cross-attention and must not drop ``clip_fea``
+        # in_dim 36: WAN2.2 image-to-video ([noise | mask | image latent]).  A CLIP image embedding (WAN2.1 I2V / FLF2V,
+        # Fun-InP) gets the executor with the image cross-attention only when its structure is complete; anything else
+        # with ``img_emb`` keeps the torch replica, which must not drop ``clip_fea``
         if (p.dim // p.num_heads == 128 and tuple(p.patch_size) == (1, 2, 2) and p.in_dim in (16, 36)
-                and p.out_dim == 16 and not p.has_img_emb):
-            from .wan_exec import build_wan_executor
-            return build_wan_executor
+                and p.out_dim == 16):
+            if not p.has_img_emb and not p.img_cross_attn:
+                from .wan_exec import build_wan_executor
+                return build_wan_executor
+            if p.clip_ok and p.clip_dim % 64 == 0:
+                from .wan_exec import build_wan_clip_executor
+                return build_wan_clip_executor
     elif fam == "zimage":
         if p.dim // p.n_heads == 128 and p.patch_size == 2 and p.in_channels == 16 and p.ffn_hidden % 32 == 0:
             from .zimage_exec import build_zimage_executor

@@ -107,6 +107,17 @@ class DiTExecutor(nn.Module):
     def _geometry(shape, context) -> tuple:
         return (shape[0],) + tuple(shape[2:]) + (context.shape[1],)
 
+    @staticmethod
+    def _conditioning(inputs: tuple) -> tuple:
+        """The step inputs that ``_geometry``, ``_prepare_ctx`` and ``_cond_sig`` take: the context (WAN with CLIP image
+        conditioning adds ``clip_fea``)."""
+        return inputs[1:2]
+
+    @staticmethod
+    def _cond_sig(context) -> tuple:
+        """What ``_prepare_ctx`` stores in ``ws["ctx_sig"]`` for this conditioning."""
+        return conditioning_sig(context)
+
     def _mod(self, ws, key, idx: int):
         """``idx``-th modulation vector of block ``key`` in the step's modulation table (each is as wide as ``X``)."""
         width = ws["X"].shape[-1]
@@ -130,19 +141,19 @@ class DiTExecutor(nn.Module):
     def _forward(self, x, *step_inputs):
         with torch.cuda.device(self.device):
             x, *inputs = self._prep(x, *step_inputs)
-            ws = self.workspace(*self._geometry(x.shape, inputs[1]))
+            ws = self.workspace(*self._geometry(x.shape, *self._conditioning(inputs)))
             out = torch.empty(self.out_shape(tuple(x.shape)), dtype=x.dtype, device=x.device)
             if self._prepare_ctx is not None:
-                self._prepare_ctx(ws, inputs[1])
+                self._prepare_ctx(ws, *self._conditioning(inputs))
             self._run(ws, x.data_ptr(), *inputs, out)
             return out
 
     def _forward_shard(self, x_src_ptr: int, shape, out_ptr: int, out_sample_off: int, *step_inputs) -> None:
         with torch.cuda.device(self.device):
             key, inputs = self._shard_args(x_src_ptr, shape, out_ptr, out_sample_off, *step_inputs)
-            ws = self.workspace(*self._geometry(shape, inputs[1]))
+            ws = self.workspace(*self._geometry(shape, *self._conditioning(inputs)))
             if self._prepare_ctx is not None:
-                self._prepare_ctx(ws, inputs[1])
+                self._prepare_ctx(ws, *self._conditioning(inputs))
             self._graphs.run(key, lambda: self._run(ws, x_src_ptr, *inputs, None, out_ptr=out_ptr,
                                                     out_sample_off=out_sample_off))
 
@@ -150,19 +161,19 @@ class DiTExecutor(nn.Module):
         with torch.cuda.device(self.device):
             key, inputs = self._shard_args(x_src_ptr, shape, out_ptr, out_sample_off, *step_inputs)
             if self._prepare_ctx is not None:
-                ws = self.workspace(*self._geometry(shape, inputs[1]))
-                if ws["ctx_sig"] != conditioning_sig(inputs[1]):
+                ws = self.workspace(*self._geometry(shape, *self._conditioning(inputs)))
+                if ws["ctx_sig"] != self._cond_sig(*self._conditioning(inputs)):
                     return 0                # conditioning changed: take the Python path once (eager precompute)
         return self._graphs.exec_handle(key)
 
     def _denoise(self, x, inputs: tuple, sigmas, out, out_ptr, out_sample_off, x_src_ptr, t_src_ptr, **src_ptrs):
         """``src_ptrs``: peer pointers of family-specific per-sample inputs, passed on to ``_run`` (FLUX: ``g_ptr``)."""
         with torch.cuda.device(self.device):
-            ws = self.workspace(*self._geometry(x.shape, inputs[1]))
+            ws = self.workspace(*self._geometry(x.shape, *self._conditioning(inputs)))
             if out is None and out_ptr is None:
                 out = ws["OUT"]
             if self._prepare_ctx is not None:
-                self._prepare_ctx(ws, inputs[1])
+                self._prepare_ctx(ws, *self._conditioning(inputs))
 
             def body():
                 self._run(ws, x_src_ptr if x_src_ptr is not None else x.data_ptr(), *inputs, out, x_in=x, sigmas=sigmas,

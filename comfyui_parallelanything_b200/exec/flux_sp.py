@@ -88,7 +88,7 @@ class FluxUlysses(UlyssesBase):
         H, Wd, Lt = x.shape[2], x.shape[3], context.shape[1]
         return H % 2 == 0 and Wd % 2 == 0 and Lt % n == 0 and ((H // 2) * (Wd // 2)) % n == 0 and Lt >= n
 
-    def geometry(self, x, context) -> tuple:
+    def geometry(self, x, context, kwargs=None) -> tuple:
         return (x.shape[2], x.shape[3], context.shape[1])
 
     def io_key(self, x, context, kwargs) -> tuple:

@@ -126,13 +126,50 @@ def _wan(m: nn.Module) -> Optional[SimpleNamespace]:
         heads = getattr(b0.self_attn, "num_heads", None) or dim // 128
     patch = tuple(int(v) for v in pe.shape[2:])
     out_dim = int(m.head.head.weight.shape[0]) // (patch[0] * patch[1] * patch[2])
+    clip_dim, clip_pos, clip_ok = _wan_clip(m, dim)
     return SimpleNamespace(
         in_dim=int(pe.shape[1]), out_dim=out_dim, dim=dim, ffn_dim=int(b0.ffn[0].weight.shape[0]), num_heads=int(heads),
         num_layers=len(m.blocks), text_dim=int(m.text_embedding[0].weight.shape[1]),
         text_len=int(_hint(m, "text_len", default=512)), freq_dim=int(m.time_embedding[0].weight.shape[1]),
         patch_size=patch, eps=float(_hint(m, "eps", default=1e-6)),
         # CLIP image projection of WAN2.1 I2V / FLF2V and the Fun models: their blocks add an image cross-attention
-        has_img_emb=getattr(m, "img_emb", None) is not None)
+        has_img_emb=getattr(m, "img_emb", None) is not None,
+        # clip_ok: ``img_emb.proj`` is exactly LayerNorm, Linear, GELU, Linear, LayerNorm and every block's cross-attention
+        # has ``k_img`` / ``v_img`` / ``norm_k_img`` - the structure the native image cross-attention implements
+        clip_dim=clip_dim, clip_pos_tokens=clip_pos, clip_ok=clip_ok,
+        img_cross_attn=any(hasattr(blk.cross_attn, "k_img") for blk in m.blocks))
+
+
+def _wan_clip(m: nn.Module, dim: int) -> Tuple[int, int, bool]:
+    """(clip_dim, clip_pos_tokens, complete) of WAN's CLIP image branch; (0, 0, False) when there is none."""
+    emb = getattr(m, "img_emb", None)
+    proj = getattr(emb, "proj", None)
+    if emb is None or not isinstance(proj, nn.Sequential) or len(proj) != 5:
+        return 0, 0, False
+    n0, l1, act, l3, n4 = proj
+    if not (isinstance(n0, nn.LayerNorm) and isinstance(n4, nn.LayerNorm) and isinstance(act, nn.GELU)
+            and getattr(act, "approximate", "none") == "none" and _has_linear(l1) and _has_linear(l3)
+            and n0.elementwise_affine and n4.elementwise_affine):
+        return 0, 0, False
+    clip_dim = int(l1.weight.shape[1])
+    if (tuple(n0.weight.shape) != (clip_dim,) or tuple(l1.weight.shape) != (clip_dim, clip_dim)
+            or tuple(l3.weight.shape) != (dim, clip_dim) or tuple(n4.weight.shape) != (dim,)):
+        return 0, 0, False
+    pos = getattr(emb, "emb_pos", None)
+    clip_pos = 0
+    if isinstance(pos, torch.Tensor):
+        if pos.dim() != 3 or pos.shape[2] != clip_dim:
+            return 0, 0, False
+        clip_pos = int(pos.shape[1])
+    for blk in m.blocks:
+        ca = blk.cross_attn
+        if not (_has_linear(getattr(ca, "k_img", None)) and _has_linear(getattr(ca, "v_img", None))
+                and isinstance(getattr(ca, "norm_k_img", None), nn.Module)
+                and tuple(ca.k_img.weight.shape) == (dim, dim) and tuple(ca.v_img.weight.shape) == (dim, dim)
+                and ca.k_img.bias is not None and ca.v_img.bias is not None
+                and tuple(norm_scale(ca.norm_k_img).shape) == (dim,)):
+            return clip_dim, clip_pos, False
+    return clip_dim, clip_pos, True
 
 
 # --------------------------------------------------------------------------------------------- Z-Image / NextDiT

@@ -52,7 +52,7 @@ class UlyssesBase:
     def accepts(self, x, context) -> bool:
         raise NotImplementedError
 
-    def geometry(self, x, context) -> tuple:
+    def geometry(self, x, context, kwargs=None) -> tuple:
         raise NotImplementedError
 
     def out_shape(self, x) -> tuple:

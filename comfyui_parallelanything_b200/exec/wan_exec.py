@@ -142,6 +142,10 @@ class WanExecutor(DiTExecutor):
         ws["ctx_sig"] = sig
         return 2 + 2 * self.n_blocks
 
+    def _cross_attention(self, ws, i: int, out) -> None:
+        """Block ``i``'s cross-attention of the step's ``CQ`` rows against the cached text K/V, into ``out``."""
+        ops.attention(self._heads(ws["CQ"], 0, 1), self._heads(ws["CKV"][i], 0, 2), self._heads(ws["CKV"][i], 1, 2), out=out)
+
     def _run(self, ws, x_ptr, t, ctx, out, x_in=None, sigmas=None, out_ptr=None, out_sample_off=0, t_ptr=None,
              x_copy=None):
         W, dim, B, L = self.W, self.dim, ws["B"], ws["L"]
@@ -176,8 +180,7 @@ class WanExecutor(DiTExecutor):
             ops.layernorm_modulate(X, XM, gamma=W[f"b{i}.n3.g"], beta=W[f"b{i}.n3.b"], eps=self.eps)
             n += block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
             C.rms_rope(ws["CQ"], W[f"b{i}.cnq"], None, self.eps)
-            ops.attention(self._heads(ws["CQ"], 0, 1), self._heads(ws["CKV"][i], 0, 2), self._heads(ws["CKV"][i], 1, 2),
-                          out=ATT)
+            self._cross_attention(ws, i, ATT)
             n += block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
             # ---- FFN
             ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=self.eps)
@@ -201,3 +204,135 @@ class WanExecutor(DiTExecutor):
 
 def build_wan_executor(model: nn.Module, device, **kw) -> WanExecutor:
     return WanExecutor(model, device, **kw)
+
+
+class WanClipExecutor(WanExecutor):
+    """WAN2.1 I2V / FLF2V and Fun-InP: ``WanExecutor`` plus the CLIP image branch.
+
+    The image projection (``img_emb``: LayerNorm, Linear, erf-GELU, Linear, LayerNorm, FLF2V's ``emb_pos``) and every
+    block's image K/V (``k_img`` / ``v_img`` + ``norm_k_img``) depend on ``clip_fea`` only: like the text K/V they run
+    eagerly when the text or the image conditioning changed and sit in the workspace's fixed ``CKVI`` buffers.  Per step
+    each block's cross-attention is ONE two-source attention launch, ``softmax(q Kt^T) Vt + softmax(q Ki^T) Vi``.
+    ``clip_fea=None`` reproduces the reference model: the image branch then attends over the text tokens.
+    Step entry points take ``clip_fea`` after ``context`` (``denoise_step(x, t, ctx, clip_fea, sigmas, ...)``)."""
+
+    conditioning_kwargs = ("clip_fea",)
+
+    def __init__(self, model: "wan_model.WanModel", device, cuda_graphs: bool = False, fp8: bool = False):
+        super().__init__(model, device, cuda_graphs=cuda_graphs, fp8=fp8)
+        p, d, W = self.params, self.device, self.W
+        if not p.clip_ok:
+            raise ValueError("WanClipExecutor needs img_emb.proj = (LayerNorm, Linear, GELU, Linear, LayerNorm) and "
+                             "k_img / v_img / norm_k_img in every block")
+        self.clip_dim, self.clip_pos_tokens = p.clip_dim, p.clip_pos_tokens
+        proj = model.img_emb.proj
+        W["img.n0.g"], W["img.n0.b"] = _bf(proj[0].weight, d), _bf(proj[0].bias, d)
+        W["img.l1.w"], W["img.l1.b"] = _bf(proj[1].weight, d), _bf(proj[1].bias, d)
+        W["img.l3.w"], W["img.l3.b"] = _bf(proj[3].weight, d), _bf(proj[3].bias, d)
+        W["img.n4.g"], W["img.n4.b"] = _bf(proj[4].weight, d), _bf(proj[4].bias, d)
+        W["img.emb_pos"] = _bf(model.img_emb.emb_pos, d) if self.clip_pos_tokens else None
+        self.img_eps = (float(proj[0].eps), float(proj[4].eps))
+        for i, blk in enumerate(model.blocks):
+            ca = blk.cross_attn
+            W[f"b{i}.ckvi.w"] = torch.cat([_bf(ca.k_img.weight, d), _bf(ca.v_img.weight, d)], 0).contiguous()
+            W[f"b{i}.ckvi.b"] = torch.cat([_bf(ca.k_img.bias, d), _bf(ca.v_img.bias, d)], 0).contiguous()
+            W[f"b{i}.cnki"] = _bf(recognize.norm_scale(ca.norm_k_img), d)
+
+    # ------------------------------------------------------------------ geometry / conditioning
+    @staticmethod
+    def _conditioning(inputs: tuple) -> tuple:
+        return inputs[1:3]
+
+    @staticmethod
+    def _geometry(shape, context, clip_fea=None) -> tuple:
+        """+ ``Li``, the number of CLIP tokens (0: no ``clip_fea``, the image K/V then come from the text)."""
+        return (shape[0],) + tuple(shape[2:]) + (context.shape[1], clip_fea.shape[1] if clip_fea is not None else 0)
+
+    @staticmethod
+    def _cond_sig(context, clip_fea=None) -> tuple:
+        return conditioning_sig(context), (conditioning_sig(clip_fea) if clip_fea is not None else None)
+
+    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int, Li: int = 0) -> dict:
+        ws = super()._new_workspace(B, T, H, Wd, Lc)
+        e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=self.device)  # noqa: E731
+        ws["Li"] = Li
+        if Li:
+            ws["CLIP_H"], ws["CLIP"] = e(B, Li, self.clip_dim), e(B, Li, self.dim)
+        ws["CKVI"] = [e(B, Li or Lc, 2 * self.dim) for _ in range(self.n_blocks)]
+        return ws
+
+    def _inputs(self, B: int, timesteps, context, clip_fea=None) -> tuple:
+        timesteps, context = super()._inputs(B, timesteps, context)
+        if clip_fea is not None:
+            if clip_fea.shape[0] != context.shape[0]:
+                raise ValueError(f"clip_fea has batch {clip_fea.shape[0]}, context has {context.shape[0]}")
+            if clip_fea.dim() != 3 or clip_fea.shape[2] != self.clip_dim:
+                raise ValueError(f"clip_fea must be [B, Li, {self.clip_dim}], got {tuple(clip_fea.shape)}")
+            clip_fea = clip_fea.to(device=self.device, dtype=torch.bfloat16).contiguous()
+        return timesteps, context, clip_fea
+
+    def _prep(self, x, timesteps, context, clip_fea=None):
+        x = x.to(device=self.device, dtype=torch.bfloat16).contiguous()
+        return (x,) + self._inputs(x.shape[0], timesteps, context, clip_fea)
+
+    def _prepare_ctx(self, ws, ctx, clip_fea=None) -> int:
+        """Text path of ``WanExecutor._prepare_ctx`` plus the image projection and every block's image K/V (+ k
+        RMSNorm), all eager and only when the text or the CLIP conditioning changed."""
+        sig = self._cond_sig(ctx, clip_fea)
+        if ws["ctx_sig"] == sig:
+            return 0
+        ws["ctx_sig"] = None
+        n = super()._prepare_ctx(ws, ctx)
+        W, dim = self.W, self.dim
+        C = ops.require()
+        src = ws["CTX"]
+        if clip_fea is not None:
+            e = clip_fea
+            if W["img.emb_pos"] is not None:       # FLF2V: clip_fea[:, :P] + emb_pos[:, :Li] (<= 514 x 1280 elements)
+                e = (e[:, :W["img.emb_pos"].shape[1]] + W["img.emb_pos"][:, :e.shape[1]]).contiguous()
+            ln = ops.layernorm_modulate(e, gamma=W["img.n0.g"], beta=W["img.n0.b"], eps=self.img_eps[0])
+            ops.gemm(ln, W["img.l1.w"], "gelu_erf", out=ws["CLIP_H"], bias=W["img.l1.b"])
+            t = torch.empty_like(ws["CLIP"])
+            ops.gemm(ws["CLIP_H"], W["img.l3.w"], "bias", out=t, bias=W["img.l3.b"])
+            ops.layernorm_modulate(t, ws["CLIP"], gamma=W["img.n4.g"], beta=W["img.n4.b"], eps=self.img_eps[1])
+            src = ws["CLIP"]
+            n += 4
+        for i in range(self.n_blocks):
+            ops.gemm(src, W[f"b{i}.ckvi.w"], "bias", out=ws["CKVI"][i], bias=W[f"b{i}.ckvi.b"])
+            C.rms_rope(ws["CKVI"][i][:, :, :dim], W[f"b{i}.cnki"], None, self.eps)
+        ws["ctx_sig"] = sig
+        return n + 2 * self.n_blocks
+
+    def _cross_attention(self, ws, i: int, out) -> None:
+        ckv, ckvi = ws["CKV"][i], ws["CKVI"][i]
+        ops.attention(self._heads(ws["CQ"], 0, 1), self._heads(ckv, 0, 2), self._heads(ckv, 1, 2), out=out,
+                      kv2=(self._heads(ckvi, 0, 2), self._heads(ckvi, 1, 2)))
+
+    def _run(self, ws, x_ptr, t, ctx, clip_fea, out, **kw):    # clip_fea is consumed by _prepare_ctx
+        return super()._run(ws, x_ptr, t, ctx, out, **kw)
+
+    # ------------------------------------------------------------------ step entry points
+    @torch.no_grad()
+    def forward(self, x, timesteps, context=None, clip_fea=None, transformer_options=None, **kwargs):
+        return self._forward(x, timesteps, context, clip_fea)
+
+    @torch.no_grad()
+    def forward_shard(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int, clip_fea=None,
+                      **_ignored):
+        """``DiTExecutor.forward_shard`` with the CLIP image features."""
+        self._forward_shard(x_src_ptr, shape, out_ptr, out_sample_off, timesteps, context, clip_fea)
+
+    def shard_graph_handle(self, x_src_ptr: int, shape, timesteps, context, out_ptr: int, out_sample_off: int,
+                           clip_fea=None, **_ignored) -> int:
+        return self._graph_handle(x_src_ptr, shape, out_ptr, out_sample_off, timesteps, context, clip_fea)
+
+    @torch.no_grad()
+    def denoise_step(self, x, timesteps, context, clip_fea, sigmas, out=None, out_ptr=None, out_sample_off=0,
+                     x_src_ptr: Optional[int] = None, t_src_ptr: Optional[int] = None):
+        """``DiTExecutor.denoise_step`` with the CLIP image features (``None``: image branch over the text)."""
+        return self._denoise(x, (timesteps, context, clip_fea), sigmas, out, out_ptr, out_sample_off, x_src_ptr,
+                             t_src_ptr)
+
+
+def build_wan_clip_executor(model: nn.Module, device, **kw) -> WanClipExecutor:
+    return WanClipExecutor(model, device, **kw)

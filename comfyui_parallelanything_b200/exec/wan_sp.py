@@ -11,7 +11,8 @@ latency as one GPU.  Here, as for FLUX (``flux_sp.py``):
     [all tokens, my heads] before it and one turns the result back after it (csrc/comm/sp_a2a.cu, device-side flag
     handshake, epochs in device memory -> the whole share of a GPU is one CUDA graph);
   * text cross-attention needs no exchange: every GPU holds the (step-invariant, cached) K/V of the 512 text tokens and
-    attends with its own query tokens;
+    attends with its own query tokens; WAN2.1 I2V / FLF2V hold the image K/V of the CLIP tokens the same way and run the
+    executor's two-source cross-attention;
   * the head GEMM's unpatchify epilogue stores each GPU's token rows straight into the lead GPU's output (NVLink).
 """
 from __future__ import annotations
@@ -84,11 +85,39 @@ class WanUlysses(UlyssesBase):
     def out_shape(self, x) -> tuple:
         return self.ex[0].out_shape(tuple(x.shape))
 
-    def geometry(self, x, context) -> tuple:
-        return (x.shape[2], x.shape[3], x.shape[4], context.shape[1])
+    def _clip(self, kwargs):
+        """``clip_fea`` of the step when the replicas take CLIP image conditioning, else None."""
+        if not getattr(self.ex[0], "conditioning_kwargs", ()):
+            return None
+        c = kwargs.get("clip_fea")
+        return c if isinstance(c, torch.Tensor) else None
 
-    def workspace(self, T: int, H: int, Wd: int, Lc: int) -> list:
-        key = (T, H, Wd, Lc)
+    def slot_buffers(self, device, x, context, kwargs) -> dict:
+        st = super().slot_buffers(device, x, context, kwargs)
+        clip = self._clip(kwargs)
+        if clip is not None:
+            st["clip"], st["clip_src"] = torch.empty(tuple(clip.shape), dtype=torch.bfloat16, device=device), None
+        return st
+
+    def stage(self, st: dict, timesteps, context, kwargs, cache_conditioning: bool) -> None:
+        super().stage(st, timesteps, context, kwargs, cache_conditioning)
+        clip = self._clip(kwargs)
+        if clip is not None:
+            ident = (id(clip), clip.data_ptr(), clip._version)
+            if not cache_conditioning or st["clip_src"] is None or st["clip_src"][0] != ident:
+                st["clip"].copy_(clip, non_blocking=True)
+                st["clip_src"] = (ident, clip)
+
+    def io_key(self, x, context, kwargs) -> tuple:
+        clip = self._clip(kwargs)
+        return super().io_key(x, context, kwargs) + ((tuple(clip.shape),) if clip is not None else ())
+
+    def geometry(self, x, context, kwargs=None) -> tuple:
+        clip = self._clip(kwargs or {})
+        return (x.shape[2], x.shape[3], x.shape[4], context.shape[1], clip.shape[1] if clip is not None else 0)
+
+    def workspace(self, T: int, H: int, Wd: int, Lc: int, Li: int = 0) -> list:
+        key = (T, H, Wd, Lc, Li)
         got = self._ws.get(key)
         if got is not None:
             return got
@@ -115,6 +144,12 @@ class WanUlysses(UlyssesBase):
             ws["CTX_H"], ws["CTX"] = e(1, Lc, dim), e(1, Lc, dim)
             ws["CQ"] = e(1, Ll, dim)
             ws["CKV"] = [e(1, Lc, 2 * dim) for _ in range(ex.n_blocks)]
+            if getattr(ex, "conditioning_kwargs", ()):
+                # CLIP image branch: projection scratch and every block's image K/V (from the text without clip_fea)
+                ws["Li"] = Li
+                if Li:
+                    ws["CLIP_H"], ws["CLIP"] = e(1, Li, ex.clip_dim), e(1, Li, dim)
+                ws["CKVI"] = [e(1, Li or Lc, 2 * dim) for _ in range(ex.n_blocks)]
             ws["ROPE"] = ex.rope(T, H, Wd)[g * Ll:(g + 1) * Ll].contiguous()       # RoPE rows of MY tokens
             ws["ctx_sig"] = None
             wss.append(ws)
@@ -127,8 +162,12 @@ class WanUlysses(UlyssesBase):
         return wss
 
     def pre_step(self, g: int, wss, st: dict) -> None:
-        # text embedding + every block's cross-attention K/V: only when the conditioning changed, never in the graph
-        self.ex[g]._prepare_ctx(wss[g], st["ctx"])
+        # text embedding + every block's cross-attention K/V (and the image K/V of a CLIP model): only when the
+        # conditioning changed, never in the graph
+        if "CKVI" in wss[g]:
+            self.ex[g]._prepare_ctx(wss[g], st["ctx"], st.get("clip"))
+        else:
+            self.ex[g]._prepare_ctx(wss[g], st["ctx"])
 
     # ------------------------------------------------------------------ one GPU's share of the step
     def run_rank(self, g: int, wss, x_ptr: int, st: dict, out_ptr: int) -> int:
@@ -172,11 +211,11 @@ class WanUlysses(UlyssesBase):
             self._exchange(g, ws, slot + 1, "ATT")
             slot += 2
             nl += 8 + block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2))
-            # ---- text cross attention: my query tokens against the replicated text K/V
+            # ---- cross attention: my query tokens against the replicated text (and image) K/V
             ops.layernorm_modulate(X, XM, gamma=W[f"b{i}.n3.g"], beta=W[f"b{i}.n3.b"], eps=ex.eps)
             nl += block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
             C.rms_rope(ws["CQ"], W[f"b{i}.cnq"], None, ex.eps)
-            ops.attention(ex._heads(ws["CQ"], 0, 1), ex._heads(ws["CKV"][i], 0, 2), ex._heads(ws["CKV"][i], 1, 2), out=ATT)
+            ex._cross_attention(ws, i, ATT)
             nl += 3 + block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
             # ---- FFN
             ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=ex.eps)

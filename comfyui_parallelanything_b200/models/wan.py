@@ -36,6 +36,8 @@ class WanParams:
     freq_dim: int = 256
     patch_size: Tuple[int, int, int] = (1, 2, 2)
     eps: float = 1e-6
+    clip_dim: int = 0               # CLIP image feature width (1280) of WAN2.1 I2V / FLF2V / Fun-InP; 0 = no image branch
+    clip_pos_tokens: int = 0        # FLF2V: learned position embedding over 2 x 257 CLIP tokens (514)
 
 
 def wan22_a14b_params() -> WanParams:
@@ -46,6 +48,17 @@ def wan22_i2v_a14b_params() -> WanParams:
     """WAN2.2-I2V-A14B: the T2V layer stack with a 36-channel input ([noise 16 | mask 4 | image latent 16], concatenated
     by the sampler before every call) and the 16 noise channels as output."""
     return WanParams(in_dim=36)
+
+
+def wan21_i2v_14b_params() -> WanParams:
+    """WAN2.1-I2V-14B (480p and 720p): the A14B layer stack, 36-channel input and a CLIP image cross-attention in every
+    block (257 image tokens of width 1280)."""
+    return WanParams(in_dim=36, clip_dim=1280)
+
+
+def wan21_flf2v_14b_params() -> WanParams:
+    """WAN2.1-FLF2V-14B (first and last frame): as I2V, with 2 x 257 CLIP tokens and their position embedding."""
+    return WanParams(in_dim=36, clip_dim=1280, clip_pos_tokens=514)
 
 
 def wan_tiny_params() -> WanParams:
@@ -93,6 +106,48 @@ class WanCrossAttention(WanSelfAttention):
         return self.o(o.transpose(1, 2).reshape(b, s, n * d))
 
 
+class WanI2VCrossAttention(WanCrossAttention):
+    """Text plus CLIP image cross-attention of WAN2.1 I2V / FLF2V (ComfyUI ``comfy/ldm/wan/model.py``,
+    ``WanI2VCrossAttention``): ``o(attn(q, norm_k(k(txt)), v(txt)) + attn(q, norm_k_img(k_img(img)), v_img(img)))`` with
+    ``img = context[:, :context_img_len]`` and ``txt = context[:, context_img_len:]``.  ``context_img_len = None`` makes
+    both slices the whole context, so the image branch then attends over the text tokens too."""
+
+    def __init__(self, dim: int, num_heads: int, eps: float):
+        super().__init__(dim, num_heads, eps)
+        self.k_img, self.v_img = nn.Linear(dim, dim), nn.Linear(dim, dim)
+        self.norm_k_img = WanRMSNorm(dim, eps)
+
+    def forward(self, x, context, context_img_len=None):  # type: ignore[override]
+        img = context[:, :context_img_len]
+        txt = context[:, context_img_len:]
+        b, s, _ = x.shape
+        n, d = self.num_heads, self.head_dim
+        q = self.norm_q(self.q(x)).view(b, s, n, d).transpose(1, 2)
+
+        def attend(k, v):
+            return F.scaled_dot_product_attention(q, k.view(b, -1, n, d).transpose(1, 2), v.view(b, -1, n, d).transpose(1, 2))
+
+        o = attend(self.norm_k(self.k(txt)), self.v(txt)) + attend(self.norm_k_img(self.k_img(img)), self.v_img(img))
+        return self.o(o.transpose(1, 2).reshape(b, s, n * d))
+
+
+class WanImageProjection(nn.Module):
+    """ComfyUI's ``MLPProj``: CLIP vision features [B, Li, 1280] -> [B, Li, dim] image context tokens.
+    ``proj = LayerNorm, Linear, GELU (exact erf), Linear, LayerNorm`` (both norms affine); FLF2V adds ``emb_pos``
+    [1, 514, 1280], applied as ``clip_fea[:, :P] + emb_pos[:, :Li]`` with ``P = emb_pos.shape[1]``."""
+
+    def __init__(self, clip_dim: int, dim: int, pos_tokens: int = 0):
+        super().__init__()
+        self.proj = nn.Sequential(nn.LayerNorm(clip_dim), nn.Linear(clip_dim, clip_dim), nn.GELU(),
+                                  nn.Linear(clip_dim, dim), nn.LayerNorm(dim))
+        self.emb_pos = nn.Parameter(torch.randn(1, pos_tokens, clip_dim) * 0.02) if pos_tokens else None
+
+    def forward(self, clip_fea):
+        if self.emb_pos is not None:
+            clip_fea = clip_fea[:, :self.emb_pos.shape[1]] + self.emb_pos[:, :clip_fea.shape[1]].to(clip_fea.dtype)
+        return self.proj(clip_fea)
+
+
 class WanAttentionBlock(nn.Module):
     def __init__(self, dim: int, ffn_dim: int, num_heads: int, eps: float):
         super().__init__()
@@ -104,11 +159,14 @@ class WanAttentionBlock(nn.Module):
         self.ffn = nn.Sequential(nn.Linear(dim, ffn_dim), nn.GELU(approximate="tanh"), nn.Linear(ffn_dim, dim))
         self.modulation = nn.Parameter(torch.randn(1, 6, dim) / dim ** 0.5)
 
-    def forward(self, x, e, freqs, context):
+    def forward(self, x, e, freqs, context, context_img_len=None):
         e = (self.modulation.to(e.dtype) + e).chunk(6, dim=1)
         y = self.self_attn(self.norm1(x) * (1 + e[1]) + e[0], freqs)
         x = x + y * e[2]
-        x = x + self.cross_attn(self.norm3(x), context)
+        if isinstance(self.cross_attn, WanI2VCrossAttention):
+            x = x + self.cross_attn(self.norm3(x), context, context_img_len)
+        else:
+            x = x + self.cross_attn(self.norm3(x), context)
         y = self.ffn(self.norm2(x) * (1 + e[4]) + e[3])
         return x + y * e[5]
 
@@ -146,6 +204,14 @@ class WanModel(nn.Module):
         self.head = Head(p.dim, p.out_dim, self.patch_size, p.eps)
         d = p.dim // p.num_heads
         self.rope_embedder = EmbedND(dim=d, theta=10000, axes_dim=[d - 4 * (d // 6), 2 * (d // 6), 2 * (d // 6)])
+        self.img_emb = None
+        if p.clip_dim:
+            # created after every other module, so models without the image branch draw the same random numbers
+            self.img_emb = WanImageProjection(p.clip_dim, p.dim, p.clip_pos_tokens)
+            for blk in self.blocks:
+                ca = WanI2VCrossAttention(p.dim, p.num_heads, p.eps)
+                ca.load_state_dict(blk.cross_attn.state_dict(), strict=False)
+                blk.cross_attn = ca
         if dtype is not None or device is not None:
             self.to(device=device, dtype=dtype)
 
@@ -173,9 +239,13 @@ class WanModel(nn.Module):
         e = self.time_embedding(timestep_embedding(timesteps, self.freq_dim, time_factor=1.0).to(x.dtype))
         e0 = self.time_projection(e).unflatten(1, (6, self.dim))
         ctx = self.text_embedding(context)
+        context_img_len = None
+        if clip_fea is not None and self.img_emb is not None:
+            ctx = torch.cat([self.img_emb(clip_fea), ctx], 1)
+            context_img_len = clip_fea.shape[-2]
         freqs = self.rope_embedder(self.make_ids(x.shape[0], *grid, x.device))
         for blk in self.blocks:
-            x = blk(x, e0, freqs, ctx)
+            x = blk(x, e0, freqs, ctx, context_img_len)
         x = self.head(x, e)
         return self.unpatchify(x, grid)
 
@@ -208,3 +278,14 @@ def i2v_inputs(params: WanParams, batch: int, frames: int = 16, height: int = 72
     t = (torch.rand(batch, generator=g) * 1000).to(device=device, dtype=dtype)
     ctx = torch.randn(batch, params.text_len, params.text_dim, generator=g).to(device=device, dtype=dtype)
     return dict(x=x, timesteps=t, context=ctx)
+
+
+def clip_inputs(params: WanParams, batch: int, frames: int = 16, height: int = 720, width: int = 1280, device="cpu",
+                dtype=torch.bfloat16, seed: int = 0, clip_tokens: Optional[int] = None):
+    """``i2v_inputs`` plus ``clip_fea`` [B, Li, clip_dim]: CLIP vision features of the conditioning image (Li = 257), or of
+    the first and last frame for FLF2V (Li = 514 = ``clip_pos_tokens``)."""
+    out = i2v_inputs(params, batch, frames, height, width, device, dtype, seed)
+    li = clip_tokens or params.clip_pos_tokens or 257
+    g = torch.Generator(device="cpu").manual_seed(seed + 1)
+    out["clip_fea"] = torch.randn(batch, li, params.clip_dim, generator=g).to(device=device, dtype=dtype)
+    return out

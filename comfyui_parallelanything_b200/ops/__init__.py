@@ -50,6 +50,7 @@ def native_ok(device) -> bool:
 
 EPI = {
     "bias": 0, "gelu": 1, "silu": 2, "gate_res": 3, "qkv_rope": 4, "euler_unpatch": 5, "geglu": 6, "res": 7, "bias_bcast": 8, "swiglu": 9,
+    "gelu_erf": 10,     # exact erf GELU (nn.GELU()); "gelu" is the tanh approximation
 }
 
 
@@ -141,13 +142,18 @@ def timestep_embedding(t: torch.Tensor, dim: int = 256, time_factor: float = 100
 ATTENTION_VARIANT = int(os.environ.get("PA_ATTENTION", "2"))    # 1: one query tile per CTA, 2: ping-pong (two)
 
 
-def attention(q, k, v, out=None, scale: Optional[float] = None, variant: Optional[int] = None):
-    """q,k,v: [B,H,L,D] bf16 views (D = 64 / 128, innermost contiguous) -> out [B, Lq, H*D]."""
+def attention(q, k, v, out=None, scale: Optional[float] = None, variant: Optional[int] = None, kv2=None):
+    """q,k,v: [B,H,L,D] bf16 views (D = 64 / 128, innermost contiguous) -> out [B, Lq, H*D].
+
+    ``kv2 = (k2, v2)``: a second key/value source ([B, H, Lk2, 128] views, head dim 128 only); the result is then
+    ``softmax(q k^T) v + softmax(q k2^T) v2``, computed in one launch of the two-source ping-pong kernel whatever
+    ``variant`` / ``PA_ATTENTION`` select (WAN2.1 image-to-video: text plus CLIP image cross-attention)."""
     b, h, lq, d = q.shape
     if out is None:
         out = torch.empty(b, lq, h * d, dtype=torch.bfloat16, device=q.device)
+    k2, v2 = kv2 if kv2 is not None else (None, None)
     require().attention(q, k, v, out, float(scale if scale is not None else d ** -0.5),
-                        ATTENTION_VARIANT if variant is None else variant)
+                        ATTENTION_VARIANT if variant is None else variant, k2, v2)
     return out
 
 

@@ -409,21 +409,31 @@ class _SpmdTextDiTEngine(SpmdFluxEngine):
     kernel_pulled_inputs = ("x", "t")
 
     def _launch(self, loc: dict, fused: bool):
+        # WAN2.1 I2V / FLF2V: the CLIP image features follow the context
+        cond = (loc["ctx"], loc["clip"]) if "clip" in loc else (loc["ctx"],)
         if fused:
-            self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"],
+            self.ex.denoise_step(loc["x"], loc["t"], *cond, loc["sig"],
                                  out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
                                  x_src_ptr=self._src("x", self._row_bytes("x")), t_src_ptr=self._src("t", 2))
             return None
-        return self.ex.denoise_step(loc["x"], loc["t"], loc["ctx"], loc["sig"])
+        return self.ex.denoise_step(loc["x"], loc["t"], *cond, loc["sig"])
 
 
 class SpmdWanEngine(_SpmdTextDiTEngine):
     """WAN2.x video DiT replicas (``exec/wan_exec.py``).  ``height``/``width`` are pixel sizes, ``frames`` the
     number of LATENT frames; the video latent is staged as [B, in_dim, T, H/8, W/8] (16 channels for text-to-video, 36
-    for image-to-video) and the result as [B, out_dim = 16, T, H/8, W/8]."""
+    for image-to-video) and the result as [B, out_dim = 16, T, H/8, W/8].  Executors with CLIP image conditioning
+    (WAN2.1 I2V / FLF2V) add a ``"clip"`` input [B, clip_tokens, clip_dim] after ``"sig"`` (default 257 tokens, the
+    model's ``clip_pos_tokens`` for FLF2V), read through a peer TMA descriptor like ``"ctx"``."""
 
-    def __init__(self, executor, global_batch: int, frames: int, height: int, width: int, txt_len: int, **kw):
+    tma_peer_inputs = ("ctx", "clip")
+
+    def __init__(self, executor, global_batch: int, frames: int, height: int, width: int, txt_len: int,
+                 clip_tokens: int = 0, **kw):
         self.T = frames
+        self.Li = 0
+        if getattr(executor, "conditioning_kwargs", ()):
+            self.Li = clip_tokens or executor.clip_pos_tokens or 257
         super().__init__(executor, global_batch, height, width, txt_len, **kw)
 
     def _latent_channels(self) -> int:
@@ -431,8 +441,12 @@ class SpmdWanEngine(_SpmdTextDiTEngine):
 
     def _make_spec(self, B: int) -> dict:
         p, bf = self.ex.params, torch.bfloat16
-        return {"x": ((B, self.C, self.T, self.H, self.W), bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
-                "sig": ((B, 2), torch.float32), "out": ((B, p.out_dim, self.T, self.H, self.W), bf)}
+        spec = {"x": ((B, self.C, self.T, self.H, self.W), bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
+                "sig": ((B, 2), torch.float32)}
+        if self.Li:
+            spec["clip"] = ((B, self.Li, p.clip_dim), bf)
+        spec["out"] = ((B, p.out_dim, self.T, self.H, self.W), bf)
+        return spec
 
 
 class SpmdZImageEngine(_SpmdTextDiTEngine):

@@ -674,6 +674,131 @@ def wan_i2v_executor_tiny_fp8():
 
 
 @check
+def attention_two_kv():
+    """Two-source attention ``softmax(q K1^T) V1 + softmax(q K2^T) V2`` (WAN2.1 text + CLIP image cross-attention)
+    through the strided views the executor passes (q from a [B, L, H*128] buffer, K/V from [B, L, 2*H*128] buffers),
+    including 1- and 2-key tail tiles (257 / 514 image tokens) and a text length that is not a multiple of 128."""
+    res = {"name": "attention_two_kv", "ok": True}
+    for (B, H, Lq, L1, L2) in ((1, 2, 260, 512, 257), (2, 4, 1000, 512, 514), (1, 40, 3600, 512, 257),
+                               (2, 2, 300, 77, 257)):
+        dim = H * 128
+        qb = _rand(B, Lq, dim, seed=1)
+        kv1, kv2 = _rand(B, L1, 2 * dim, seed=2), _rand(B, L2, 2 * dim, seed=3)
+        heads = lambda t, w, n: t.view(B, t.shape[1], n, H, 128)[:, :, w].permute(0, 2, 1, 3)  # noqa: E731
+        q, k1, v1, k2, v2 = heads(qb, 0, 1), heads(kv1, 0, 2), heads(kv1, 1, 2), heads(kv2, 0, 2), heads(kv2, 1, 2)
+        want = (F.scaled_dot_product_attention(q.float(), k1.float(), v1.float())
+                + F.scaled_dot_product_attention(q.float(), k2.float(), v2.float()))
+        want = want.transpose(1, 2).reshape(B, Lq, dim)
+        out = torch.zeros(B, Lq, dim, dtype=torch.bfloat16, device=_dev())
+        ops.attention(q, k1, v1, out=out, kv2=(k2, v2))
+        r = _cmp("attention_two_kv", out, want, 0.02)
+        tag = f"{B}x{H}x{Lq}x{L1}x{L2}"
+        res[tag + "_mean_rel"] = r["mean_rel"]
+        res[tag + "_max_rel"] = r["max_rel"]
+        res["ok"] = res["ok"] and r["ok"]
+    # device time at the WAN2.1-I2V 720p shape: one two-source launch against two one-source launches (which would
+    # still need an add to combine their outputs)
+    B, H, Lq, L1, L2 = 1, 40, 14400, 512, 257
+    dim = H * 128
+    qb, kv1, kv2 = _rand(B, Lq, dim, seed=4), _rand(B, L1, 2 * dim, seed=5), _rand(B, L2, 2 * dim, seed=6)
+    heads = lambda t, w, n: t.view(B, t.shape[1], n, H, 128)[:, :, w].permute(0, 2, 1, 3)  # noqa: E731
+    q, k1, v1, k2, v2 = heads(qb, 0, 1), heads(kv1, 0, 2), heads(kv1, 1, 2), heads(kv2, 0, 2), heads(kv2, 1, 2)
+    out, o1, o2 = (torch.empty(B, Lq, dim, dtype=torch.bfloat16, device=_dev()) for _ in range(3))
+    runs = {"two_source_us": lambda: ops.attention(q, k1, v1, out=out, kv2=(k2, v2)),
+            "two_launches_us": lambda: (ops.attention(q, k1, v1, out=o1), ops.attention(q, k2, v2, out=o2))}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for name, fn in list(runs.items()) * 2:          # alternated, the second pass is reported
+        for _ in range(5):
+            fn()
+        e0.record()
+        for _ in range(50):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        res[name] = round(e0.elapsed_time(e1) / 50 * 1000, 1)
+    res["speed_shape"] = [B, H, Lq, L1, L2]
+    res["gpu"] = torch.cuda.get_device_name()
+    return res
+
+
+@check
+def gemm_gelu_erf():
+    """``gelu_erf`` epilogue: exact erf GELU (nn.GELU(), WAN's CLIP image projection), 1280-wide like that projection."""
+    a, w, b = _rand(2, 257, 1280), _rand(1280, 1280, scale=0.03), _rand(1280)
+    out = torch.zeros(2, 257, 1280, dtype=torch.bfloat16, device=_dev())
+    ops.gemm(a, w, "gelu_erf", out=out, bias=b)
+    return _cmp("gemm_gelu_erf", out, F.gelu(_gemm_ref(a, w, b)), 0.012)
+
+
+def _wan_clip_case(fp8: bool, flf2v: bool) -> dict:
+    """Tiny WAN2.1 I2V (or FLF2V: 514 CLIP tokens + ``emb_pos``) executor against the fp32 oracle: ``forward`` with and
+    without ``clip_fea``, then ``denoise_step`` eager, captured and replayed twice, and once more with ``clip_fea=None``."""
+    import dataclasses
+    from ..exec.wan_exec import WanClipExecutor
+    from ..models import wan
+    p = dataclasses.replace(wan.wan_tiny_params(), in_dim=36, clip_dim=128, clip_pos_tokens=514 if flf2v else 0)
+    torch.manual_seed(5)
+    m = wan.WanModel(p).to(device=_dev(), dtype=torch.bfloat16).eval()
+    with torch.no_grad():
+        for n_, p_ in m.named_parameters():
+            if "norm" in n_ and n_.endswith("weight"):
+                p_.add_(0.1 * torch.randn_like(p_))
+    ex = WanClipExecutor(m, _dev(), cuda_graphs=True, fp8=fp8)
+    oracle = wan.WanModel(p).to(device=_dev(), dtype=torch.float32).eval()
+    oracle.load_state_dict({k: v.float() for k, v in m.state_dict().items()})
+    inp = wan.clip_inputs(p, 2, frames=8, height=128, width=192, device=_dev(), dtype=torch.bfloat16, seed=6)
+    tol = 0.05 if fp8 else 0.03
+    name = ("wan_flf2v" if flf2v else "wan_clip") + "_executor_tiny" + ("_fp8" if fp8 else "")
+    f32 = lambda d: {k: (v.float() if v is not None else None) for k, v in d.items()}  # noqa: E731
+    with torch.no_grad():
+        got = ex(**inp)
+        want = oracle(**f32(inp))
+        got0 = ex(**dict(inp, clip_fea=None))
+        want0 = oracle(**f32(dict(inp, clip_fea=None)))
+    r = _cmp(name, got, want, tol)
+    r0 = _cmp(name + "_no_clip", got0, want0, tol)
+    r["no_clip_mean_rel"] = r0["mean_rel"]
+    r["ok"] = r["ok"] and r0["ok"] and tuple(got.shape) == (2, 16) + tuple(inp["x"].shape[2:])
+    sig = torch.tensor([[1.0, 0.8], [0.6, 0.5]], device=_dev())
+    x, t, c, cf = ex._prep(inp["x"], inp["timesteps"], inp["context"], inp["clip_fea"])
+    worst = 0.0
+    for it in range(5):                                 # eager, capture, replay, replay; then without clip_fea
+        x[:, :16].mul_(0.9)
+        clip = cf if it < 4 else None
+        nxt = ex.denoise_step(x, t, c, clip, sig).clone()
+        with torch.no_grad():
+            v = oracle(x.float(), t.float(), context=c.float(), clip_fea=clip.float() if clip is not None else None)
+        want2 = x[:, :16].float() + (sig[:, 1] - sig[:, 0])[:, None, None, None, None] * v
+        r2 = _cmp(name + "_euler", nxt, want2, tol)
+        worst = max(worst, r2["mean_rel"])
+        r["ok"] = r["ok"] and r2["ok"]
+    r["euler_worst_mean_rel"] = worst
+    r["graphs"] = sorted(ex._graphs.state(k) for k in list(ex._graphs._graphs))
+    r["ok"] = r["ok"] and "graph" in r["graphs"]
+    return r
+
+
+@check
+def wan_clip_executor_tiny():
+    return _wan_clip_case(False, False)
+
+
+@check
+def wan_clip_executor_tiny_fp8():
+    return _wan_clip_case(True, False)
+
+
+@check
+def wan_flf2v_executor_tiny():
+    return _wan_clip_case(False, True)
+
+
+@check
+def wan_flf2v_executor_tiny_fp8():
+    return _wan_clip_case(True, True)
+
+
+@check
 def gemm_2cta():
     """CTA-pair (cta_group::2) GEMM kernel, selected with force_bn=512: numerics on even / ragged shapes and a
     device-timed comparison with the one-CTA 128x256 kernel at a FLUX-like shape."""

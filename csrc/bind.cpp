@@ -434,7 +434,8 @@ static void add_(Tensor a, Tensor b, Tensor out) {
   check(pa::add_bf16(a.data_ptr(), b.data_ptr(), out.data_ptr(), a.numel(), cur_stream()), "add");
 }
 
-static void attention(Tensor q, Tensor k, Tensor v, Tensor out, double scale, int variant) {
+static void attention(Tensor q, Tensor k, Tensor v, Tensor out, double scale, int variant, c10::optional<Tensor> k2,
+                      c10::optional<Tensor> v2) {
   c10::cuda::CUDAGuard guard(q.device());
   TORCH_CHECK(q.dim() == 4 && k.dim() == 4 && v.dim() == 4, "q/k/v must be [B, H, L, D] views");
   const int D = (int)q.size(3);
@@ -445,6 +446,26 @@ static void attention(Tensor q, Tensor k, Tensor v, Tensor out, double scale, in
   long long qs[3] = {q.stride(0), q.stride(1), q.stride(2)};
   long long ks[3] = {k.stride(0), k.stride(1), k.stride(2)};
   long long vs[3] = {v.stride(0), v.stride(1), v.stride(2)};
+  if (k2.has_value() || v2.has_value()) {
+    // two key/value sources: always the two-source ping-pong kernel, whatever `variant` says
+    TORCH_CHECK(k2.has_value() && v2.has_value(), "attention: k2 and v2 go together");
+    const Tensor& K2 = *k2;
+    const Tensor& V2 = *v2;
+    TORCH_CHECK(D == 128, "attention: a second K/V source needs head_dim 128");
+    TORCH_CHECK(K2.dim() == 4 && V2.dim() == 4 && K2.size(3) == D && V2.size(3) == D && K2.stride(3) == 1 &&
+                    V2.stride(3) == 1 && K2.scalar_type() == at::kBFloat16 && V2.scalar_type() == at::kBFloat16,
+                "attention: k2/v2 must be bf16 [B, H, L2, 128] views with a contiguous innermost dim");
+    TORCH_CHECK(K2.size(0) == q.size(0) && K2.size(1) == q.size(1) && V2.sizes() == K2.sizes() &&
+                    k.size(0) == q.size(0) && k.size(1) == q.size(1) && v.sizes() == k.sizes(),
+                "attention: batch / heads / lengths of the key and value sources do not match");
+    long long ks2[3] = {K2.stride(0), K2.stride(1), K2.stride(2)};
+    long long vs2[3] = {V2.stride(0), V2.stride(1), V2.stride(2)};
+    check(pa::attention2_kv2_bf16(q.data_ptr(), k.data_ptr(), v.data_ptr(), K2.data_ptr(), V2.data_ptr(), out.data_ptr(),
+                                  out.stride(1), out.stride(0), (int)q.size(0), (int)q.size(1), (int)q.size(2),
+                                  (int)k.size(2), (int)K2.size(2), qs, ks, vs, ks2, vs2, (float)scale, cur_stream()),
+          "attention2_kv2");
+    return;
+  }
   if (variant >= 20 && variant <= 250) {      // timing experiments of the ping-pong kernel (garbage results)
     check(pa::attention2_debug(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), out.stride(1), out.stride(0),
                                (int)q.size(0), (int)q.size(1), (int)q.size(2), (int)k.size(2), variant - 20, qs, ks, vs,
@@ -593,7 +614,7 @@ PYBIND11_MODULE(_C, m) {
   m.def("silu", &silu_);
   m.def("add", &add_);
   m.def("attention", &attention, py::arg("q"), py::arg("k"), py::arg("v"), py::arg("out"), py::arg("scale"),
-        py::arg("variant") = 1);
+        py::arg("variant") = 1, py::arg("k2") = py::none(), py::arg("v2") = py::none());
   m.def("attention2_trace", &attention2_trace);
   m.def("attention_fp8out", &attention_fp8out);
   m.def("attention3_trace", &attention3_trace);

@@ -85,6 +85,11 @@ int attention3_bf16(const void* q, const void* k, const void* v, void* out, long
 int attention2_bf16(const void* q, const void* k, const void* v, void* out, long long ldo, long long o_bstride, int B,
                     int H, int Lq, int Lk, int D, const long long* q_strides, const long long* k_strides,
                     const long long* v_strides, float scale, cudaStream_t st);
+// two key/value sources (head dim 128): out = softmax(q k^T) v + softmax(q k2^T) v2, one launch
+int attention2_kv2_bf16(const void* q, const void* k, const void* v, const void* k2, const void* v2, void* out,
+                        long long ldo, long long o_bstride, int B, int H, int Lq, int Lk, int Lk2,
+                        const long long* q_strides, const long long* k_strides, const long long* v_strides,
+                        const long long* k2_strides, const long long* v2_strides, float scale, cudaStream_t st);
 
 // small-KV cross-attention (Lk <= 128, head_dim 64): a CTA pair shares one multicast K/V tile (csrc/kernels/xattn_cluster.cu)
 int xattn_cluster_bf16(const void* q, const void* k, const void* v, void* out, long long ldo, long long o_bstride, int B,

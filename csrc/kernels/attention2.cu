@@ -9,6 +9,12 @@
 //   TMEM        S_A @0, S_B @128 (fp32, 128 cols), O_A @256, O_B @384; P_X (bf16) overwrites the first 64
 //               columns of S_X once S_X sits in registers and feeds the P.V MMA as a TMEM A operand.
 //   registers   setmaxnreg: 56 for the producer/MMA warpgroup, 208 for the softmax warpgroups.
+//
+// KV2 (D = 128, NS = 1): two key/value sources, out = softmax(q K1^T) V1 + softmax(q K2^T) V2 in one launch (WAN2.1
+// I2V / FLF2V cross-attention: text tokens and CLIP image tokens).  The producer streams the n1 tiles of source 1 and
+// then the n2 tiles of source 2 through the same rings (only the tensor map and the key row change); at tile n1 the
+// softmax warpgroups store the normalised segment-1 rows as bf16, restart the running max / sum and release the first
+// segment-2 P.V (accumulate = 0) through `o_drain`; the final store adds the segment-1 row back in fp32 and rounds once.
 #include <cuda_bf16.h>
 #include <cuda_fp8.h>
 #include <cuda_runtime.h>
@@ -63,11 +69,48 @@ struct Cfg {
 // row maxima exchanged through shared memory): two warps per scheduler work on the same tile, so one warp's MUFU.EX2
 // stalls are filled with the other's FMA-pipe work and the  S -> P  latency (the period-setting chain once the MMAs
 // issue back to back) roughly halves.  640 threads, setmaxnreg 56 / 104 (640 x 96 registers at launch).
-template <int D, int DBG, int NS>
+// KV2: this thread's normalised 128-column O row (tensor memory) -> bf16 at `dst`; `add`: sum with the bf16 row that is
+// already there (segment 1) in fp32 and round once
+__device__ __forceinline__ void store_o_row(uint32_t o_addr, __nv_bfloat16* dst, float inv, bool add, bool row_ok) {
+#pragma unroll 1
+  for (int c = 0; c < 4; ++c) {
+    uint32_t t[32];
+    ptx::tmem_ld_32x32b_x32(o_addr + c * 32, t);
+    ptx::tmem_ld_wait();
+    if (row_ok) {
+#pragma unroll
+      for (int i = 0; i < 32; i += 8) {
+        float f[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) f[e] = __uint_as_float(t[i + e]) * inv;
+        uint4* d = reinterpret_cast<uint4*>(dst + c * 32 + i);
+        if (add) {
+          const uint4 prev = *d;
+          const __nv_bfloat162* pv = reinterpret_cast<const __nv_bfloat162*>(&prev);
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float2 pf = __bfloat1622float2(pv[e]);
+            f[2 * e] += pf.x;
+            f[2 * e + 1] += pf.y;
+          }
+        }
+        uint4 u;
+        __nv_bfloat162* hv = reinterpret_cast<__nv_bfloat162*>(&u);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) hv[e] = __floats2bfloat162_rn(f[2 * e], f[2 * e + 1]);
+        *d = u;
+      }
+    }
+  }
+}
+
+template <int D, int DBG, int NS, bool KV2 = false>
 __global__ void __launch_bounds__(128 + 256 * NS, 1)
 attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                   const __grid_constant__ CUtensorMap tmV, __nv_bfloat16* __restrict__ out, long long ldo,
-                  long long o_bstride, int H, int Lq, int Lk, float scale_log2, const Fp8Out f8) {
+                  long long o_bstride, int H, int Lq, int Lk, float scale_log2, const Fp8Out f8,
+                  const __grid_constant__ CUtensorMap tmK2, const __grid_constant__ CUtensorMap tmV2, int Lk2) {
+  static_assert(!KV2 || (D == 128 && NS == 1 && DBG == 0), "two K/V sources: D = 128, NS = 1 only");
   using C = Cfg<D>;
   constexpr int BN = C::BN;
   constexpr uint32_t SLICE = C::SLICE, TILE = C::TILE;
@@ -84,17 +127,23 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
   uint64_t* o_full = bars + 13;     // 2
   uint64_t* p_hi = bars + 15;       // 2: P_X keys 64..127 stored
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 17);
+  uint64_t* o_drain = bars + 18;    // 2 (KV2): segment-1 O of tile X stored, its TMEM columns may be overwritten
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int warp_u = __shfl_sync(0xffffffffu, warp, 0);      // provably warp-uniform role index
   const int q0 = blockIdx.x * 256;
   const int bh = blockIdx.y;
-  const int n_kv = (Lk + BN - 1) / BN;
+  const int n1 = (Lk + BN - 1) / BN;                  // key tiles of source 1
+  const int n_kv = KV2 ? n1 + (Lk2 + BN - 1) / BN : n1;
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmQ);
     ptx::prefetch_tmap(&tmK);
     ptx::prefetch_tmap(&tmV);
+    if constexpr (KV2) {
+      ptx::prefetch_tmap(&tmK2);
+      ptx::prefetch_tmap(&tmV2);
+    }
   }
   if (warp == 1 && lane == 0) {
     ptx::mbar_init(q_full, 1);
@@ -107,6 +156,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       ptx::mbar_init(&p_full[i], 4);
       ptx::mbar_init(&p_hi[i], 4);
       ptx::mbar_init(&o_full[i], 1);
+      if constexpr (KV2) ptx::mbar_init(&o_drain[i], 4);
     }
     ptx::fence_barrier_init();
     ptx::fence_proxy_async_smem();
@@ -139,17 +189,31 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         if (leader) {
           PA_TR(4, j, 0);
           ptx::mbar_arrive_expect_tx(&k_full[s], TILE);
+          if (KV2 && j >= n1) {                            // ring and phase run over both sources; map and row switch
 #pragma unroll
-          for (int sl = 0; sl < D / 64; ++sl)
-            ptx::tma_load_4d_s(smem_base + C::OFF_K + s * TILE + sl * SLICE, &tmK, &k_full[s], sl * 64, j * BN, hh, hb);
+            for (int sl = 0; sl < D / 64; ++sl)
+              ptx::tma_load_4d_s(smem_base + C::OFF_K + s * TILE + sl * SLICE, &tmK2, &k_full[s], sl * 64, (j - n1) * BN,
+                                 hh, hb);
+          } else {
+#pragma unroll
+            for (int sl = 0; sl < D / 64; ++sl)
+              ptx::tma_load_4d_s(smem_base + C::OFF_K + s * TILE + sl * SLICE, &tmK, &k_full[s], sl * 64, j * BN, hh, hb);
+          }
         }
         ptx::mbar_wait(&v_empty[s], ph ^ 1);
         if (leader) {
           PA_TR(4, j, 1);
           ptx::mbar_arrive_expect_tx(&v_full[s], TILE);
+          if (KV2 && j >= n1) {
 #pragma unroll
-          for (int sl = 0; sl < D / 64; ++sl)
-            ptx::tma_load_4d_s(smem_base + C::OFF_V + s * TILE + sl * SLICE, &tmV, &v_full[s], sl * 64, j * BN, hh, hb);
+            for (int sl = 0; sl < D / 64; ++sl)
+              ptx::tma_load_4d_s(smem_base + C::OFF_V + s * TILE + sl * SLICE, &tmV2, &v_full[s], sl * 64, (j - n1) * BN,
+                                 hh, hb);
+          } else {
+#pragma unroll
+            for (int sl = 0; sl < D / 64; ++sl)
+              ptx::tma_load_4d_s(smem_base + C::OFF_V + s * TILE + sl * SLICE, &tmV, &v_full[s], sl * 64, j * BN, hh, hb);
+          }
         }
       }
       __syncwarp();
@@ -190,6 +254,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
 #pragma unroll 1
         for (int x = 0; x < 2; ++x) {
           ptx::mbar_wait(&p_full[x], j & 1);
+          if (KV2 && j == n1) ptx::mbar_wait(&o_drain[x], 0);   // segment-1 O of tile x has left tensor memory
           ptx::tc_fence_after();
           if (leader) {
             PA_TR(x, j, 0);
@@ -202,7 +267,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
                                 (j | kk) != 0);
               } else {
                 ptx::mma_f16_ts(tmem_u + 256 + x * 128, tmem_u + x * 128 + kk * 8, vd + kk * 128, IDESC_PV,
-                                (j | kk) != 0);
+                                ((KV2 && j >= n1 ? j - n1 : j) | kk) != 0);
               }
             }
           }
@@ -255,6 +320,22 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     const unsigned long long sl2 = pack2(scale_log2, scale_log2);
 
     for (int j = 0; j < n_kv; ++j) {
+      if (KV2 && j == n1) {
+        // segment 1 done: store it normalised, restart the running max / sum, hand O's columns back to the MMA warp
+        ptx::mbar_wait(&o_full[x], (n1 - 1) & 1);
+        ptx::tc_fence_after();
+        const int q_row = q0 + x * 128 + r;
+        const int b = bh / H, h = bh - b * H;
+        store_o_row(o_addr, out + b * o_bstride + static_cast<long long>(q_row) * ldo + h * D, 1.0f / l, false,
+                    q_row < Lq);
+        m_used = -INFINITY;
+        l = 0.f;
+        ptx::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) ptx::mbar_arrive(&o_drain[x]);
+      }
+      const bool seg2 = KV2 && j >= n1;
+      const int jj = seg2 ? j - n1 : j;                  // tile index inside its own source
       ptx::mbar_wait(&s_full[x], j & 1);
       if (tracer) PA_TR(2 + x, j, 0);
       ptx::tc_fence_after();
@@ -289,7 +370,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         if (tracer) PA_TR(2 + x, j, 4);
         continue;
       }
-      const int kv_left = Lk - j * BN - half * CW;
+      const int kv_left = (seg2 ? Lk2 : Lk) - jj * BN - half * CW;
       if (kv_left < CW) {
 #pragma unroll
         for (int i = 0; i < CW; ++i)
@@ -318,7 +399,7 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         const float alpha = need ? ex2f((m_used - m_new) * scale_log2) : 1.0f;
         if (need) m_used = m_new;
         l *= alpha;
-        if (j > 0) {
+        if (jj > 0) {
           ptx::mbar_wait(&o_full[x], (j - 1) & 1);
           ptx::tc_fence_after();
 #pragma unroll 1
@@ -389,7 +470,9 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     const float inv = 1.0f / l;
     const int b = bh / H, h = bh - b * H;
     __nv_bfloat16* dst = out + b * o_bstride + static_cast<long long>(q_row) * ldo + h * D + half * OW;
-    if (f8.q != nullptr && NS == 1 && D == 128) {
+    if (KV2) {
+      store_o_row(o_addr, dst, inv, true, q_row < Lq);
+    } else if (f8.q != nullptr && NS == 1 && D == 128) {
       // MX-quantised output: each 32-column TMEM chunk of this thread's row is one MX block (amax -> UE8M0 scale ->
       // e4m3); half the bytes of the bf16 store and no separate quantise kernel before the projection GEMM
       uint8_t* qrow = f8.q + b * f8.bstride + static_cast<long long>(q_row) * f8.ld8 + h * D;
@@ -463,12 +546,20 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
   }
 }
 
-template <int D, int DBG, int NS = 1>
+// second K/V source of a KV2 launch
+struct Kv2 {
+  const void *k, *v;
+  int Lk;
+  const long long *ks, *vs;
+};
+
+template <int D, int DBG, int NS = 1, bool KV2 = false>
 static int launch(const void* q, const void* k, const void* v, void* out, long long ldo, long long o_bstride, int B,
                   int H, int Lq, int Lk, const long long* qs, const long long* ks, const long long* vs, float scale,
-                  cudaStream_t st, Fp8Out f8 = Fp8Out{nullptr, nullptr, 0, 0, 0, 0}) {
+                  cudaStream_t st, Fp8Out f8 = Fp8Out{nullptr, nullptr, 0, 0, 0, 0},
+                  Kv2 kv2 = Kv2{nullptr, nullptr, 0, nullptr, nullptr}) {
   using C = Cfg<D>;
-  CUtensorMap tq, tk, tv;
+  CUtensorMap tq, tk, tv, tk2, tv2;
   const uint32_t box[4] = {64, 128, 1, 1};
   auto mk = [&](CUtensorMap* m, const void* p, int L, const long long* s3) {
     uint64_t dims[4] = {(uint64_t)D, (uint64_t)L, (uint64_t)H, (uint64_t)B};
@@ -478,18 +569,26 @@ static int launch(const void* q, const void* k, const void* v, void* out, long l
   if (mk(&tq, q, Lq, qs)) return -20;
   if (mk(&tk, k, Lk, ks)) return -21;
   if (mk(&tv, v, Lk, vs)) return -22;
+  if (KV2) {
+    if (mk(&tk2, kv2.k, kv2.Lk, kv2.ks)) return -23;
+    if (mk(&tv2, kv2.v, kv2.Lk, kv2.vs)) return -24;
+  } else {
+    tk2 = tk;                                            // unused by the one-source kernel
+    tv2 = tv;
+  }
   static bool attr_set[64] = {false};
   int dev = 0;
   cudaGetDevice(&dev);
   if (!attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(attention2_kernel<D, DBG, NS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(attention2_kernel<D, DBG, NS, KV2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)C::SMEM);
     if (e != cudaSuccess) return (int)e;
     attr_set[dev] = true;
   }
   dim3 grid((Lq + 255) / 256, B * H);
-  attention2_kernel<D, DBG, NS><<<grid, 128 + 256 * NS, C::SMEM, st>>>(tq, tk, tv, static_cast<__nv_bfloat16*>(out), ldo, o_bstride, H, Lq,
-                                                   Lk, scale * 1.4426950408889634f, f8);
+  attention2_kernel<D, DBG, NS, KV2><<<grid, 128 + 256 * NS, C::SMEM, st>>>(
+      tq, tk, tv, static_cast<__nv_bfloat16*>(out), ldo, o_bstride, H, Lq, Lk, scale * 1.4426950408889634f, f8, tk2, tv2,
+      kv2.Lk);
   return (int)cudaGetLastError();
 }
 }  // namespace a2
@@ -502,6 +601,18 @@ int attention2_bf16(const void* q, const void* k, const void* v, void* out, long
   if (D == 128) return a2::launch<128, 0>(q, k, v, out, ldo, o_bstride, B, H, Lq, Lk, qs, ks, vs, scale, st);
   if (D == 64) return a2::launch<64, 0>(q, k, v, out, ldo, o_bstride, B, H, Lq, Lk, qs, ks, vs, scale, st);
   return -11;
+}
+
+// head_dim 128 only: out = softmax(q k^T) v + softmax(q k2^T) v2 in one launch (the query tiles are loaded once)
+int attention2_kv2_bf16(const void* q, const void* k, const void* v, const void* k2, const void* v2, void* out,
+                        long long ldo, long long o_bstride, int B, int H, int Lq, int Lk, int Lk2, const long long* qs,
+                        const long long* ks, const long long* vs, const long long* ks2, const long long* vs2, float scale,
+                        cudaStream_t st) {
+  for (int i = 0; i < 3; ++i)
+    if (qs[i] % 8 || ks[i] % 8 || vs[i] % 8 || ks2[i] % 8 || vs2[i] % 8) return -10;
+  if (Lk < 1 || Lk2 < 1) return -13;
+  return a2::launch<128, 0, 1, true>(q, k, v, out, ldo, o_bstride, B, H, Lq, Lk, qs, ks, vs, scale, st,
+                                     a2::Fp8Out{nullptr, nullptr, 0, 0, 0, 0}, a2::Kv2{k2, v2, Lk2, ks2, vs2});
 }
 
 // head_dim 128 only: the output goes out MX-quantised (e4m3 [B, rows8, ld8] + scale chunks) for a following fp8 GEMM

@@ -16,6 +16,7 @@ enum EpiMode : int {
   EPI_RES = 7,          // out = residual + acc + bias
   EPI_BIAS_BCAST = 8,   // out = acc + bias + gate[b, n]   (per-sample channel bias, e.g. time embedding)
   EPI_SWIGLU = 9,       // same interleaving as EPI_GEGLU: out[:, n/2] = a * silu(g)
+  EPI_BIAS_GELU_ERF = 10,  // out = gelu(acc + bias), exact erf form (nn.GELU()); EPI_BIAS_GELU is the tanh form
 };
 
 struct GemmParams {

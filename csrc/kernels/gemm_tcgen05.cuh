@@ -532,6 +532,9 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tadd
         if (p.mode == EPI_BIAS_GELU) {
 #pragma unroll
           for (int e = 0; e < 8; ++e) x[e] = gelu_tanh(x[e]);
+        } else if (p.mode == EPI_BIAS_GELU_ERF) {
+#pragma unroll
+          for (int e = 0; e < 8; ++e) x[e] = gelu_erf(x[e]);
         } else if (p.mode == EPI_BIAS_SILU) {
 #pragma unroll
           for (int e = 0; e < 8; ++e) x[e] = silu(x[e]);

@@ -8,7 +8,8 @@ import time
 
 
 def run(a, hb, model_name: str, build_model, host: dict, config: dict) -> int:
-    """``build_model(lead_device) -> nn.Module``; ``host``: pinned inputs x / timesteps / context / sig."""
+    """``build_model(lead_device) -> nn.Module``; ``host``: pinned inputs x / timesteps / context / sig (+ clip_fea for
+    WAN2.1 I2V / FLF2V, passed on every call like the sampler's conditioning)."""
     hb.quiet_stdout()
     rank, world, _local = hb.dist_env()
     if hb.host_only_group(rank, world):
@@ -41,12 +42,14 @@ def run(a, hb, model_name: str, build_model, host: dict, config: dict) -> int:
         nxt = x[:, :e.shape[1]] + (sig[:, 1] - sig[:, 0]).view(-1, *ones).to(x.dtype) * e
         return nxt if nxt.shape[1] == x.shape[1] else torch.cat([nxt, x[:, e.shape[1]:]], 1)
 
+    cond = {k: d[k] for k in ("clip_fea",) if k in d}                  # step-invariant extra conditioning
+    cond_e2e = {k: stage[k] for k in cond}
     state = {"x": d["x"]}
 
     def step_device():
         with torch.no_grad():
             x = state["x"]
-            e = model(x, d["timesteps"], context=d["context"])
+            e = model(x, d["timesteps"], context=d["context"], **cond)
             state["x"] = euler(x, e, d["sig"])
 
     def step_e2e():
@@ -54,7 +57,7 @@ def run(a, hb, model_name: str, build_model, host: dict, config: dict) -> int:
             fresh = {k: torch.empty_like(v) for k, v in stage.items() if k in ("x", "timesteps")}
             for k in stage:
                 (fresh.get(k, stage[k])).copy_(host[k], non_blocking=True)
-            e = model(fresh["x"], fresh["timesteps"], context=stage["context"])
+            e = model(fresh["x"], fresh["timesteps"], context=stage["context"], **cond_e2e)
             result_host.copy_(euler(fresh["x"], e, stage["sig"]), non_blocking=True)
 
     def sync_all():
@@ -81,8 +84,8 @@ def run(a, hb, model_name: str, build_model, host: dict, config: dict) -> int:
     extra = {}
     if a.gpus > 1:
         with torch.no_grad():
-            got = model(d["x"], d["timesteps"], context=d["context"]).clone()
-            want = eng.slots[0].replica(d["x"], d["timesteps"], context=d["context"]).clone()
+            got = model(d["x"], d["timesteps"], context=d["context"], **cond).clone()
+            want = eng.slots[0].replica(d["x"], d["timesteps"], context=d["context"], **cond).clone()
         sync_all()
         extra["output_matches_n1"] = hb.rel_err(got, want)
     if getattr(eng, "_ulysses", None) is not None:

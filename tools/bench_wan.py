@@ -2,9 +2,11 @@
 """Secondary benchmark: WAN2.2-A14B-sized video DiT (14.3 B params, random init), 720p x 16 frames (latent
 [16, 4, 90, 160] -> 14 400 tokens per sample), batch 8, bf16 - BASELINE.json config 4.  Same protocol and JSON line as
 bench.py (one step = forward + Euler update; device-timed, max over ranks; e2e with per-step H2D/D2H).  ``--i2v`` runs
-WAN2.2-I2V-A14B instead: the same layer stack on a 36-channel input ([noise 16 | mask 4 | image latent 16]).
+WAN2.2-I2V-A14B instead: the same layer stack on a 36-channel input ([noise 16 | mask 4 | image latent 16]).  ``--clip``
+runs WAN2.1-I2V-14B (that input plus 257 CLIP image tokens and an image cross-attention in every block), ``--flf2v``
+WAN2.1-FLF2V-14B (514 CLIP tokens of the first and last frame).
 
-    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8] [--i2v]
+    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8] [--i2v | --clip | --flf2v]
     python -m torch.distributed.run --nproc-per-node 8 ... tools/bench_wan.py --gpus 8
 """
 from __future__ import annotations
@@ -19,13 +21,23 @@ import bench as hb  # noqa: E402  (helpers: ClockSampler, timed, emit, dist_env,
 
 MODEL_NAME = "WAN2.2-A14B video DiT 720p x 16 frames"
 I2V_MODEL_NAME = "WAN2.2-I2V-A14B video DiT 720p x 16 frames"
+CLIP_MODEL_NAME = "WAN2.1-I2V-14B video DiT 720p x 16 frames (257 CLIP tokens)"
+FLF2V_MODEL_NAME = "WAN2.1-FLF2V-14B video DiT 720p x 16 frames (514 CLIP tokens)"
 
 
-def host_inputs(B, cap_len, i2v=False):
+def model_name(a) -> str:
+    return FLF2V_MODEL_NAME if a.flf2v else CLIP_MODEL_NAME if a.clip else I2V_MODEL_NAME if a.i2v else MODEL_NAME
+
+
+def host_inputs(B, cap_len, a):
     import torch
     from comfyui_parallelanything_b200.models import wan
-    cfg = wan.wan22_i2v_a14b_params() if i2v else wan.wan22_a14b_params()
-    make = wan.i2v_inputs if i2v else wan.example_inputs
+    if a.flf2v or a.clip:
+        cfg, make = (wan.wan21_flf2v_14b_params() if a.flf2v else wan.wan21_i2v_14b_params()), wan.clip_inputs
+    elif a.i2v:
+        cfg, make = wan.wan22_i2v_a14b_params(), wan.i2v_inputs
+    else:
+        cfg, make = wan.wan22_a14b_params(), wan.example_inputs
     inp = make(cfg, B, frames=16, height=720, width=1280, device="cpu", dtype=torch.bfloat16)
     inp["sig"] = torch.tensor([[1.0, 0.875]] * B, dtype=torch.float32)
     return cfg, {k: v.pin_memory() for k, v in inp.items()}
@@ -36,8 +48,8 @@ def run_nodes(a) -> int:
     import torch
     import _nodes_bench
     from comfyui_parallelanything_b200.models import wan
-    cfg, host = host_inputs(a.batch, a.cap_len, a.i2v)
-    name = I2V_MODEL_NAME if a.i2v else MODEL_NAME
+    cfg, host = host_inputs(a.batch, a.cap_len, a)
+    name = model_name(a)
 
     def build(lead):
         with torch.device(lead):
@@ -60,6 +72,8 @@ def main() -> int:
                     help="nodes = ONE process through the ComfyUI node API, new latent tensor every step (batch 1 -> "
                          "sequence-parallel over all GPUs)")
     ap.add_argument("--i2v", action="store_true", help="WAN2.2-I2V-A14B (36-channel input) instead of T2V")
+    ap.add_argument("--clip", action="store_true", help="WAN2.1-I2V-14B (36-channel input + CLIP image cross-attention)")
+    ap.add_argument("--flf2v", action="store_true", help="WAN2.1-FLF2V-14B (as --clip, 514 CLIP tokens)")
     a = ap.parse_args()
     if a.api == "nodes":
         return run_nodes(a)
@@ -81,18 +95,19 @@ def main() -> int:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
     from comfyui_parallelanything_b200.models import wan
-    cfg, host = host_inputs(B, a.cap_len, a.i2v)
+    cfg, host = host_inputs(B, a.cap_len, a)
+    clip = "clip_fea" in host
     result_host = torch.empty(B, 16, 4, 90, 160, dtype=torch.bfloat16).pin_memory()
     h2d = sum(v.numel() * v.element_size() for v in host.values())
     d2h = result_host.numel() * result_host.element_size()
     launches = 0
     eng = None
     if a.impl == "ours":
-        from comfyui_parallelanything_b200.exec.wan_exec import WanExecutor
+        from comfyui_parallelanything_b200.exec.wan_exec import WanClipExecutor, WanExecutor
         torch.manual_seed(1234)
         with torch.device(dev):
             model = wan.WanModel(cfg, dtype=torch.bfloat16).eval()
-        ex = WanExecutor(model, dev, cuda_graphs=True, fp8=(a.dtype == "fp8"))
+        ex = (WanClipExecutor if clip else WanExecutor)(model, dev, cuda_graphs=True, fp8=(a.dtype == "fp8"))
         del model
         torch.cuda.empty_cache()
         if world == 1:
@@ -100,19 +115,22 @@ def main() -> int:
             stage = {k: torch.empty_like(v, device=dev) for k, v in host.items()}
             out_buf = torch.empty(B, 16, 4, 90, 160, dtype=torch.bfloat16, device=dev)
 
+            cond = ("context", "clip_fea") if clip else ("context",)
+
             def step_device():
-                ex.denoise_step(d["x"], d["timesteps"], d["context"], d["sig"], out=out_buf)
+                ex.denoise_step(d["x"], d["timesteps"], *(d[k] for k in cond), d["sig"], out=out_buf)
 
             def step_e2e():
                 for k in stage:
                     stage[k].copy_(host[k], non_blocking=True)
                 ex.invalidate_conditioning()        # the staged conditioning is re-sent every step: recompute it
-                ex.denoise_step(stage["x"], stage["timesteps"], stage["context"], stage["sig"], out=out_buf)
+                ex.denoise_step(stage["x"], stage["timesteps"], *(stage[k] for k in cond), stage["sig"], out=out_buf)
                 result_host.copy_(out_buf, non_blocking=True)
         else:
             from comfyui_parallelanything_b200.parallel.spmd import SpmdWanEngine
-            eng = SpmdWanEngine(ex, B, 4, 720, 1280, a.cap_len, weights=pcts)
-            order = [host[k] for k in ("x", "timesteps", "context", "sig")]
+            eng = SpmdWanEngine(ex, B, 4, 720, 1280, a.cap_len, weights=pcts,
+                                clip_tokens=host["clip_fea"].shape[1] if clip else 0)
+            order = [host[k] for k in ("x", "timesteps", "context", "sig") + (("clip_fea",) if clip else ())]
             if rank == 0:
                 eng.stage_inputs(*order)
             torch.cuda.synchronize()
@@ -157,16 +175,19 @@ def main() -> int:
             def euler(x, e, sig):       # I2V: the update covers the predicted noise channels of x
                 return x[:, :e.shape[1]] + (sig[:, 1] - sig[:, 0]).view(-1, 1, 1, 1, 1).to(x.dtype) * e
 
+            kw = {"clip_fea": d["clip_fea"]} if clip else {}
+            kw_e2e = {"clip_fea": stage["clip_fea"]} if clip else {}
+
             def step_device():
                 with torch.no_grad():
-                    e = model(d["x"], d["timesteps"], context=d["context"])
+                    e = model(d["x"], d["timesteps"], context=d["context"], **kw)
                     return euler(d["x"], e, d["sig"])
 
             def step_e2e():
                 for k in stage:
                     stage[k].copy_(host[k], non_blocking=True)
                 with torch.no_grad():
-                    e = model(stage["x"], stage["timesteps"], context=stage["context"])
+                    e = model(stage["x"], stage["timesteps"], context=stage["context"], **kw_e2e)
                     result_host.copy_(euler(stage["x"], e, stage["sig"]), non_blocking=True)
         else:
             def step_device():
@@ -195,7 +216,7 @@ def main() -> int:
                  "e2e": {"value": round(1000.0 / ms_e2e, 4), "unit": "steps/s", "ms_per_step": round(ms_e2e, 3),
                          "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
                  "output_finite": bool(torch.isfinite(result_host.float()).all().item()),
-                 "config": {"model": I2V_MODEL_NAME if a.i2v else MODEL_NAME, "global_batch": B, "text_len": a.cap_len, "baseline_config": 4, "parallelism": par}})
+                 "config": {"model": model_name(a), "global_batch": B, "text_len": a.cap_len, "baseline_config": 4, "parallelism": par}})
     return 0
 
 

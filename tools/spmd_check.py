@@ -97,7 +97,8 @@ def bcast_check(rank, world, dev) -> int:
 
 def other_family(family, rank, world, dev) -> int:
     """Same comparison for the SDXL-class UNet (``unet``), Z-Image (``zimage``) and the WAN video DiT engines: ``wan``
-    (text-to-video, 16 latent channels) and ``wan_i2v`` (image-to-video: 36 input channels, 16 output channels)."""
+    (text-to-video, 16 latent channels), ``wan_i2v`` (image-to-video: 36 input channels, 16 output channels) and
+    ``wan_clip`` (WAN2.1 image-to-video: ``wan_i2v`` plus CLIP image features staged as the ``"clip"`` input)."""
     import torch
     import torch.distributed as dist
     from comfyui_parallelanything_b200.parallel import spmd
@@ -125,21 +126,30 @@ def other_family(family, rank, world, dev) -> int:
         want = ex.denoise_step(*order).clone()
         make = lambda backend, w: spmd.SpmdZImageEngine(ex, B, 256, 384, 40, weights=w, backend=backend)  # noqa: E731
     else:
-        from comfyui_parallelanything_b200.exec.wan_exec import WanExecutor
+        import dataclasses
+        from comfyui_parallelanything_b200.exec.wan_exec import WanClipExecutor, WanExecutor
         from comfyui_parallelanything_b200.models import wan
         p = wan.wan_tiny_params()
         make_inputs = wan.example_inputs
         if family == "wan_i2v":
-            import dataclasses
             p, make_inputs = dataclasses.replace(p, in_dim=36), wan.i2v_inputs
+        elif family == "wan_clip":
+            p, make_inputs = dataclasses.replace(p, in_dim=36, clip_dim=128), wan.clip_inputs
         torch.manual_seed(2)
-        ex = WanExecutor(wan.WanModel(p).to(device=dev, dtype=torch.bfloat16).eval(), dev, cuda_graphs=True)
+        cls = WanClipExecutor if family == "wan_clip" else WanExecutor
+        ex = cls(wan.WanModel(p).to(device=dev, dtype=torch.bfloat16).eval(), dev, cuda_graphs=True)
         inp = make_inputs(p, B, frames=8, height=128, width=192, device=dev, dtype=torch.bfloat16)
-        x, t, c = ex._prep(inp["x"], inp["timesteps"], inp["context"])
-        order = [x, t, c, sig]
-        want = ex.denoise_step(*order).clone()
+        if family == "wan_clip":
+            x, t, c, cf = ex._prep(inp["x"], inp["timesteps"], inp["context"], inp["clip_fea"])
+            want = ex.denoise_step(x, t, c, cf, sig).clone()
+            order = [x, t, c, sig, cf]                  # the engine's input order: "clip" follows "sig"
+        else:
+            x, t, c = ex._prep(inp["x"], inp["timesteps"], inp["context"])
+            order = [x, t, c, sig]
+            want = ex.denoise_step(*order).clone()
+        li = cf.shape[1] if family == "wan_clip" else 0
         make = lambda backend, w: spmd.SpmdWanEngine(ex, B, x.shape[2], 128, 192, c.shape[1], weights=w,  # noqa: E731
-                                                     backend=backend)
+                                                     backend=backend, clip_tokens=li)
     res = {}
     for backend, tma_peer in (("fused", "1"), ("fused", "0"), ("nccl", "0")):
         os.environ["PA_TMA_PEER"] = tma_peer
