@@ -648,19 +648,19 @@ class ParallelEngine:
         lead_dev = self.lead_device
         lead_stream = torch.cuda.current_stream(lead_dev)
         bf = torch.bfloat16
-        key = sp.io_key(x, context, kwargs)
+        key = sp.io_key(x, timesteps, context, kwargs)
         io = self._io.get(key)
         if io is None:
             io = {"x": torch.empty(tuple(x.shape), dtype=bf, device=lead_dev),
                   "out": torch.empty(sp.out_shape(x), dtype=bf, device=lead_dev),
-                  "slots": [sp.slot_buffers(slot.device, x, context, kwargs) for slot in self.slots]}
+                  "slots": [sp.slot_buffers(slot.device, x, timesteps, context, kwargs) for slot in self.slots]}
             if len(self._io) >= 8:
                 self._io.pop(next(iter(self._io)))
             self._io[key] = io
         t0 = time.perf_counter()
         xs, out = io["x"], io["out"]
         xs.copy_(x, non_blocking=True)
-        wss = sp.workspace(*sp.geometry(x, context, kwargs))
+        wss = sp.workspace(*sp.geometry(x, timesteps, context, kwargs))
         for g, (slot, st) in enumerate(zip(self.slots, io["slots"])):
             with torch.cuda.device(slot.device), torch.cuda.stream(slot.stream), torch.no_grad():
                 slot.stream.wait_stream(lead_stream)

@@ -101,11 +101,13 @@ def builder_for(module: nn.Module) -> Optional[Callable]:
             from .flux_exec import build_flux_executor
             return build_flux_executor
     elif fam == "wan":
-        # in_dim 36: WAN2.2 image-to-video ([noise | mask | image latent]).  A CLIP image embedding (WAN2.1 I2V / FLF2V,
-        # Fun-InP) gets the executor with the image cross-attention only when its structure is complete; anything else
-        # with ``img_emb`` keeps the torch replica, which must not drop ``clip_fea``
-        if (p.dim // p.num_heads == 128 and tuple(p.patch_size) == (1, 2, 2) and p.in_dim in (16, 36)
-                and p.out_dim == 16):
+        # (in_dim, out_dim) = (36, 16): WAN2.2 image-to-video ([noise | mask | image latent]); (48, 48): WAN2.2 TI2V-5B
+        # (WAN2.2 VAE latent, per-frame timesteps).  A CLIP image embedding (WAN2.1 I2V / FLF2V, Fun-InP) gets the
+        # executor with the image cross-attention only when its structure is complete; anything else with ``img_emb``
+        # keeps the torch replica, which must not drop ``clip_fea``
+        from .wan_exec import WAN_CHANNELS
+        if (p.dim // p.num_heads == 128 and tuple(p.patch_size) == (1, 2, 2)
+                and (p.in_dim, p.out_dim) in WAN_CHANNELS):
             if not p.has_img_emb and not p.img_cross_attn:
                 from .wan_exec import build_wan_executor
                 return build_wan_executor

@@ -107,6 +107,10 @@ class DiTExecutor(nn.Module):
     def _geometry(shape, context) -> tuple:
         return (shape[0],) + tuple(shape[2:]) + (context.shape[1],)
 
+    def _geometry_of(self, shape, inputs: tuple) -> tuple:
+        """Workspace geometry of a step with latent ``shape`` and step inputs ``inputs`` (timesteps first)."""
+        return self._geometry(shape, *self._conditioning(inputs))
+
     @staticmethod
     def _conditioning(inputs: tuple) -> tuple:
         """The step inputs that ``_geometry``, ``_prepare_ctx`` and ``_cond_sig`` take: the context (WAN with CLIP image
@@ -134,14 +138,15 @@ class DiTExecutor(nn.Module):
 
     def _shard_args(self, x_src_ptr: int, shape, out_ptr: int, out_sample_off: int, *step_inputs):
         inputs = self._inputs(shape[0], *step_inputs)
-        key = ("shard", tuple(shape), tuple(inputs[1].shape), x_src_ptr, out_ptr, out_sample_off) + _ptrs(inputs)
+        key = (("shard", tuple(shape), tuple(inputs[1].shape), x_src_ptr, out_ptr, out_sample_off) + _ptrs(inputs)
+               + (tuple(inputs[0].shape),))
         return key, inputs
 
     # ------------------------------------------------------------------ step entry points
     def _forward(self, x, *step_inputs):
         with torch.cuda.device(self.device):
             x, *inputs = self._prep(x, *step_inputs)
-            ws = self.workspace(*self._geometry(x.shape, *self._conditioning(inputs)))
+            ws = self.workspace(*self._geometry_of(x.shape, inputs))
             out = torch.empty(self.out_shape(tuple(x.shape)), dtype=x.dtype, device=x.device)
             if self._prepare_ctx is not None:
                 self._prepare_ctx(ws, *self._conditioning(inputs))
@@ -151,7 +156,7 @@ class DiTExecutor(nn.Module):
     def _forward_shard(self, x_src_ptr: int, shape, out_ptr: int, out_sample_off: int, *step_inputs) -> None:
         with torch.cuda.device(self.device):
             key, inputs = self._shard_args(x_src_ptr, shape, out_ptr, out_sample_off, *step_inputs)
-            ws = self.workspace(*self._geometry(shape, *self._conditioning(inputs)))
+            ws = self.workspace(*self._geometry_of(shape, inputs))
             if self._prepare_ctx is not None:
                 self._prepare_ctx(ws, *self._conditioning(inputs))
             self._graphs.run(key, lambda: self._run(ws, x_src_ptr, *inputs, None, out_ptr=out_ptr,
@@ -161,7 +166,7 @@ class DiTExecutor(nn.Module):
         with torch.cuda.device(self.device):
             key, inputs = self._shard_args(x_src_ptr, shape, out_ptr, out_sample_off, *step_inputs)
             if self._prepare_ctx is not None:
-                ws = self.workspace(*self._geometry(shape, *self._conditioning(inputs)))
+                ws = self.workspace(*self._geometry_of(shape, inputs))
                 if ws["ctx_sig"] != self._cond_sig(*self._conditioning(inputs)):
                     return 0                # conditioning changed: take the Python path once (eager precompute)
         return self._graphs.exec_handle(key)
@@ -169,7 +174,7 @@ class DiTExecutor(nn.Module):
     def _denoise(self, x, inputs: tuple, sigmas, out, out_ptr, out_sample_off, x_src_ptr, t_src_ptr, **src_ptrs):
         """``src_ptrs``: peer pointers of family-specific per-sample inputs, passed on to ``_run`` (FLUX: ``g_ptr``)."""
         with torch.cuda.device(self.device):
-            ws = self.workspace(*self._geometry(x.shape, *self._conditioning(inputs)))
+            ws = self.workspace(*self._geometry_of(x.shape, inputs))
             if out is None and out_ptr is None:
                 out = ws["OUT"]
             if self._prepare_ctx is not None:
@@ -181,7 +186,8 @@ class DiTExecutor(nn.Module):
                           x_copy=x if (x_src_ptr is not None and self.fused_embed) else None, **src_ptrs)
 
             key = ((tuple(x.shape), tuple(inputs[1].shape), out_ptr or 0, out_sample_off, x_src_ptr or 0, t_src_ptr or 0)
-                   + tuple(p or 0 for p in src_ptrs.values()) + _ptrs((x, sigmas, out) + tuple(inputs)))
+                   + tuple(p or 0 for p in src_ptrs.values()) + _ptrs((x, sigmas, out) + tuple(inputs))
+                   + (tuple(inputs[0].shape),))
             self._graphs.run(key, body)
             return out
 

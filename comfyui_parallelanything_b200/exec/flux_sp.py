@@ -88,16 +88,16 @@ class FluxUlysses(UlyssesBase):
         H, Wd, Lt = x.shape[2], x.shape[3], context.shape[1]
         return H % 2 == 0 and Wd % 2 == 0 and Lt % n == 0 and ((H // 2) * (Wd // 2)) % n == 0 and Lt >= n
 
-    def geometry(self, x, context, kwargs=None) -> tuple:
+    def geometry(self, x, timesteps, context, kwargs=None) -> tuple:
         return (x.shape[2], x.shape[3], context.shape[1])
 
-    def io_key(self, x, context, kwargs) -> tuple:
+    def io_key(self, x, timesteps, context, kwargs) -> tuple:
         y = kwargs.get("y")
         return ("sp", tuple(x.shape), tuple(context.shape), None if y is None else tuple(y.shape),
                 kwargs.get("guidance") is not None)
 
-    def slot_buffers(self, device, x, context, kwargs) -> dict:
-        st = super().slot_buffers(device, x, context, kwargs)
+    def slot_buffers(self, device, x, timesteps, context, kwargs) -> dict:
+        st = super().slot_buffers(device, x, timesteps, context, kwargs)
         bf = torch.bfloat16
         st["y"] = torch.zeros(1, self.ex[0].params.vec_in_dim, dtype=bf, device=device)
         st["g"] = torch.ones(1, dtype=bf, device=device)

@@ -52,7 +52,7 @@ class UlyssesBase:
     def accepts(self, x, context) -> bool:
         raise NotImplementedError
 
-    def geometry(self, x, context, kwargs=None) -> tuple:
+    def geometry(self, x, timesteps, context, kwargs=None) -> tuple:
         raise NotImplementedError
 
     def out_shape(self, x) -> tuple:
@@ -62,21 +62,23 @@ class UlyssesBase:
     def workspace(self, *geometry) -> list:
         raise NotImplementedError
 
-    def slot_buffers(self, device, x, context, kwargs) -> dict:
+    def slot_buffers(self, device, x, timesteps, context, kwargs) -> dict:
         """Fixed per-GPU staging buffers for the step inputs other than the latent (a sampler passes fresh tensors)."""
         bf = torch.bfloat16
         return {"t": torch.empty(1, dtype=bf, device=device),
                 "ctx": torch.empty(tuple(context.shape), dtype=bf, device=device), "ctx_src": None}
 
     def stage(self, st: dict, timesteps, context, kwargs, cache_conditioning: bool) -> None:
-        """Copy this step's inputs into one GPU's staging buffers (called on that GPU's stream)."""
-        st["t"].copy_(timesteps.reshape(-1)[:1], non_blocking=True)
+        """Copy this step's inputs into one GPU's staging buffers (called on that GPU's stream).  The ``"t"`` buffer's
+        shape says how many timesteps are staged: one, or one per latent frame (WAN2.2 TI2V)."""
+        t = st["t"]
+        t.copy_(timesteps.reshape(-1)[:t.numel()].view(t.shape), non_blocking=True)
         ident = (id(context), context.data_ptr(), context._version)
         if not cache_conditioning or st["ctx_src"] is None or st["ctx_src"][0] != ident:
             st["ctx"].copy_(context, non_blocking=True)
             st["ctx_src"] = (ident, context)
 
-    def io_key(self, x, context, kwargs) -> tuple:
+    def io_key(self, x, timesteps, context, kwargs) -> tuple:
         return ("sp", tuple(x.shape), tuple(context.shape))
 
     def pre_step(self, g: int, wss, st: dict) -> None:

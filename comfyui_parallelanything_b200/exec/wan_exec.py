@@ -6,7 +6,10 @@ LayerNorm kernel) plus what WAN needs on top:
   * the video latent ``[B, in_dim, T, H, W]`` is patchified by the fused scatter kernel as a ``T*H`` tall image
     (Conv3d(1,2,2) == the same 2x2 patch GEMM applied per frame), timestep sinusoid included.  ``in_dim`` is 16 for
     text-to-video and 36 for WAN2.2 image-to-video, whose input is ``[noise 16 | mask 4 | image latent 16]``; the output
-    and the Euler update always cover the ``out_dim`` = 16 noise channels;
+    and the Euler update cover the ``out_dim`` = 16 noise channels.  WAN2.2 TI2V-5B has 48 channels in and out;
+  * per-frame timesteps (WAN2.2 TI2V, ``[B, T]``): the time path embeds ``B*T`` timesteps, and the LayerNorm kernel and
+    the gated-residual epilogues look up each row's modulation vectors by frame (``mod_rows`` / ``gate_rows`` = tokens
+    per frame) instead of by sample;
   * q/k use a *full-width* RMSNorm (over all heads) followed by 3-D RoPE: a dedicated in-place kernel on
     the fused QKV GEMM output; attention then reads q/k/v through strided 4-D TMA views;
   * per-block modulation = learned table + time projection: one broadcast-add kernel builds all 40x6
@@ -29,16 +32,36 @@ from ..models import flux as flux_model
 from ..models import wan as wan_model
 
 
+#: (in_dim, out_dim) of the WAN models the executor runs: text-to-video, WAN2.2 image-to-video, WAN2.2 TI2V-5B
+WAN_CHANNELS = ((16, 16), (36, 16), (48, 48))
+
+
+def frame_steps(timesteps: torch.Tensor, shape) -> int:
+    """Timesteps per sample of a step on a latent of ``shape`` [B, C, T, H, W]: 1 for ``[B]`` / ``[B, 1]``, T for one
+    per latent frame ``[B, T]`` (WAN2.2 TI2V).  Any other shape raises ``ValueError``."""
+    if timesteps.dim() <= 1 or (timesteps.dim() == 2 and timesteps.shape[1] == 1):
+        return 1
+    if timesteps.dim() == 2 and tuple(timesteps.shape) == (shape[0], shape[2]):
+        return int(shape[2])
+    raise ValueError(f"timesteps must be [B], [B, 1] or one per latent frame [B, T] = {(shape[0], shape[2])}, got "
+                     f"{tuple(timesteps.shape)}")
+
+
 class WanExecutor(DiTExecutor):
+    """WAN2.x DiT step on the native kernels.  ``timesteps`` are ``[B]``, ``[B, 1]`` or one per latent frame ``[B, T]``
+    (WAN2.2 TI2V: ComfyUI turns the denoise mask into 0 on the start-image frame and t elsewhere).
+    ``denoise_step`` applies one Euler update per sample with its ``sigmas`` [B, 2] to every frame; keeping the
+    start-image frame fixed is the sampler's denoise-mask blend, not the model's."""
+
     pa_family = "wan"
 
     def __init__(self, model: "wan_model.WanModel", device, cuda_graphs: bool = False, fp8: bool = False):
         super().__init__(model, device, cuda_graphs)
         d, p = self.device, self.params
         self.dim, self.heads = p.dim, p.num_heads
-        if p.dim // p.num_heads != 128 or tuple(p.patch_size) != (1, 2, 2) or p.in_dim not in (16, 36) or p.out_dim != 16:
-            raise ValueError("WanExecutor is specialised for head_dim 128, patch (1,2,2), 16 (T2V) or 36 (I2V) input "
-                             "and 16 output latent channels")
+        if p.dim // p.num_heads != 128 or tuple(p.patch_size) != (1, 2, 2) or (p.in_dim, p.out_dim) not in WAN_CHANNELS:
+            raise ValueError("WanExecutor is specialised for head_dim 128, patch (1,2,2) and (input, output) latent "
+                             f"channels in {WAN_CHANNELS}")
         W: Dict[str, Optional[torch.Tensor]] = {}
 
         def lin(name, m):
@@ -98,7 +121,17 @@ class WanExecutor(DiTExecutor):
         """[B, in_dim, T, H, W] -> [B, out_dim, T, H, W] (image-to-video predicts only the noise channels)."""
         return (shape[0], self.params.out_dim) + tuple(shape[2:])
 
-    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int) -> dict:
+    def _inputs(self, B: int, timesteps, context) -> tuple:
+        if timesteps.dim() == 2 and timesteps.shape[1] == 1:
+            timesteps = timesteps.reshape(-1)
+        return super()._inputs(B, timesteps, context)
+
+    def _geometry_of(self, shape, inputs: tuple) -> tuple:
+        """``_geometry`` + the timesteps per sample (1, or T with per-frame timesteps)."""
+        return super()._geometry_of(shape, inputs) + (frame_steps(inputs[0], shape),)
+
+    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int, Tt: int = 1) -> dict:
+        """``Tt`` timesteps per sample: the time path and the modulation tables have ``B*Tt`` rows."""
         d, dim = self.device, self.dim
         L = T * (H // 2) * (Wd // 2)
         e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=d)  # noqa: E731
@@ -107,10 +140,11 @@ class WanExecutor(DiTExecutor):
         ws["QKV"] = e(B, L, 3 * dim)
         ws["ATT"] = e(B, L, dim)
         ws["FF"] = e(B, L, self.params.ffn_dim)
-        ws["T1"], ws["E_H"], ws["E"], ws["SE"] = e(B, 256), e(B, dim), e(B, dim), e(B, dim)
-        ws["E0"] = e(B, 6 * dim)
-        ws["MOD"] = e(B, self.n_blocks, 6 * dim)
-        ws["HSHIFT"], ws["HSCALE"] = e(B, 1, dim), e(B, 1, dim)
+        n = B * Tt
+        ws["T1"], ws["E_H"], ws["E"], ws["SE"] = e(n, 256), e(n, dim), e(n, dim), e(n, dim)
+        ws["E0"] = e(n, 6 * dim)
+        ws["MOD"] = e(n, self.n_blocks, 6 * dim)
+        ws["HSHIFT"], ws["HSCALE"] = e(n, 1, dim), e(n, 1, dim)
         ws["CTX_H"], ws["CTX"] = e(B, Lc, dim), e(B, Lc, dim)
         ws["CQ"] = e(B, L, dim)
         ws["CKV"] = [e(B, Lc, 2 * dim) for _ in range(self.n_blocks)]
@@ -153,9 +187,11 @@ class WanExecutor(DiTExecutor):
         n = 0
         X, XM, QKV, ATT, FF, MOD, ROPE = ws["X"], ws["XM"], ws["QKV"], ws["ATT"], ws["FF"], ws["MOD"], ws["ROPE"]
         TH = ws["T"] * ws["H"]
-        # fused scatter: video latent (as a T*H tall image) -> patch GEMM ; timestep sinusoid
+        # per-frame timesteps: every row looks its modulation vectors up by frame (tokens per frame rows per vector)
+        fr = frame_lookup(ws)
+        # fused scatter: video latent (as a T*H tall image) -> patch GEMM ; sinusoids of all B*Tt timesteps
         C.scatter_patch_embed(W["patch.w"], W["patch.b"], x_ptr, t_ptr if t_ptr is not None else t.data_ptr(), 0,
-                              ws["T1"], None, x_copy, X, self.params.in_dim, TH, ws["Wd"], 1.0)
+                              ws["T1"], None, x_copy, X, self.params.in_dim, TH, ws["Wd"], 1.0, ws["T1"].shape[0])
         ops.gemm(ws["T1"], W["time0.w"], "silu", out=ws["E_H"], bias=W["time0.b"])
         ops.gemm(ws["E_H"], W["time2.w"], "bias", out=ws["E"], bias=W["time2.b"])
         C.silu(ws["E"], ws["SE"])
@@ -170,12 +206,12 @@ class WanExecutor(DiTExecutor):
 
         for i in range(self.n_blocks):
             # ---- self attention
-            ops.layernorm_modulate(X, XM, scale=mod(i, 1), shift=mod(i, 0), eps=self.eps)
+            ops.layernorm_modulate(X, XM, scale=mod(i, 1), shift=mod(i, 0), eps=self.eps, **fr["ln"])
             n += block_linear(W, XM, f"b{i}.qkv", "bias", out=QKV)
             C.rms_rope(QKV[:, :, :dim], W[f"b{i}.nq"], ROPE, self.eps)
             C.rms_rope(QKV[:, :, dim:2 * dim], W[f"b{i}.nk"], ROPE, self.eps)
             ops.attention(self._heads(QKV, 0, 3), self._heads(QKV, 1, 3), self._heads(QKV, 2, 3), out=ATT)
-            n += block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2))
+            n += block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2), **fr["gate"])
             # ---- text cross attention
             ops.layernorm_modulate(X, XM, gamma=W[f"b{i}.n3.g"], beta=W[f"b{i}.n3.b"], eps=self.eps)
             n += block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
@@ -183,12 +219,12 @@ class WanExecutor(DiTExecutor):
             self._cross_attention(ws, i, ATT)
             n += block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
             # ---- FFN
-            ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=self.eps)
+            ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=self.eps, **fr["ln"])
             n += block_linear(W, XM, f"b{i}.f0", "gelu", out=FF)
-            n += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5))
+            n += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5), **fr["gate"])
             n += 8
         # ---- head: AdaLN + Linear + unpatchify (+ Euler, + peer store)
-        ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=self.eps)
+        ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=self.eps, **fr["ln"])
         p = self.params
         head_gather(XM, W["head.w"], W["head.b"], p.out_dim, TH, ws["Wd"], out=out, out_ptr=out_ptr,
                     out_sample_off=out_sample_off, x_in=x_in, sigmas=sigmas,
@@ -200,6 +236,17 @@ class WanExecutor(DiTExecutor):
     @torch.no_grad()
     def forward(self, x, timesteps, context=None, clip_fea=None, transformer_options=None, **kwargs):
         return self._forward(x, timesteps, context)
+
+
+def frame_lookup(ws: dict, row_off: int = 0) -> dict:
+    """Keyword arguments that make the LayerNorm kernel (``"ln"``) and the gated-residual GEMMs (``"gate"``) of a
+    workspace with per-frame timesteps read frame ``(global row) / (tokens per frame)`` of the ``B*T``-row modulation
+    tables; ``row_off``: global token index of the workspace's first row (a sequence-parallel slice).  Empty with one
+    timestep per sample, so those launches stay the per-sample ones."""
+    if ws["T1"].shape[0] == ws["B"]:
+        return {"ln": {}, "gate": {}}
+    hw = (ws["H"] // 2) * (ws["Wd"] // 2)
+    return {"ln": dict(mod_rows=hw, mod_row_off=row_off), "gate": dict(gate_rows=hw, gate_row_off=row_off)}
 
 
 def build_wan_executor(model: nn.Module, device, **kw) -> WanExecutor:
@@ -252,8 +299,8 @@ class WanClipExecutor(WanExecutor):
     def _cond_sig(context, clip_fea=None) -> tuple:
         return conditioning_sig(context), (conditioning_sig(clip_fea) if clip_fea is not None else None)
 
-    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int, Li: int = 0) -> dict:
-        ws = super()._new_workspace(B, T, H, Wd, Lc)
+    def _new_workspace(self, B: int, T: int, H: int, Wd: int, Lc: int, Li: int = 0, Tt: int = 1) -> dict:
+        ws = super()._new_workspace(B, T, H, Wd, Lc, Tt)
         e = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=self.device)  # noqa: E731
         ws["Li"] = Li
         if Li:

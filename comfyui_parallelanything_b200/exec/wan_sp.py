@@ -10,6 +10,9 @@ latency as one GPU.  Here, as for FLUX (``flux_sp.py``):
   * self-attention runs on ``H / N`` heads over ALL tokens: one peer-pull exchange turns [my tokens, all heads] into
     [all tokens, my heads] before it and one turns the result back after it (csrc/comm/sp_a2a.cu, device-side flag
     handshake, epochs in device memory -> the whole share of a GPU is one CUDA graph);
+  * per-frame timesteps (WAN2.2 TI2V): the replicated time path embeds one timestep per latent frame, and the
+    LayerNorm / gated-residual lookups use the slice's global token index, so a slice that starts mid-frame reads the
+    right frame's modulation vectors;
   * text cross-attention needs no exchange: every GPU holds the (step-invariant, cached) K/V of the 512 text tokens and
     attends with its own query tokens; WAN2.1 I2V / FLF2V hold the image K/V of the CLIP tokens the same way and run the
     executor's two-source cross-attention;
@@ -25,6 +28,7 @@ from .. import ops
 from . import block_linear
 from .dit import head_gather
 from .sp_common import UlyssesBase, attention_variant
+from .wan_exec import frame_lookup, frame_steps
 
 
 def supported(executors) -> Optional[str]:
@@ -92,8 +96,11 @@ class WanUlysses(UlyssesBase):
         c = kwargs.get("clip_fea")
         return c if isinstance(c, torch.Tensor) else None
 
-    def slot_buffers(self, device, x, context, kwargs) -> dict:
-        st = super().slot_buffers(device, x, context, kwargs)
+    def slot_buffers(self, device, x, timesteps, context, kwargs) -> dict:
+        st = super().slot_buffers(device, x, timesteps, context, kwargs)
+        tt = frame_steps(timesteps, x.shape)
+        if tt > 1:
+            st["t"] = torch.empty(1, tt, dtype=torch.bfloat16, device=device)      # one timestep per latent frame
         clip = self._clip(kwargs)
         if clip is not None:
             st["clip"], st["clip_src"] = torch.empty(tuple(clip.shape), dtype=torch.bfloat16, device=device), None
@@ -108,16 +115,20 @@ class WanUlysses(UlyssesBase):
                 st["clip"].copy_(clip, non_blocking=True)
                 st["clip_src"] = (ident, clip)
 
-    def io_key(self, x, context, kwargs) -> tuple:
+    def io_key(self, x, timesteps, context, kwargs) -> tuple:
         clip = self._clip(kwargs)
-        return super().io_key(x, context, kwargs) + ((tuple(clip.shape),) if clip is not None else ())
+        return (super().io_key(x, timesteps, context, kwargs) + ((tuple(clip.shape),) if clip is not None else ())
+                + (frame_steps(timesteps, x.shape),))
 
-    def geometry(self, x, context, kwargs=None) -> tuple:
+    def geometry(self, x, timesteps, context, kwargs=None) -> tuple:
         clip = self._clip(kwargs or {})
-        return (x.shape[2], x.shape[3], x.shape[4], context.shape[1], clip.shape[1] if clip is not None else 0)
+        return (x.shape[2], x.shape[3], x.shape[4], context.shape[1], clip.shape[1] if clip is not None else 0,
+                frame_steps(timesteps, x.shape))
 
-    def workspace(self, T: int, H: int, Wd: int, Lc: int, Li: int = 0) -> list:
-        key = (T, H, Wd, Lc, Li)
+    def workspace(self, T: int, H: int, Wd: int, Lc: int, Li: int = 0, Tt: int = 1) -> list:
+        """``Tt`` timesteps (1, or one per latent frame): the replicated time path and modulation tables have Tt
+        rows."""
+        key = (T, H, Wd, Lc, Li, Tt)
         got = self._ws.get(key)
         if got is not None:
             return got
@@ -137,10 +148,10 @@ class WanUlysses(UlyssesBase):
             ws["ATTF"] = e(1, L, hpg * 128)
             ws["ATT"] = e(1, Ll, dim)
             ws["FF"] = e(1, Ll, ex.params.ffn_dim)
-            ws["T1"], ws["E_H"], ws["E"], ws["SE"] = e(1, 256), e(1, dim), e(1, dim), e(1, dim)
-            ws["E0"] = e(1, 6 * dim)
-            ws["MOD"] = e(1, ex.n_blocks, 6 * dim)
-            ws["HSHIFT"], ws["HSCALE"] = e(1, 1, dim), e(1, 1, dim)
+            ws["T1"], ws["E_H"], ws["E"], ws["SE"] = e(Tt, 256), e(Tt, dim), e(Tt, dim), e(Tt, dim)
+            ws["E0"] = e(Tt, 6 * dim)
+            ws["MOD"] = e(Tt, ex.n_blocks, 6 * dim)
+            ws["HSHIFT"], ws["HSCALE"] = e(Tt, 1, dim), e(Tt, 1, dim)
             ws["CTX_H"], ws["CTX"] = e(1, Lc, dim), e(1, Lc, dim)
             ws["CQ"] = e(1, Ll, dim)
             ws["CKV"] = [e(1, Lc, 2 * dim) for _ in range(ex.n_blocks)]
@@ -176,7 +187,8 @@ class WanUlysses(UlyssesBase):
         L, Ll, hpg = ws["L"], ws["Ll"], ws["hpg"]
         X, XM, QKV, ATT, FF, MOD, ROPE = ws["X"], ws["XM"], ws["QKV"], ws["ATT"], ws["FF"], ws["MOD"], ws["ROPE"]
         TH = ws["T"] * ws["H"]
-        t = st["t"]
+        t = st["t"].reshape(-1)
+        fr = frame_lookup(ws, row_off=g * Ll)             # per-frame timesteps: frame of each global token row
         nl = 0
         # ---- embedders: patchify the whole clip (a T*H tall image), embed only my token slice; time path is replicated
         C.patchify(x_ptr, ws["TOK"], 1, ex.params.in_dim, TH, ws["Wd"], 2)
@@ -201,7 +213,7 @@ class WanUlysses(UlyssesBase):
         slot = 0
         for i in range(ex.n_blocks):
             # ---- self attention: token-sliced QKV + q/k norm + RoPE, head-sliced attention between two exchanges
-            ops.layernorm_modulate(X, XM, scale=mod(i, 1), shift=mod(i, 0), eps=ex.eps)
+            ops.layernorm_modulate(X, XM, scale=mod(i, 1), shift=mod(i, 0), eps=ex.eps, **fr["ln"])
             nl += block_linear(W, XM, f"b{i}.qkv", "bias", out=QKV)
             C.rms_rope(QKV[:, :, :dim], W[f"b{i}.nq"], ROPE, ex.eps)
             C.rms_rope(QKV[:, :, dim:2 * dim], W[f"b{i}.nk"], ROPE, ex.eps)
@@ -210,7 +222,7 @@ class WanUlysses(UlyssesBase):
                           variant=att_variant)
             self._exchange(g, ws, slot + 1, "ATT")
             slot += 2
-            nl += 8 + block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2))
+            nl += 8 + block_linear(W, ATT, f"b{i}.o", "gate_res", out=X, residual=X, gate=mod(i, 2), **fr["gate"])
             # ---- cross attention: my query tokens against the replicated text (and image) K/V
             ops.layernorm_modulate(X, XM, gamma=W[f"b{i}.n3.g"], beta=W[f"b{i}.n3.b"], eps=ex.eps)
             nl += block_linear(W, XM, f"b{i}.cq", "bias", out=ws["CQ"])
@@ -218,11 +230,11 @@ class WanUlysses(UlyssesBase):
             ex._cross_attention(ws, i, ATT)
             nl += 3 + block_linear(W, ATT, f"b{i}.co", "res", out=X, residual=X)
             # ---- FFN
-            ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=ex.eps)
+            ops.layernorm_modulate(X, XM, scale=mod(i, 4), shift=mod(i, 3), eps=ex.eps, **fr["ln"])
             nl += 1 + block_linear(W, XM, f"b{i}.f0", "gelu", out=FF)
-            nl += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5))
+            nl += block_linear(W, FF, f"b{i}.f2", "gate_res", out=X, residual=X, gate=mod(i, 5), **fr["gate"])
         # ---- head on my tokens: AdaLN + Linear + unpatchify, rows stored into the LEAD GPU's output
-        ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=ex.eps)
+        ops.layernorm_modulate(X, XM, scale=ws["HSCALE"][:, 0], shift=ws["HSHIFT"][:, 0], eps=ex.eps, **fr["ln"])
         head_gather(XM, W["head.w"], W["head.b"], ex.params.out_dim, TH, ws["Wd"], out_ptr=out_ptr, tok_off=g * Ll)
         self._end_step(g)
         nl += 3

@@ -57,7 +57,7 @@ class ZImageUlysses(UlyssesBase):
         H, Wd, Lc = x.shape[2], x.shape[3], context.shape[1]
         return H % 2 == 0 and Wd % 2 == 0 and Lc % n == 0 and ((H // 2) * (Wd // 2)) % n == 0 and Lc >= n
 
-    def geometry(self, x, context, kwargs=None) -> tuple:
+    def geometry(self, x, timesteps, context, kwargs=None) -> tuple:
         return (x.shape[2], x.shape[3], context.shape[1])
 
     def workspace(self, H: int, Wd: int, Lc: int) -> list:

@@ -4,7 +4,9 @@ Shape of the public WAN 2.1/2.2 T2V transformer as ComfyUI instantiates it:
 ``patch_embedding`` Conv3d(1,2,2), text/time embedders, ``blocks`` of
 (self-attn with full-width RMS q/k norm + 3-D RoPE, cross-attn to the text,
 GELU-tanh FFN) modulated by a 6-way time projection, and a modulated head.
-WAN2.2-A14B uses dim 5120 / ffn 13824 / 40 heads / 40 layers per expert.
+WAN2.2-A14B uses dim 5120 / ffn 13824 / 40 heads / 40 layers per expert.  WAN2.2-TI2V-5B (48 latent channels in and
+out, WAN2.2 VAE) also takes one timestep per latent frame: ``timesteps`` [B, T_lat] modulate each frame's tokens with
+that frame's vectors.
 
 Note the block list is called ``blocks`` — the reference's pipeline planner only
 looks at ``double_blocks/single_blocks/transformer_blocks/layers``
@@ -59,6 +61,13 @@ def wan21_i2v_14b_params() -> WanParams:
 def wan21_flf2v_14b_params() -> WanParams:
     """WAN2.1-FLF2V-14B (first and last frame): as I2V, with 2 x 257 CLIP tokens and their position embedding."""
     return WanParams(in_dim=36, clip_dim=1280, clip_pos_tokens=514)
+
+
+def wan22_ti2v_5b_params() -> WanParams:
+    """WAN2.2-TI2V-5B: 48 latent channels in and out (WAN2.2 VAE, 16x spatial and 4x temporal compression), dim 3072,
+    30 layers.  In image-to-video mode it takes per-frame timesteps (``ti2v_inputs``)."""
+    return WanParams(in_dim=48, out_dim=48, dim=3072, ffn_dim=14336, num_heads=24, num_layers=30, text_dim=4096,
+                     freq_dim=256)
 
 
 def wan_tiny_params() -> WanParams:
@@ -131,6 +140,11 @@ class WanI2VCrossAttention(WanCrossAttention):
         return self.o(o.transpose(1, 2).reshape(b, s, n * d))
 
 
+def frame_rows(v: torch.Tensor, tokens: int) -> torch.Tensor:
+    """Per-frame vectors [B, T, dim] -> per-token [B, tokens, dim]: frame f's vector on each of its tokens/T tokens."""
+    return v.repeat_interleave(tokens // v.shape[1], dim=1)
+
+
 class WanImageProjection(nn.Module):
     """ComfyUI's ``MLPProj``: CLIP vision features [B, Li, 1280] -> [B, Li, dim] image context tokens.
     ``proj = LayerNorm, Linear, GELU (exact erf), Linear, LayerNorm`` (both norms affine); FLF2V adds ``emb_pos``
@@ -160,7 +174,10 @@ class WanAttentionBlock(nn.Module):
         self.modulation = nn.Parameter(torch.randn(1, 6, dim) / dim ** 0.5)
 
     def forward(self, x, e, freqs, context, context_img_len=None):
-        e = (self.modulation.to(e.dtype) + e).chunk(6, dim=1)
+        if e.dim() == 4:            # per-frame timesteps: e [B, T, 6, dim]
+            e = [frame_rows(v, x.shape[1]) for v in (self.modulation.to(e.dtype).unsqueeze(0) + e).unbind(2)]
+        else:
+            e = (self.modulation.to(e.dtype) + e).chunk(6, dim=1)
         y = self.self_attn(self.norm1(x) * (1 + e[1]) + e[0], freqs)
         x = x + y * e[2]
         if isinstance(self.cross_attn, WanI2VCrossAttention):
@@ -179,7 +196,11 @@ class Head(nn.Module):
         self.modulation = nn.Parameter(torch.randn(1, 2, dim) / dim ** 0.5)
 
     def forward(self, x, e):
-        e = (self.modulation.to(e.dtype) + e.unsqueeze(1)).chunk(2, dim=1)
+        if e.dim() == 3:            # per-frame timesteps: e [B, T, dim]
+            e = (self.modulation.to(e.dtype).unsqueeze(0) + e.unsqueeze(2)).unbind(2)
+            e = [frame_rows(v, x.shape[1]) for v in e]
+        else:
+            e = (self.modulation.to(e.dtype) + e.unsqueeze(1)).chunk(2, dim=1)
         return self.head(self.norm(x) * (1 + e[1]) + e[0])
 
 
@@ -232,12 +253,21 @@ class WanModel(nn.Module):
         return u.reshape(b, c, t * pt, h * ph, w * pw)
 
     def forward(self, x, timesteps, context=None, clip_fea=None, transformer_options=None, **kwargs):
-        # x: [B, C, T, H, W]
+        # x: [B, C, T, H, W]; timesteps: [B], [B, 1] or one per latent frame [B, T] (WAN2.2 TI2V)
         x = self.patch_embedding(x)
         grid = x.shape[2:]
         x = x.flatten(2).transpose(1, 2)
-        e = self.time_embedding(timestep_embedding(timesteps, self.freq_dim, time_factor=1.0).to(x.dtype))
-        e0 = self.time_projection(e).unflatten(1, (6, self.dim))
+        if timesteps.dim() == 2 and timesteps.shape[1] == 1:
+            timesteps = timesteps[:, 0]
+        if timesteps.dim() == 2:
+            if timesteps.shape[1] != grid[0]:
+                raise ValueError(f"per-frame timesteps {tuple(timesteps.shape)} do not match {grid[0]} latent frames")
+            e = self.time_embedding(timestep_embedding(timesteps.flatten(), self.freq_dim, time_factor=1.0).to(x.dtype))
+            e = e.unflatten(0, tuple(timesteps.shape))                          # [B, T, dim]
+            e0 = self.time_projection(e).unflatten(2, (6, self.dim))           # [B, T, 6, dim]
+        else:
+            e = self.time_embedding(timestep_embedding(timesteps, self.freq_dim, time_factor=1.0).to(x.dtype))
+            e0 = self.time_projection(e).unflatten(1, (6, self.dim))
         ctx = self.text_embedding(context)
         context_img_len = None
         if clip_fea is not None and self.img_emb is not None:
@@ -289,3 +319,20 @@ def clip_inputs(params: WanParams, batch: int, frames: int = 16, height: int = 7
     g = torch.Generator(device="cpu").manual_seed(seed + 1)
     out["clip_fea"] = torch.randn(batch, li, params.clip_dim, generator=g).to(device=device, dtype=dtype)
     return out
+
+
+def ti2v_inputs(params: WanParams, batch: int, frames: int = 121, height: int = 704, width: int = 1280, device="cpu",
+                dtype=torch.bfloat16, seed: int = 0):
+    """WAN2.2 TI2V image-to-video step inputs, as ComfyUI builds them for the 5B model: the WAN2.2 VAE latent
+    [B, 48, (frames - 1) // 4 + 1, height / 16, width / 16] whose first frame holds the encoded start image, and one
+    timestep per latent frame [B, T_lat]: 0 on the image frame, t on every other frame.  1280 x 704 x 121 frames is a
+    31 x 44 x 80 latent (27 280 tokens)."""
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    lt = (frames - 1) // 4 + 1
+    x = torch.randn(batch, params.in_dim, lt, height // 16, width // 16, generator=g)
+    x[:, :, 0] = 0.5 * torch.randn(batch, params.in_dim, height // 16, width // 16, generator=g)    # "image latent"
+    t = (torch.rand(batch, 1, generator=g) * 1000).expand(batch, lt).clone()
+    t[:, 0] = 0.0
+    ctx = torch.randn(batch, params.text_len, params.text_dim, generator=g)
+    return dict(x=x.to(device=device, dtype=dtype), timesteps=t.to(device=device, dtype=dtype),
+                context=ctx.to(device=device, dtype=dtype))

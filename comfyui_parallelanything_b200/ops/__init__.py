@@ -56,7 +56,9 @@ EPI = {
 
 def gemm(a: torch.Tensor, w: torch.Tensor, mode: str = "bias", **kw) -> None:
     """``out = epilogue(a @ w.T)`` on tcgen05 tensor cores.  ``a``: [M,K] or [B,rows,K] view
-    (last dim contiguous), ``w``: [N,K].  See csrc/bind.cpp for the keyword arguments."""
+    (last dim contiguous), ``w``: [N,K].  See csrc/bind.cpp for the keyword arguments; ``gate_res`` with
+    ``gate_rows=`` / ``gate_row_off=`` reads one gate row per group of rows, like ``layernorm_modulate``'s
+    ``mod_rows``."""
     require().gemm(a, w, EPI[mode], **kw)
 
 
@@ -104,10 +106,14 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
     return out
 
 
-def layernorm_modulate(x, out=None, scale=None, shift=None, gamma=None, beta=None, eps: float = 1e-6):
+def layernorm_modulate(x, out=None, scale=None, shift=None, gamma=None, beta=None, eps: float = 1e-6,
+                       mod_rows: int = 0, mod_row_off: int = 0):
+    """``out = LayerNorm(x) [* gamma + beta] * (1 + scale) + shift`` per row; ``scale`` / ``shift``: per-sample [B, D]
+    views.  ``mod_rows`` > 0: [G, D] views with one vector per group of ``mod_rows`` rows instead (a video frame's
+    tokens); row r of sample b reads vector ``(b * rows + r + mod_row_off) // mod_rows``."""
     if out is None:
         out = torch.empty_like(x)
-    require().layernorm_modulate(x, out, scale, shift, gamma, beta, eps)
+    require().layernorm_modulate(x, out, scale, shift, gamma, beta, eps, mod_rows, mod_row_off)
     return out
 
 

@@ -100,7 +100,8 @@ class SpmdFluxEngine:
         self.rank, self.world = dist.get_rank(), dist.get_world_size()
         self.dev = torch.device("cuda", torch.cuda.current_device())
         self.backend = backend
-        self.B, self.H, self.W, self.Lt = global_batch, height // 8, width // 8, txt_len
+        f = self._pixels_per_latent()
+        self.B, self.H, self.W, self.Lt = global_batch, height // f, width // f, txt_len
         self.C = self._latent_channels()
         w = list(weights) if weights is not None else [1.0 / self.world] * self.world
         self.sizes = chain_mod.split_sizes(global_batch, chain_mod.normalize_weights(w), split_mode)
@@ -142,6 +143,10 @@ class SpmdFluxEngine:
                  self.off_local + self.n_local, B, backend)
 
     # -------------------------------------------------------------- family hooks (FLUX defaults)
+    def _pixels_per_latent(self) -> int:
+        """Spatial compression of the family's VAE (pixel size / latent size)."""
+        return 8
+
     def _latent_channels(self) -> int:
         return self.ex.params.in_channels // 4
 
@@ -414,7 +419,8 @@ class _SpmdTextDiTEngine(SpmdFluxEngine):
         if fused:
             self.ex.denoise_step(loc["x"], loc["t"], *cond, loc["sig"],
                                  out_ptr=self.heap.peer_ptr(0, self.off["out"]), out_sample_off=self.off_local,
-                                 x_src_ptr=self._src("x", self._row_bytes("x")), t_src_ptr=self._src("t", 2))
+                                 x_src_ptr=self._src("x", self._row_bytes("x")),
+                                 t_src_ptr=self._src("t", self._row_bytes("t")))
             return None
         return self.ex.denoise_step(loc["x"], loc["t"], *cond, loc["sig"])
 
@@ -422,26 +428,33 @@ class _SpmdTextDiTEngine(SpmdFluxEngine):
 class SpmdWanEngine(_SpmdTextDiTEngine):
     """WAN2.x video DiT replicas (``exec/wan_exec.py``).  ``height``/``width`` are pixel sizes, ``frames`` the
     number of LATENT frames; the video latent is staged as [B, in_dim, T, H/8, W/8] (16 channels for text-to-video, 36
-    for image-to-video) and the result as [B, out_dim = 16, T, H/8, W/8].  Executors with CLIP image conditioning
-    (WAN2.1 I2V / FLF2V) add a ``"clip"`` input [B, clip_tokens, clip_dim] after ``"sig"`` (default 257 tokens, the
-    model's ``clip_pos_tokens`` for FLF2V), read through a peer TMA descriptor like ``"ctx"``."""
+    for image-to-video) and the result as [B, out_dim = 16, T, H/8, W/8].  WAN2.2 TI2V-5B (48 channels in and out) has
+    a 16x VAE: [B, 48, T, H/16, W/16].  ``frame_timesteps``: ``"t"`` is [B, T], one timestep per latent frame (TI2V
+    image-to-video), and the fused patch-embed kernel pulls T of them per sample.  Executors with CLIP image
+    conditioning (WAN2.1 I2V / FLF2V) add a ``"clip"`` input [B, clip_tokens, clip_dim] after ``"sig"`` (default 257
+    tokens, the model's ``clip_pos_tokens`` for FLF2V), read through a peer TMA descriptor like ``"ctx"``."""
 
     tma_peer_inputs = ("ctx", "clip")
 
     def __init__(self, executor, global_batch: int, frames: int, height: int, width: int, txt_len: int,
-                 clip_tokens: int = 0, **kw):
+                 clip_tokens: int = 0, frame_timesteps: bool = False, **kw):
         self.T = frames
+        self.Tt = frames if frame_timesteps else 1
         self.Li = 0
         if getattr(executor, "conditioning_kwargs", ()):
             self.Li = clip_tokens or executor.clip_pos_tokens or 257
         super().__init__(executor, global_batch, height, width, txt_len, **kw)
+
+    def _pixels_per_latent(self) -> int:
+        return 16 if self.ex.params.out_dim == 48 else 8          # WAN2.2 VAE (48 channels) / WAN2.1 VAE
 
     def _latent_channels(self) -> int:
         return self.ex.params.in_dim
 
     def _make_spec(self, B: int) -> dict:
         p, bf = self.ex.params, torch.bfloat16
-        spec = {"x": ((B, self.C, self.T, self.H, self.W), bf), "t": ((B,), bf), "ctx": ((B, self.Lt, p.text_dim), bf),
+        t = (B, self.Tt) if self.Tt > 1 else (B,)
+        spec = {"x": ((B, self.C, self.T, self.H, self.W), bf), "t": (t, bf), "ctx": ((B, self.Lt, p.text_dim), bf),
                 "sig": ((B, 2), torch.float32)}
         if self.Li:
             spec["clip"] = ((B, self.Li, p.clip_dim), bf)

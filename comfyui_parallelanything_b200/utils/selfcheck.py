@@ -673,6 +673,193 @@ def wan_i2v_executor_tiny_fp8():
     return _wan_i2v_case(True)
 
 
+def _frames_ref(v: torch.Tensor, rows: int, off: int, B: int, L: int) -> torch.Tensor:
+    """[G, D] per-group vectors -> [B, L, D] per-row vectors: row r of sample b reads group (b*L + r + off) // rows."""
+    idx = (torch.arange(B * L, device=v.device) + off) // rows
+    return v.float()[idx].view(B, L, -1)
+
+
+@check
+def layernorm_modulate_per_frame():
+    """LayerNorm + modulate with one scale / shift row per video frame (``mod_rows``): 130 rows per frame (not a
+    multiple of 128 or of the 8 warps per block), D = 3072, a [B*T, 6, D] table like the WAN modulation table, and a
+    token slice that starts mid-frame (``mod_row_off``, sequence parallelism)."""
+    B, T, HW, D = 2, 3, 130, 3072
+    L = T * HW
+    x = _rand(B, L, D)
+    table = _rand(B * T, 6, D, scale=0.3, seed=3)
+    sc, sh = table[:, 1], table[:, 0]
+    out = ops.layernorm_modulate(x, scale=sc, shift=sh, mod_rows=HW)
+    ln = F.layer_norm(x.float(), (D,), eps=1e-6)
+    want = ln * (1 + _frames_ref(sc, HW, 0, B, L)) + _frames_ref(sh, HW, 0, B, L)
+    r = _cmp("layernorm_modulate_per_frame", out, want, 0.01)
+    # batch 1, rows [off, off + Ll) of the clip: the slice's first row is in the middle of frame 0
+    off, Ll = 57, 200
+    xs = x[:1, off:off + Ll]
+    o2 = ops.layernorm_modulate(xs, scale=sc[:T], shift=sh[:T], mod_rows=HW, mod_row_off=off)
+    w2 = (F.layer_norm(xs.float(), (D,), eps=1e-6) * (1 + _frames_ref(sc[:T], HW, off, 1, Ll))
+          + _frames_ref(sh[:T], HW, off, 1, Ll))
+    r2 = _cmp("slice", o2, w2, 0.01)
+    # per sample (no mod_rows) must stay what it was: same bits as a [B, D] view
+    o3 = ops.layernorm_modulate(x, scale=sc[::T], shift=sh[::T])
+    w3 = ln * (1 + sc[::T].float()[:, None]) + sh[::T].float()[:, None]
+    r3 = _cmp("per_sample", o3, w3, 0.01)
+    r["slice_mean_rel"], r["per_sample_mean_rel"] = r2["mean_rel"], r3["mean_rel"]
+    r["ok"] = r["ok"] and r2["ok"] and r3["ok"]
+    return r
+
+
+@check
+def gemm_gate_res_per_frame():
+    """Gated-residual epilogue with one gate row per video frame (``gate_rows``), frame boundaries inside 128-row
+    tiles (80 and 130 rows per frame): bf16 one-CTA, CTA pair (force_bn=512), MXFP8 one-CTA and CTA-pair kernels (the
+    pair kernels need >= 256 rows per sample: 320 and 260 here, the last tile ragged), and a token slice that starts
+    mid-frame (``gate_row_off``)."""
+    res = {"name": "gemm_gate_res_per_frame", "ok": True}
+    worst = 0.0
+    for HW, T in ((80, 4), (130, 2)):
+        B, K, N = 2, 256, 512
+        L = T * HW
+        a, w, b = _rand(B, L, K, seed=1), _rand(N, K, scale=0.05, seed=2), _rand(N, seed=3)
+        gates = _rand(B * T, 6, N, seed=4)[:, 2]                       # strided [B*T, N] view of a modulation table
+        resid = _rand(B, L, N, seed=5)
+        want = resid.float() + _frames_ref(gates, HW, 0, B, L) * _gemm_ref(a, w, b)
+        cases = [("bf16", None), ("bf16_pair", 512)]
+        for tag, bn in cases:
+            out = resid.clone()
+            kw = dict(force_bn=bn) if bn else {}
+            ops.gemm(a, w, "gate_res", out=out, bias=b, residual=out, gate=gates, gate_rows=HW, **kw)
+            r = _cmp(tag, out, want, 0.012)
+            worst = max(worst, r["mean_rel"])
+            res[f"{tag}_hw{HW}_ok"] = r["ok"]
+            res["ok"] = res["ok"] and r["ok"]
+        aq, sfa = ops.quantize_mxfp8(a)
+        wq, sfb = ops.quantize_mxfp8(w, 224)
+        exact = (resid.float() + _frames_ref(gates, HW, 0, B, L)
+                 * (ops.dequantize_mxfp8(aq, sfa) @ ops.dequantize_mxfp8(wq, sfb, 224)[0].t() + b.float()))
+        for pair in (0, 1):
+            out = resid.clone()
+            ops.gemm_fp8(aq, sfa, wq, sfb, "gate_res", 224, out=out, bias=b, residual=out, gate=gates, gate_rows=HW,
+                         pair=pair)
+            r = _cmp(f"mxfp8_pair{pair}", out, exact, 0.012)
+            worst = max(worst, r["mean_rel"])
+            res[f"mxfp8_pair{pair}_hw{HW}_ok"] = r["ok"]
+            res["ok"] = res["ok"] and r["ok"]
+    # batch-1 token slice starting mid-frame, as a sequence-parallel rank sees it
+    HW, T, off, Ll, K, N = 80, 3, 120, 120, 256, 512
+    a, w, b = _rand(1, Ll, K, seed=6), _rand(N, K, scale=0.05, seed=7), _rand(N, seed=8)
+    gates, resid = _rand(T, N, seed=9), _rand(1, Ll, N, seed=10)
+    out = resid.clone()
+    ops.gemm(a, w, "gate_res", out=out, bias=b, residual=out, gate=gates, gate_rows=HW, gate_row_off=off)
+    r = _cmp("slice", out, resid.float() + _frames_ref(gates, HW, off, 1, Ll) * _gemm_ref(a, w, b), 0.012)
+    res["slice_ok"] = r["ok"]
+    res["ok"] = res["ok"] and r["ok"]
+    res["mean_rel"] = max(worst, r["mean_rel"])
+    return res
+
+
+@check
+def scatter_patch_embed_per_frame_t():
+    """Fused scatter kernel of a 48-channel WAN2.2 TI2V latent (three 64-column K blocks, K = 192) with one timestep
+    per latent frame: ``n_t`` = B*T sinusoids."""
+    from ..models import flux
+    C_ = ops.require()
+    m = flux.Flux.__new__(flux.Flux)
+    m.patch_size = 2
+    B, Cc, T, Hl, Wl, N = 2, 48, 3, 16, 20, 768
+    x = _rand(B, Cc, T * Hl, Wl)                      # [B, C, T, H, W] as the kernel reads it: a T*H tall image
+    w, b = _rand(N, 4 * Cc, scale=0.1), _rand(N)
+    t = torch.tensor([[0.0, 700.0, 700.0], [0.0, 450.0, 450.0]], device=_dev(), dtype=torch.bfloat16)
+    Li = T * (Hl // 2) * (Wl // 2)
+    X = torch.zeros(B, Li, N, dtype=torch.bfloat16, device=_dev())
+    t_emb = torch.zeros(B * T, 256, dtype=torch.bfloat16, device=_dev())
+    xc = torch.zeros_like(x)
+    C_.scatter_patch_embed(w, b, x.data_ptr(), t.data_ptr(), 0, t_emb, None, xc, X, Cc, T * Hl, Wl, 1.0, B * T)
+    r = _cmp("scatter_patch_embed_per_frame_t", X, _gemm_ref(flux.Flux.patchify(m, x), w, b), 0.012)
+    r2 = _cmp("temb", t_emb, flux.timestep_embedding(t.reshape(-1), 256, time_factor=1.0), 0.01)
+    r["temb_mean_rel"] = r2["mean_rel"]
+    r["ok"] = r["ok"] and r2["ok"] and bool(torch.equal(xc, x))
+    return r
+
+
+@check
+def euler_unpatch_c48():
+    """Head GEMM with the Euler / unpatchify epilogue for 48 latent channels (N = 192, WAN2.2 TI2V)."""
+    B, C, Hl, Wl, hid = 2, 48, 32, 40, 256
+    L = (Hl // 2) * (Wl // 2)
+    h, w, b = _rand(B, L, hid), _rand(C * 4, hid, scale=0.06), _rand(C * 4)
+    x = _rand(B, C, Hl, Wl)
+    sig = torch.tensor([[1.0, 0.9], [0.5, 0.25]], device=_dev())
+    xo = torch.zeros(B, C, Hl, Wl, dtype=torch.bfloat16, device=_dev())
+    ops.gemm(h, w, "euler_unpatch", bias=b, x_in=x, x_out=xo, sigmas=sig, C=C, Hl=Hl, Wl=Wl)
+    v = _gemm_ref(h, w, b).view(B, Hl // 2, Wl // 2, C, 2, 2).permute(0, 3, 1, 4, 2, 5).reshape(B, C, Hl, Wl)
+    want = x.float() + (sig[:, 1] - sig[:, 0])[:, None, None, None] * v
+    return _cmp("euler_unpatch_c48", xo, want, 0.012)
+
+
+def _per_frame_cmp(name: str, got: torch.Tensor, want: torch.Tensor, tol: float) -> dict:
+    """``_cmp`` of the whole clip and of every latent frame on its own (dim 2): a per-sample modulation lookup is wrong
+    on some frames only, which the whole-clip mean could hide."""
+    r = _cmp(name, got, want, tol)
+    frames = [_cmp(f"{name}_f{f}", got[:, :, f], want[:, :, f], tol) for f in range(got.shape[2])]
+    r["frame_mean_rel"] = [round(fr["mean_rel"], 5) for fr in frames]
+    r["ok"] = r["ok"] and all(fr["ok"] for fr in frames)
+    return r
+
+
+def _wan_ti2v_case(fp8: bool) -> dict:
+    """Tiny WAN2.2 TI2V executor (48 channels in and out, per-frame timesteps, 80 tokens per frame) against the fp32
+    oracle: ``forward``, then ``denoise_step`` eager, captured and replayed twice with the latent AND the per-frame
+    timesteps changed in place between the calls (the graph must read both)."""
+    import dataclasses
+    from ..exec.wan_exec import WanExecutor
+    from ..models import wan
+    p = dataclasses.replace(wan.wan_tiny_params(), in_dim=48, out_dim=48)
+    torch.manual_seed(5)
+    m = wan.WanModel(p).to(device=_dev(), dtype=torch.bfloat16).eval()
+    ex = WanExecutor(m, _dev(), cuda_graphs=True, fp8=fp8)
+    oracle = wan.WanModel(p).to(device=_dev(), dtype=torch.float32).eval()
+    oracle.load_state_dict({k: v.float() for k, v in m.state_dict().items()})
+    inp = wan.ti2v_inputs(p, 2, frames=9, height=256, width=320, device=_dev(), dtype=torch.bfloat16, seed=6)
+    inp["timesteps"][:, 1:] = torch.tensor([[700.0], [450.0]], device=_dev(), dtype=torch.bfloat16)
+    tol = 0.05 if fp8 else 0.03
+    name = "wan_ti2v_executor_tiny" + ("_fp8" if fp8 else "")
+    with torch.no_grad():
+        got = ex(**inp)
+        want = oracle(**{k: v.float() for k, v in inp.items()})
+    r = _per_frame_cmp(name, got, want, tol)
+    r["ok"] = r["ok"] and tuple(got.shape) == tuple(inp["x"].shape)
+    sig = torch.tensor([[1.0, 0.8], [0.6, 0.5]], device=_dev())
+    x, t, c = ex._prep(inp["x"], inp["timesteps"], inp["context"])
+    worst = 0.0
+    for it in range(4):                                 # eager, capture, replay, replay
+        x.mul_(0.9)
+        t[:, 1:].sub_(100.0)                            # new per-frame timesteps, same buffer
+        t[1, 0] = 50.0 * it                             # the image frame's timestep changes too
+        nxt = ex.denoise_step(x, t, c, sig).clone()
+        with torch.no_grad():
+            v = oracle(x.float(), t.float(), context=c.float())
+        want2 = x.float() + (sig[:, 1] - sig[:, 0])[:, None, None, None, None] * v
+        r2 = _per_frame_cmp(name + "_euler", nxt, want2, tol)
+        worst = max(worst, r2["mean_rel"])
+        r["ok"] = r["ok"] and r2["ok"]
+    r["euler_worst_mean_rel"] = worst
+    r["graphs"] = sorted(ex._graphs.state(k) for k in list(ex._graphs._graphs))
+    r["ok"] = r["ok"] and "graph" in r["graphs"]
+    r["launches"] = ex.launches_per_step
+    return r
+
+
+@check
+def wan_ti2v_executor_tiny():
+    return _wan_ti2v_case(False)
+
+
+@check
+def wan_ti2v_executor_tiny_fp8():
+    return _wan_ti2v_case(True)
+
+
 @check
 def attention_two_kv():
     """Two-source attention ``softmax(q K1^T) V1 + softmax(q K2^T) V2`` (WAN2.1 text + CLIP image cross-attention)

@@ -62,6 +62,16 @@ static void parse_epilogue(const py::kwargs& kw, pa::GemmParams& p, bool check_s
     TORCH_CHECK(g.stride(-1) == 1, "gate must be contiguous in its last dim");
     p.gate = reinterpret_cast<const __nv_bfloat16*>(g.data_ptr());
     p.gate_bstride = g.dim() >= 2 ? g.stride(0) : 0;
+    if (has(kw, "gate_rows")) {
+      // one gate vector per group of gate_rows rows (video frames): the last row's group must be a row of `gate`
+      p.gate_rows = kw["gate_rows"].cast<int>();
+      p.gate_row_off = has(kw, "gate_row_off") ? kw["gate_row_off"].cast<int>() : 0;
+      TORCH_CHECK(p.mode == pa::EPI_GATE_RES, "gate_rows needs the gate_res epilogue");
+      TORCH_CHECK(p.gate_rows > 0 && p.gate_row_off >= 0, "gate_rows must be > 0, gate_row_off >= 0");
+      TORCH_CHECK(g.dim() == 2, "gate_rows needs a 2-D [groups, N] gate view");
+      TORCH_CHECK(((long long)p.batch * p.rows - 1 + p.gate_row_off) / p.gate_rows < g.size(0),
+                  "gate_rows: the last row's group is outside the gate's ", g.size(0), " rows");
+    }
   }
   if (has(kw, "out8")) {
     // fused MXFP8 output: e4m3 bytes [batch, rows8, ld8] contiguous + scale chunks; written at column out8_col_off
@@ -221,8 +231,11 @@ static void conv(Tensor x, Tensor w, int taps, int stride, int mode, py::kwargs 
         "conv_bf16");
 }
 
+// scale / shift: [B, D] views (one vector per sample), or with mod_rows > 0 [G, D] views with one vector per group of
+// mod_rows rows: row r of sample b reads vector (b * rows + r + mod_row_off) / mod_rows (video frames)
 static void layernorm_modulate(Tensor x, Tensor out, c10::optional<Tensor> scale, c10::optional<Tensor> shift,
-                               c10::optional<Tensor> gamma, c10::optional<Tensor> beta, double eps) {
+                               c10::optional<Tensor> gamma, c10::optional<Tensor> beta, double eps, int mod_rows,
+                               int mod_row_off) {
   c10::cuda::CUDAGuard guard(x.device());
   int b, rows, ob, orows;
   long long ldx, xbs, ldo, obs;
@@ -233,9 +246,18 @@ static void layernorm_modulate(Tensor x, Tensor out, c10::optional<Tensor> scale
   const void *sc = nullptr, *sh = nullptr;
   if (scale) { sc = scale->data_ptr(); mod_bs = scale->dim() >= 2 ? scale->stride(0) : 0; TORCH_CHECK(scale->stride(-1) == 1); }
   if (shift) { sh = shift->data_ptr(); long long s2 = shift->dim() >= 2 ? shift->stride(0) : 0; TORCH_CHECK(!scale || s2 == mod_bs, "scale/shift batch strides differ"); mod_bs = s2; }
+  if (mod_rows > 0) {
+    TORCH_CHECK(mod_row_off >= 0, "mod_row_off must be >= 0");
+    const long long last = ((long long)b * rows - 1 + mod_row_off) / mod_rows;
+    for (const c10::optional<Tensor>* m : {&scale, &shift})
+      if (*m) TORCH_CHECK((*m)->dim() == 2 && last < (*m)->size(0), "mod_rows: the last row's group ", last,
+                          " is outside the [", (*m)->size(0), ", D] scale / shift view");
+  } else {
+    TORCH_CHECK(mod_rows == 0 && mod_row_off == 0, "mod_row_off needs mod_rows > 0");      // one vector per sample
+  }
   check(pa::layernorm_modulate(x.data_ptr(), ldx, xbs, out.data_ptr(), ldo, obs, sc, sh, mod_bs,
                                gamma ? gamma->data_ptr() : nullptr, beta ? beta->data_ptr() : nullptr, b, rows,
-                               (int)x.size(-1), (float)eps, cur_stream()),
+                               (int)x.size(-1), (float)eps, mod_rows, mod_row_off, cur_stream()),
         "layernorm_modulate");
 }
 
@@ -300,9 +322,10 @@ static void patchify(uintptr_t x_ptr, Tensor out, int B, int C, int H, int W, in
 
 // Fused scatter: peer latent shard -> patchify -> img_in GEMM (+ bias) -> X[:, Lt:], plus the
 // sinusoidal embeddings of the shard's timesteps / guidance values (read from the peer).
+// n_t: timesteps to embed into t_emb (0: one per sample; samples x frames with per-frame timesteps)
 static void scatter_patch_embed(Tensor W, Tensor bias, uintptr_t x_src, uintptr_t t_src, uintptr_t g_src, Tensor t_emb,
                                 c10::optional<Tensor> g_emb, c10::optional<Tensor> x_copy, Tensor out, int C, int Hl,
-                                int Wl, double time_factor) {
+                                int Wl, double time_factor, int n_t) {
   c10::cuda::CUDAGuard guard(out.device());
   // up to 16 channels the patch is one 64-column K block; wider latents use the plain [N, 4*C] patch reshape
   const int64_t K = C <= 16 ? 64 : 4 * (int64_t)C;
@@ -321,6 +344,10 @@ static void scatter_patch_embed(Tensor W, Tensor bias, uintptr_t x_src, uintptr_
   p.out = reinterpret_cast<__nv_bfloat16*>(out.data_ptr());
   p.bias = reinterpret_cast<const __nv_bfloat16*>(bias.data_ptr());
   p.n = ob; p.C = C; p.Hl = Hl; p.Wl = Wl; p.N = (int)W.size(0); p.Li = orows;
+  p.n_t = n_t > 0 ? n_t : ob;
+  TORCH_CHECK(p.n_t % ob == 0 && (p.g_src == nullptr || p.n_t == ob), "n_t must be a multiple of the ", ob,
+              " samples (and equal to it with guidance)");
+  TORCH_CHECK(t_emb.numel() >= (int64_t)p.n_t * 256, "t_emb must hold n_t = ", p.n_t, " rows of 256");
   TORCH_CHECK(p.Li == (Hl / 2) * (Wl / 2), "out rows must equal the number of 2x2 patches");
   p.time_factor = (float)time_factor;
   check(pa::scatter_patch_embed(W.data_ptr(), W.stride(0), p, cur_stream()), "scatter_patch_embed");
@@ -599,10 +626,12 @@ PYBIND11_MODULE(_C, m) {
   m.def("layernorm_modulate_fp8", &layernorm_modulate_fp8);
   m.def("layernorm_modulate", &layernorm_modulate, py::arg("x"), py::arg("out"), py::arg("scale") = py::none(),
         py::arg("shift") = py::none(), py::arg("gamma") = py::none(), py::arg("beta") = py::none(),
-        py::arg("eps") = 1e-6);
+        py::arg("eps") = 1e-6, py::arg("mod_rows") = 0, py::arg("mod_row_off") = 0);
   m.def("timestep_embedding", &timestep_embedding);
   m.def("patchify", &patchify);
-  m.def("scatter_patch_embed", &scatter_patch_embed);
+  m.def("scatter_patch_embed", &scatter_patch_embed, py::arg("W"), py::arg("bias"), py::arg("x_src"), py::arg("t_src"),
+        py::arg("g_src"), py::arg("t_emb"), py::arg("g_emb"), py::arg("x_copy"), py::arg("out"), py::arg("C"),
+        py::arg("Hl"), py::arg("Wl"), py::arg("time_factor"), py::arg("n_t") = 0);
   m.def("scatter_conv_in", &scatter_conv_in);
   m.def("nchw_to_nhwc_pad", &nchw_to_nhwc_pad);
   m.def("upsample2x", &upsample2x);

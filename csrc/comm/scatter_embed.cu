@@ -143,9 +143,10 @@ scatter_patch_embed_kernel(const __grid_constant__ CUtensorMap tmW, const __grid
     }
     __syncwarp();
   } else if (warp == 3) {
-    // timestep / guidance sinusoidal embeddings of the shard (values read from the lead GPU)
+    // timestep / guidance sinusoidal embeddings of the shard (values read from the lead GPU): n_t timesteps (n, or
+    // one per video frame), guidance values only with n_t == n
     if (blockIdx.x == 0) {
-      for (int i = lane; i < p.n * 128; i += 32) {
+      for (int i = lane; i < p.n_t * 128; i += 32) {
         const int s = i >> 7, f = i & 127;
         const float freq = __expf(-9.210340371976184f * static_cast<float>(f) * (1.0f / 128.0f));   // ln(1e4)
         float sn, cs;
@@ -285,6 +286,7 @@ static int launch_scatter_patch_embed(const CUtensorMap& tw, const CUtensorMap& 
 int scatter_patch_embed(const void* W, long long ldw, const ScatterEmbedParams& p, cudaStream_t st) {
   using namespace se;
   if (p.C < 1 || p.C > MAX_KB * 16 || (p.C > 16 && (p.C & 1)) || p.N % 32 || (p.Wl & 1)) return -1;
+  if (p.n_t < p.n || (p.g_src != nullptr && p.n_t != p.n)) return -3;
   const int nkb = p.C <= 16 ? 1 : (p.C + 15) / 16;
   CUtensorMap tw;
   uint64_t dims[2] = {nkb == 1 ? 64u : (uint64_t)(4 * p.C), (uint64_t)p.N};

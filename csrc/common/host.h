@@ -43,7 +43,8 @@ int layernorm_modulate_fp8(const void* x, long long ldx, long long x_bs, void* q
                            const void* shift, long long mod_bs, int batch, int rows, int D, float eps, cudaStream_t st);
 int layernorm_modulate(const void* x, long long ldx, long long x_bstride, void* out, long long ldo,
                        long long o_bstride, const void* scale, const void* shift, long long mod_bstride,
-                       const void* gamma, const void* beta, int batch, int rows, int D, float eps, cudaStream_t st);
+                       const void* gamma, const void* beta, int batch, int rows, int D, float eps, int mod_rows,
+                       int mod_row_off, cudaStream_t st);   // scale/shift row = b, or (b*rows + r + mod_row_off) / mod_rows
 
 // sinusoidal embedding: out[b, :] = [cos(t*f_i) | sin(t*f_i)], f_i = exp(-ln(max_period) * i / half)
 int timestep_embedding(const void* t, void* out, long long ldo, int B, int dim, float time_factor,

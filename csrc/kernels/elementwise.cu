@@ -43,6 +43,9 @@ __device__ __forceinline__ float warp_sum(float v) {
 
 // ------------------------------------------------------------------ LayerNorm + modulate
 // One warp per row; the row (D <= 8192) is held in registers between the statistics and the write pass.
+// scale / shift row of (sample b, row r): b with mod_rows = 0 (one vector per sample), else
+// (b * rows + r + mod_row_off) / mod_rows: mod_rows = tokens per frame gives one vector per video frame (WAN2.2 TI2V
+// per-frame timesteps), and mod_row_off = the global token index of row 0 keeps that right for a token slice.
 template <int MAX_VEC>   // MAX_VEC uint4 per lane: D <= 32*8*MAX_VEC
 __global__ void __launch_bounds__(256) ln_mod_kernel(const __nv_bfloat16* __restrict__ x, long long ldx,
                                                      long long x_bs, __nv_bfloat16* __restrict__ out, long long ldo,
@@ -50,11 +53,12 @@ __global__ void __launch_bounds__(256) ln_mod_kernel(const __nv_bfloat16* __rest
                                                      const __nv_bfloat16* __restrict__ shift, long long mod_bs,
                                                      const __nv_bfloat16* __restrict__ gamma,
                                                      const __nv_bfloat16* __restrict__ beta, int batch, int rows, int D,
-                                                     float eps) {
+                                                     float eps, int mod_rows, int mod_row_off) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= batch * rows) return;
   const int b = warp / rows, r = warp - b * rows;
+  const int mb = mod_rows ? (warp + mod_row_off) / mod_rows : b;     // modulation row: the sample, or a frame of it
   const uint4* xr = reinterpret_cast<const uint4*>(x + b * x_bs + static_cast<long long>(r) * ldx);
   const int nvec = D >> 3;
   uint4 buf[MAX_VEC];
@@ -76,8 +80,8 @@ __global__ void __launch_bounds__(256) ln_mod_kernel(const __nv_bfloat16* __rest
   const float var = fmaxf(ss / D - mean * mean, 0.f);
   const float rstd = rsqrtf(var + eps);
   uint4* orow = reinterpret_cast<uint4*>(out + b * o_bs + static_cast<long long>(r) * ldo);
-  const uint4* sc = scale ? reinterpret_cast<const uint4*>(scale + b * mod_bs) : nullptr;
-  const uint4* sh = shift ? reinterpret_cast<const uint4*>(shift + b * mod_bs) : nullptr;
+  const uint4* sc = scale ? reinterpret_cast<const uint4*>(scale + mb * mod_bs) : nullptr;
+  const uint4* sh = shift ? reinterpret_cast<const uint4*>(shift + mb * mod_bs) : nullptr;
   const uint4* ga = gamma ? reinterpret_cast<const uint4*>(gamma) : nullptr;
   const uint4* be = beta ? reinterpret_cast<const uint4*>(beta) : nullptr;
 #pragma unroll
@@ -131,7 +135,8 @@ __global__ void __launch_bounds__(256) ln_mod_fast_kernel(const __nv_bfloat16* _
                                                           const __nv_bfloat16* __restrict__ shift, long long mod_bs,
                                                           const __nv_bfloat16* __restrict__ gamma,
                                                           const __nv_bfloat16* __restrict__ beta, int batch, int rows,
-                                                          int D, float eps, uint8_t* __restrict__ sf8 = nullptr) {
+                                                          int D, float eps, int mod_rows, int mod_row_off,
+                                                          uint8_t* __restrict__ sf8 = nullptr) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= batch * rows) return;
@@ -163,8 +168,10 @@ __global__ void __launch_bounds__(256) ln_mod_fast_kernel(const __nv_bfloat16* _
   const float rstd = rsqrtf(fmaxf(ss / D - mean * mean, 0.f) + eps);
   const float nmr = -mean * rstd;
   uint4* orow = reinterpret_cast<uint4*>(out + b * o_bs + static_cast<long long>(r) * ldo);
-  const uint4* sc = reinterpret_cast<const uint4*>(scale + ((FLAGS & 4) ? b * mod_bs : 0));
-  const uint4* sh = reinterpret_cast<const uint4*>(shift + ((FLAGS & 8) ? b * mod_bs : 0));
+  const int mb = !(FLAGS & 12) ? 0 : (mod_rows ? static_cast<int>(static_cast<unsigned>(warp + mod_row_off) /
+                                                                  static_cast<unsigned>(mod_rows)) : b);   // sample or frame
+  const uint4* sc = reinterpret_cast<const uint4*>(scale + ((FLAGS & 4) ? mb * mod_bs : 0));
+  const uint4* sh = reinterpret_cast<const uint4*>(shift + ((FLAGS & 8) ? mb * mod_bs : 0));
   const uint4* ga = reinterpret_cast<const uint4*>(gamma);
   const uint4* be = reinterpret_cast<const uint4*>(beta);
 #pragma unroll
@@ -245,6 +252,7 @@ __global__ void __launch_bounds__(256) ln_mod_fast_kernel(const __nv_bfloat16* _
 // sf8 scale chunks (zero-initialised by the caller).
 int layernorm_modulate_fp8(const void* x, long long ldx, long long x_bs, void* q8, void* sf8, const void* scale,
                            const void* shift, long long mod_bs, int batch, int rows, int D, float eps, cudaStream_t st) {
+  const int mod_rows = 0, mod_row_off = 0;            // one vector per sample
   if (D % 256 || ldx % 8 || x_bs % 8 || mod_bs % 8 || !scale || !shift) return -1;   // whole warps per vector step
   const long long warps = static_cast<long long>(batch) * rows;
   const int threads = 256;
@@ -255,11 +263,11 @@ int layernorm_modulate_fp8(const void* x, long long ldx, long long x_bs, void* q
   auto O = static_cast<__nv_bfloat16*>(q8);
   auto S8 = static_cast<uint8_t*>(sf8);
   if (D <= 32 * 8 * 4)
-    ln_mod_fast_kernel<4, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, S8);
+    ln_mod_fast_kernel<4, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, mod_rows, mod_row_off, S8);
   else if (D <= 32 * 8 * 12)
-    ln_mod_fast_kernel<12, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, S8);
+    ln_mod_fast_kernel<12, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, mod_rows, mod_row_off, S8);
   else if (D <= 32 * 8 * 20)
-    ln_mod_fast_kernel<20, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, S8);
+    ln_mod_fast_kernel<20, 12, true><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, 0, 0, SC, SH, mod_bs, nullptr, nullptr, batch, rows, D, eps, mod_rows, mod_row_off, S8);
   else
     return -2;
   return (int)cudaGetLastError();
@@ -269,13 +277,13 @@ template <int FLAGS>
 static bool launch_ln_fast(int blocks, int threads, cudaStream_t st, const __nv_bfloat16* X, long long ldx, long long x_bs,
                            __nv_bfloat16* O, long long ldo, long long o_bs, const __nv_bfloat16* SC,
                            const __nv_bfloat16* SH, long long mod_bs, const __nv_bfloat16* G, const __nv_bfloat16* Bt,
-                           int batch, int rows, int D, float eps) {
+                           int batch, int rows, int D, float eps, int mod_rows, int mod_row_off) {
   if (D <= 32 * 8 * 4)
-    ln_mod_fast_kernel<4, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_fast_kernel<4, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else if (D <= 32 * 8 * 12)
-    ln_mod_fast_kernel<12, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_fast_kernel<12, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else if (D <= 32 * 8 * 20)
-    ln_mod_fast_kernel<20, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_fast_kernel<20, FLAGS><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else
     return false;
   return true;
@@ -283,8 +291,9 @@ static bool launch_ln_fast(int blocks, int threads, cudaStream_t st, const __nv_
 
 int layernorm_modulate(const void* x, long long ldx, long long x_bs, void* out, long long ldo, long long o_bs,
                        const void* scale, const void* shift, long long mod_bs, const void* gamma, const void* beta,
-                       int batch, int rows, int D, float eps, cudaStream_t st) {
+                       int batch, int rows, int D, float eps, int mod_rows, int mod_row_off, cudaStream_t st) {
   if (D % 8 || ldx % 8 || ldo % 8 || x_bs % 8 || o_bs % 8 || mod_bs % 8) return -1;
+  if (mod_rows < 0 || mod_row_off < 0 || (mod_rows == 0 && mod_row_off != 0)) return -3;
   const long long warps = static_cast<long long>(batch) * rows;
   const int threads = 256;
   const int blocks = static_cast<int>((warps * 32 + threads - 1) / threads);
@@ -297,16 +306,16 @@ int layernorm_modulate(const void* x, long long ldx, long long x_bs, void* out, 
   const int flags = (G ? 1 : 0) | (Bt ? 2 : 0) | (SC ? 4 : 0) | (SH ? 8 : 0);
 #define PA_LN_FAST(F)                                                                                              \
   if (flags == F && launch_ln_fast<F>(blocks, threads, st, X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, \
-                                      D, eps))                                                                    \
+                                      D, eps, mod_rows, mod_row_off))                                            \
     return (int)cudaGetLastError();
   PA_LN_FAST(12) PA_LN_FAST(4) PA_LN_FAST(3) PA_LN_FAST(0)
 #undef PA_LN_FAST
   if (D <= 32 * 8 * 4)
-    ln_mod_kernel<4><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_kernel<4><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else if (D <= 32 * 8 * 12)
-    ln_mod_kernel<12><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_kernel<12><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else if (D <= 32 * 8 * 20)
-    ln_mod_kernel<20><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps);
+    ln_mod_kernel<20><<<blocks, threads, 0, st>>>(X, ldx, x_bs, O, ldo, o_bs, SC, SH, mod_bs, G, Bt, batch, rows, D, eps, mod_rows, mod_row_off);
   else
     return -2;
   return (int)cudaGetLastError();

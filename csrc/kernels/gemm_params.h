@@ -32,6 +32,9 @@ struct GemmParams {
   long long ldr, res_bstride;
   const __nv_bfloat16* gate;        // [batch, N] with stride gate_bstride
   long long gate_bstride;
+  // EPI_GATE_RES with gate_rows > 0: the gate row of (sample b, row r) is (b * rows + r + gate_row_off) / gate_rows
+  // instead of b (one gate vector per video frame; gate_row_off = global token index of row 0 of a token slice)
+  int gate_rows, gate_row_off;
   // Fused MXFP8 output (the NEXT GEMM's A operand, written by this epilogue instead of bf16 + a quantise kernel):
   // EPI_BIAS_GELU: every column; EPI_QKV_ROPE: the GELU'd MLP columns.  e4m3 bytes row-major [batch, rows8, ld8]
   // plus UE8M0 scale chunks in the layout of gemm_mxfp8.cu (128-row x 128-column chunks of 512 bytes).

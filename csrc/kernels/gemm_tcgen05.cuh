@@ -517,7 +517,9 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tadd
     __nv_bfloat16* orow = p.out + b * p.out_bstride + static_cast<long long>(row) * p.ldc;
     const __nv_bfloat16* rrow =
         p.residual ? p.residual + b * p.res_bstride + static_cast<long long>(row) * p.ldr : nullptr;
-    const __nv_bfloat16* grow = p.gate ? p.gate + b * p.gate_bstride : nullptr;
+    // per-frame gates: the group of THIS thread's row (a 128-row tile spans several frames)
+    const int gb = p.gate_rows ? (b * p.rows + row + p.gate_row_off) / p.gate_rows : b;
+    const __nv_bfloat16* grow = p.gate ? p.gate + gb * p.gate_bstride : nullptr;
 #pragma unroll 1
     for (int c = 0; c < BN / 32; ++c) {
       const int n = n0 + c * 32;

@@ -4,9 +4,11 @@
 bench.py (one step = forward + Euler update; device-timed, max over ranks; e2e with per-step H2D/D2H).  ``--i2v`` runs
 WAN2.2-I2V-A14B instead: the same layer stack on a 36-channel input ([noise 16 | mask 4 | image latent 16]).  ``--clip``
 runs WAN2.1-I2V-14B (that input plus 257 CLIP image tokens and an image cross-attention in every block), ``--flf2v``
-WAN2.1-FLF2V-14B (514 CLIP tokens of the first and last frame).
+WAN2.1-FLF2V-14B (514 CLIP tokens of the first and last frame).  ``--ti2v`` runs WAN2.2-TI2V-5B at its own size:
+1280 x 704 x 121 frames, a 48-channel [31, 44, 80] latent of the WAN2.2 VAE (27 280 tokens per sample), with one
+timestep per latent frame (image-to-video mode; ``--sample-timesteps``: one per sample, text-to-video mode).
 
-    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8] [--i2v | --clip | --flf2v]
+    python tools/bench_wan.py --gpus 1 [--impl reference] [--batch 8] [--i2v | --clip | --flf2v | --ti2v]
     python -m torch.distributed.run --nproc-per-node 8 ... tools/bench_wan.py --gpus 8
 """
 from __future__ import annotations
@@ -23,10 +25,18 @@ MODEL_NAME = "WAN2.2-A14B video DiT 720p x 16 frames"
 I2V_MODEL_NAME = "WAN2.2-I2V-A14B video DiT 720p x 16 frames"
 CLIP_MODEL_NAME = "WAN2.1-I2V-14B video DiT 720p x 16 frames (257 CLIP tokens)"
 FLF2V_MODEL_NAME = "WAN2.1-FLF2V-14B video DiT 720p x 16 frames (514 CLIP tokens)"
+TI2V_MODEL_NAME = "WAN2.2-TI2V-5B video DiT 1280x704 x 121 frames"
 
 
 def model_name(a) -> str:
+    if a.ti2v:
+        return TI2V_MODEL_NAME + (" (one timestep per sample)" if a.sample_timesteps else " (per-frame timesteps)")
     return FLF2V_MODEL_NAME if a.flf2v else CLIP_MODEL_NAME if a.clip else I2V_MODEL_NAME if a.i2v else MODEL_NAME
+
+
+def geometry(a) -> tuple:
+    """(pixel frames, height, width) of the workload."""
+    return (121, 704, 1280) if a.ti2v else (16, 720, 1280)
 
 
 def host_inputs(B, cap_len, a):
@@ -36,9 +46,14 @@ def host_inputs(B, cap_len, a):
         cfg, make = (wan.wan21_flf2v_14b_params() if a.flf2v else wan.wan21_i2v_14b_params()), wan.clip_inputs
     elif a.i2v:
         cfg, make = wan.wan22_i2v_a14b_params(), wan.i2v_inputs
+    elif a.ti2v:
+        cfg, make = wan.wan22_ti2v_5b_params(), wan.ti2v_inputs
     else:
         cfg, make = wan.wan22_a14b_params(), wan.example_inputs
-    inp = make(cfg, B, frames=16, height=720, width=1280, device="cpu", dtype=torch.bfloat16)
+    frames, height, width = geometry(a)
+    inp = make(cfg, B, frames=frames, height=height, width=width, device="cpu", dtype=torch.bfloat16)
+    if a.ti2v and a.sample_timesteps:
+        inp["timesteps"] = inp["timesteps"][:, 1].contiguous()
     inp["sig"] = torch.tensor([[1.0, 0.875]] * B, dtype=torch.float32)
     return cfg, {k: v.pin_memory() for k, v in inp.items()}
 
@@ -74,6 +89,10 @@ def main() -> int:
     ap.add_argument("--i2v", action="store_true", help="WAN2.2-I2V-A14B (36-channel input) instead of T2V")
     ap.add_argument("--clip", action="store_true", help="WAN2.1-I2V-14B (36-channel input + CLIP image cross-attention)")
     ap.add_argument("--flf2v", action="store_true", help="WAN2.1-FLF2V-14B (as --clip, 514 CLIP tokens)")
+    ap.add_argument("--ti2v", action="store_true",
+                    help="WAN2.2-TI2V-5B (48 channels in and out) at 1280x704 x 121 frames, per-frame timesteps")
+    ap.add_argument("--sample-timesteps", action="store_true",
+                    help="with --ti2v: one timestep per sample (text-to-video mode) instead of one per latent frame")
     a = ap.parse_args()
     if a.api == "nodes":
         return run_nodes(a)
@@ -97,7 +116,8 @@ def main() -> int:
     from comfyui_parallelanything_b200.models import wan
     cfg, host = host_inputs(B, a.cap_len, a)
     clip = "clip_fea" in host
-    result_host = torch.empty(B, 16, 4, 90, 160, dtype=torch.bfloat16).pin_memory()
+    out_shape = (B, cfg.out_dim) + tuple(host["x"].shape[2:])
+    result_host = torch.empty(out_shape, dtype=torch.bfloat16).pin_memory()
     h2d = sum(v.numel() * v.element_size() for v in host.values())
     d2h = result_host.numel() * result_host.element_size()
     launches = 0
@@ -113,7 +133,7 @@ def main() -> int:
         if world == 1:
             d = {k: v.to(dev) for k, v in host.items()}
             stage = {k: torch.empty_like(v, device=dev) for k, v in host.items()}
-            out_buf = torch.empty(B, 16, 4, 90, 160, dtype=torch.bfloat16, device=dev)
+            out_buf = torch.empty(out_shape, dtype=torch.bfloat16, device=dev)
 
             cond = ("context", "clip_fea") if clip else ("context",)
 
@@ -128,8 +148,10 @@ def main() -> int:
                 result_host.copy_(out_buf, non_blocking=True)
         else:
             from comfyui_parallelanything_b200.parallel.spmd import SpmdWanEngine
-            eng = SpmdWanEngine(ex, B, 4, 720, 1280, a.cap_len, weights=pcts,
-                                clip_tokens=host["clip_fea"].shape[1] if clip else 0)
+            _, height, width = geometry(a)
+            eng = SpmdWanEngine(ex, B, host["x"].shape[2], height, width, a.cap_len, weights=pcts,
+                                clip_tokens=host["clip_fea"].shape[1] if clip else 0,
+                                frame_timesteps=host["timesteps"].dim() == 2)
             order = [host[k] for k in ("x", "timesteps", "context", "sig") + (("clip_fea",) if clip else ())]
             if rank == 0:
                 eng.stage_inputs(*order)

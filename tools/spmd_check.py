@@ -97,8 +97,9 @@ def bcast_check(rank, world, dev) -> int:
 
 def other_family(family, rank, world, dev) -> int:
     """Same comparison for the SDXL-class UNet (``unet``), Z-Image (``zimage``) and the WAN video DiT engines: ``wan``
-    (text-to-video, 16 latent channels), ``wan_i2v`` (image-to-video: 36 input channels, 16 output channels) and
-    ``wan_clip`` (WAN2.1 image-to-video: ``wan_i2v`` plus CLIP image features staged as the ``"clip"`` input)."""
+    (text-to-video, 16 latent channels), ``wan_i2v`` (image-to-video: 36 input channels, 16 output channels),
+    ``wan_clip`` (WAN2.1 image-to-video: ``wan_i2v`` plus CLIP image features staged as the ``"clip"`` input) and
+    ``wan_ti2v`` (WAN2.2 TI2V: 48 channels in and out, one timestep per latent frame staged as ``"t"`` [B, T])."""
     import torch
     import torch.distributed as dist
     from comfyui_parallelanything_b200.parallel import spmd
@@ -135,10 +136,15 @@ def other_family(family, rank, world, dev) -> int:
             p, make_inputs = dataclasses.replace(p, in_dim=36), wan.i2v_inputs
         elif family == "wan_clip":
             p, make_inputs = dataclasses.replace(p, in_dim=36, clip_dim=128), wan.clip_inputs
+        elif family == "wan_ti2v":
+            p, make_inputs = dataclasses.replace(p, in_dim=48, out_dim=48), wan.ti2v_inputs
         torch.manual_seed(2)
         cls = WanClipExecutor if family == "wan_clip" else WanExecutor
         ex = cls(wan.WanModel(p).to(device=dev, dtype=torch.bfloat16).eval(), dev, cuda_graphs=True)
-        inp = make_inputs(p, B, frames=8, height=128, width=192, device=dev, dtype=torch.bfloat16)
+        frames, height, width = (9, 256, 384) if family == "wan_ti2v" else (8, 128, 192)   # TI2V: 16x VAE
+        inp = make_inputs(p, B, frames=frames, height=height, width=width, device=dev, dtype=torch.bfloat16)
+        if family == "wan_ti2v":
+            inp["timesteps"][:, 1:] = torch.linspace(300.0, 900.0, B, device=dev)[:, None].to(torch.bfloat16)
         if family == "wan_clip":
             x, t, c, cf = ex._prep(inp["x"], inp["timesteps"], inp["context"], inp["clip_fea"])
             want = ex.denoise_step(x, t, c, cf, sig).clone()
@@ -148,8 +154,9 @@ def other_family(family, rank, world, dev) -> int:
             order = [x, t, c, sig]
             want = ex.denoise_step(*order).clone()
         li = cf.shape[1] if family == "wan_clip" else 0
-        make = lambda backend, w: spmd.SpmdWanEngine(ex, B, x.shape[2], 128, 192, c.shape[1], weights=w,  # noqa: E731
-                                                     backend=backend, clip_tokens=li)
+        make = lambda backend, w: spmd.SpmdWanEngine(  # noqa: E731
+            ex, B, x.shape[2], height, width, c.shape[1], weights=w, backend=backend, clip_tokens=li,
+            frame_timesteps=family == "wan_ti2v")
     res = {}
     for backend, tma_peer in (("fused", "1"), ("fused", "0"), ("nccl", "0")):
         os.environ["PA_TMA_PEER"] = tma_peer
